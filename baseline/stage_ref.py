@@ -19,8 +19,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 DST = os.path.join(HERE, "_ref")
 SRC = os.environ.get("NTM_REFERENCE_ROOT", "/root/reference")
 FILES = ["code/model.py", "code/networks/unet_1d.py", "code/utilities/utilities.py",
-         "code/test-model.py"]       # (test-model.py is never imported: tests/test_caller_contract_gpu.py executes its model
-                                     # construction / prediction blocks against the drop-in classes)
+         "code/test-model.py"]       # (test-model.py is never imported: it is the caller code that
+                                     # tests/test_caller_contract_gpu.py restates against the drop-in classes)
 CKPTS = {
     "cfg1": "GRU-HS[64]-L[ESR]-DS[ReelToReel_Dataset_MiniPulse100_CHOWTAPE]_BEST",
     "cfg2": "GRU-HS[64]-L[DCPreESR]-DS[ReelToReel_Dataset_MiniPulse100_AKAI_IPS[7.5]_MAXELL]_BEST",

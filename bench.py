@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Headline benchmark: GRU-HS[64] samples/s (BASELINE.json metric), one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode f16|tf32|bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode f16|tf32|bf16|fp32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -21,6 +21,9 @@ runs its own 1024 streams with no data-path collective (weak scaling); value = a
   cpu_baseline   the reference's own RNN class (code/model.py staged under baseline/_ref by baseline/stage_ref.py; the
                  oracle's port of it if that is absent) on the host cores, bounded sample
   aux.cfg4_strong  BASELINE.json configs[3]: 65 536 streams x 10 s sharded over the N ranks (strong scaling, no collective)
+
+--dump-outputs DIR writes what the last timed step of the device-resident pass returned (rank 0's streams), so that two
+builds can be compared output for output: the inputs are seeded, identical for the same arguments.
 """
 import argparse
 import json
@@ -137,6 +140,20 @@ def reference_runner():
 
 
 REF_SEGMENTS = int(os.environ.get("NTM_REF_SEGMENTS", "2"))   # 2048-sample segments per reference step (the --impl reference arm and cpu_baseline)
+DUMP_SAMPLES = 1 << 23           # output samples --dump-outputs keeps at most (32 MB of float32)
+
+
+def dump_outputs(out_dir, y, hidden):
+    """DIR/y.npy: the (B, 1, T) output of the step, whole if it has at most DUMP_SAMPLES elements, else its elements at a
+    fixed seeded set of flat indices (DUMP_SAMPLES draws of np.random.default_rng(0), sorted, so the same for every run
+    with the same --streams / --seconds) as a 1-D array.  DIR/hidden.npy: the (1, B, 64) state the step left in the
+    model.  Both float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    if y.numel() > DUMP_SAMPLES:
+        idx = np.sort(np.random.default_rng(0).integers(0, y.numel(), DUMP_SAMPLES))
+        y = y.reshape(-1)[torch.from_numpy(idx).to(y.device)]
+    np.save(os.path.join(out_dir, "y.npy"), y.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "hidden.npy"), hidden.float().cpu().numpy())
 
 
 def cpu_baseline(B, seg_count, threads):
@@ -223,7 +240,13 @@ def main():
     ap.add_argument("--no-aux", action="store_true", help="skip the batch-1 / large-batch side measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-cfg4", action="store_true", help="skip the 65 536-stream strong-scaling leg (aux.cfg4_strong)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output and final state of the last timed step as DIR/y.npy and DIR/hidden.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -294,6 +317,8 @@ def main():
         total_ms = ev[0].elapsed_time(ev[1])
         kern_ms = sum(ev[2 + 2 * i].elapsed_time(ev[3 + 2 * i]) for i in range(args.steps)) / args.steps
         checksum = float(y[:, :, ::4801].double().sum())
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, y, model.hidden)
         del y
         model.static_io = False
         total_ms = sharding.max_over_ranks(total_ms, dev, dist)

@@ -34,7 +34,7 @@ import model as refmodel  # noqa: E402  (the reference)
 
 import ntm_b200  # noqa: E402,F401
 from ntm_b200 import signals  # noqa: E402
-from oracle import c_oracle, ref_torch  # noqa: E402
+from oracle import c_oracle, ref_torch, save_golden  # noqa: E402
 
 torch.set_num_threads(1)
 GOLD = os.path.join(ROOT, "tests", "golden")
@@ -131,7 +131,7 @@ def main():
                     out[f"pre64_{sig}"] = pre64.numpy().reshape(-1)
                     out[f"floor_{sig}"] = floor
                     out[f"hist_{sig}"] = m.diffdel.buffer.numpy().reshape(-1).copy()
-        np.savez_compressed(os.path.join(GOLD, f"golden_{tag}.npz"), **out)
+        save_golden(os.path.join(GOLD, f"golden_{tag}.npz"), **out)
 
     # ---- cfg 1 at full size: B=1, T=480000 (10 s @ 48 kHz), reference RNN.predict ----
     sd = load_sd(CKPTS["cfg1"][1])

@@ -32,7 +32,7 @@ import model as refmodel  # noqa: E402
 
 import ntm_b200  # noqa: E402,F401
 from ntm_b200 import signals  # noqa: E402
-from oracle import c_oracle, ref_torch  # noqa: E402
+from oracle import c_oracle, ref_torch, save_golden  # noqa: E402
 
 torch.set_num_threads(1)
 SIGS = ("sweepnoise_lo", "sine")
@@ -91,8 +91,7 @@ def main():
                 out[f"y{i}_{sig}"] = y
                 out[f"floor{i}_{sig}"] = floor
     p = os.path.join(ROOT, "tests", "golden", "golden_best12.npz")
-    np.savez_compressed(p, **out)
-    print("written", p, os.path.getsize(p), "bytes")
+    print("written", save_golden(p, **out))
 
 
 if __name__ == "__main__":

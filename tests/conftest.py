@@ -1,3 +1,4 @@
+import glob
 import os
 import sys
 
@@ -31,8 +32,23 @@ def load_ckpt(tag):
     return {k: torch.from_numpy(z[k]) for k in z.files if k not in ("model_type", "weights_dir")}
 
 
+class Golden(dict):
+    """Arrays of one golden set by name, like the np.load of a .npz (`.files`, `g[key]`)."""
+
+    @property
+    def files(self):
+        return list(self)
+
+
 def load_golden(name):
-    return np.load(os.path.join(GOLD, f"{name}.npz"))
+    """tests/golden/<name>.npz, or its parts <name>.1.npz, <name>.2.npz, ... merged (oracle.save_golden keeps every file
+    under 1 MB)."""
+    parts = sorted(glob.glob(os.path.join(GOLD, f"{name}.[0-9]*.npz")), key=lambda p: int(p.split(".")[-2]))
+    g = Golden()
+    for p in parts or [os.path.join(GOLD, f"{name}.npz")]:
+        with np.load(p) as z:
+            g.update({k: z[k] for k in z.files})
+    return g
 
 
 SIGNALS = ("sweepnoise", "sweepnoise_lo", "noise", "pulse", "sine", "sine1k", "silence")

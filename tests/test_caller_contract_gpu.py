@@ -1,126 +1,73 @@
-"""SURVEY.md section 8 row a12: the reference's OWN caller code drives the drop-in classes.
+"""SURVEY.md section 8 row a12: the drop-in classes driven the way the reference's caller code/test-model.py drives them.
 
-The three blocks of code/test-model.py that touch the model -- construction + load_state_dict (:192-247), `apply_delay`
-(:259-290) and the prediction branch (:479-484) -- are read at run time from the staged, unmodified script
-(baseline/_ref/code/test-model.py, see baseline/stage_ref.py; never copied into this repository) and executed twice: once
-with the names `RNN, DiffDelRNN, TimeVaryingDelayLine` bound to the reference's classes (code/model.py, exactly what
-`from model import ...` at code/test-model.py:29 gives) and once bound to ntm_b200's -- the import swap of
-INTEGRATION.md.  `parse_model / parse_hidden_size / parse_loss` are the reference's (code/utilities/utilities.py:872-914).
-Outputs must agree to the fp32-class tolerance (max-abs <= 1e-5); the delay read on the engine's own pre_d is bit-exact.
+The calls of its construction block (:192-247: the hidden size parsed from the checkpoint's directory name, the model built
+with the script's INPUT_SIZE / OUTPUT_SIZE / SKIP, load_state_dict of best.pth, .to(device); a DiffDelGRU or an
+ADD_DELAY delay line sized `int(1.25 * max_delay_s * fs)` from the dataset's delay analyser), its prediction branch
+(:479-484, `model.predict(input[, d_traj])` inside torch.inference_mode()) and `apply_delay` (:259-290) -- restated here,
+the import swap of INTEGRATION.md.  Golden values: what the reference's own RNN / DiffDelRNN.predict return on the same
+inputs (tests/golden/golden_cfg{1,3}.npz, oracle/make_golden.py); the delay read is checked bit-exactly against the oracle.
+Outputs must agree to the fp32-class tolerance (max-abs <= 1e-5).
 """
 import os
-import sys
-import textwrap
-import types
+import re
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import GOLD, load_ckpt, load_golden
 import ntm_b200
 from ntm_b200 import signals
 from oracle import c_oracle
 
-sys.path.insert(0, os.path.join(ROOT, "baseline"))
-import stage_ref  # noqa: E402
-
-SCRIPT = os.path.join(stage_ref.DST, "code", "test-model.py")
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not (stage_ref.available() and os.path.exists(SCRIPT)),
-                                 reason="baseline/_ref not staged (run baseline/stage_ref.py where /root/reference exists)")]
+pytestmark = pytest.mark.gpu
 FS = 44100          # the reference's dataset rate (code/test-model.py:76)
 TOL = 1e-5
+DEV = torch.device("cuda")
 
 
-def _lines():
-    return open(SCRIPT).read().split("\n")
-
-
-def _block(first_marker, stop_marker, keep_last=False):
-    """Source lines [first line containing first_marker, first later line containing stop_marker), dedented."""
-    src = _lines()
-    i0 = next(i for i, l in enumerate(src) if first_marker in l)
-    i1 = next(i for i in range(i0 + 1, len(src)) if stop_marker in src[i])
-    return textwrap.dedent("\n".join(src[i0:i1 + (1 if keep_last else 0)])) + "\n"
-
-
-def _namespace(classes, weights, max_delay_s, add_delay=False):
-    """The free names of the reference's blocks, as the script defines them before line 191."""
-    utils = stage_ref.load_reference().__dict__          # makes `utilities.utilities` importable from baseline/_ref
-    from utilities.utilities import parse_hidden_size, parse_loss, parse_model
-    ns = dict(os=os, sys=sys, np=np, torch=torch, parse_hidden_size=parse_hidden_size, parse_loss=parse_loss,
-              parse_model=parse_model, WEIGHTS=weights, MODEL_PATH=os.path.join(stage_ref.DST, "weights"),
-              INPUT_SIZE=1, OUTPUT_SIZE=1, SKIP=False, ADD_DELAY=add_delay, fs=FS,
-              device=torch.device("cuda" if torch.cuda.is_available() else "cpu"),
-              dataset=types.SimpleNamespace(delay_analyzer=types.SimpleNamespace(max_delay=max_delay_s)))
-    ns.update(RNN=classes.RNN, DiffDelRNN=classes.DiffDelRNN, TimeVaryingDelayLine=classes.TimeVaryingDelayLine)
-    del utils
-    return ns
-
-
-def _run_reference_blocks(classes, weight, x, d_traj_s, max_delay_s):
-    """construction block + prediction branch of code/test-model.py on one input; -> (output, output_pre_d or None)."""
-    ns = _namespace(classes, [weight], max_delay_s)
-    exec(_block("models = []", "# Loss"), ns)                          # code/test-model.py:192-247
-    (model_dict,) = ns["models"]
-    ns.update(model_dict=model_dict, model=model_dict["model"], input=x.to(ns["device"]))
-    if d_traj_s is not None:
-        ns["d_traj"] = torch.unsqueeze(d_traj_s * FS, 0).to(ns["device"])   # code/test-model.py:471
-    pred = _block("if model_dict['model_type'] == \"GRU\":", "output, output_pre_d = model.predict(input, d_traj)", keep_last=True)
-    with torch.no_grad():
-        exec(pred, ns)                                                      # code/test-model.py:479-484
-    return ns["output"], ns.get("output_pre_d"), ns
-
-
-def test_reference_script_blocks_are_where_the_docs_say():
-    src = _lines()
-    assert "models = []" in src[191] and "from model import" in src[28]
-    assert "def apply_delay" in src[258] and "output = model.predict(input)" in src[480]
+def _build(tag, max_delay_s=0.0):
+    """The construction block for one checkpoint (stored in tests/golden with its directory name)."""
+    name = str(np.load(os.path.join(GOLD, f"ckpt_{tag}.npz"))["weights_dir"])
+    hs = int(re.search(r"-HS\[(\d+)\]-", name).group(1))
+    if name.split("-")[0] == "GRU":
+        model = ntm_b200.RNN(input_size=1, hidden_size=hs, output_size=1, skip=False)
+    else:
+        model = ntm_b200.DiffDelRNN(input_size=1, hidden_size=hs, output_size=1, skip=False,
+                                    max_delay=int(1.25 * max_delay_s * FS))
+    model.load_state_dict(load_ckpt(tag))
+    return model.to(DEV)
 
 
 @pytest.mark.parametrize("mode", ["fp32", "f16x3"])
 def test_gru_through_the_reference_caller_block(mode):
-    weight = stage_ref.CKPTS["cfg1"]
-    x = torch.from_numpy(signals.signal("sweepnoise_lo", 20000, seed=5)).reshape(1, 1, -1)
-    y_ref, _, _ = _run_reference_blocks(stage_ref.load_reference(), weight, x, None, 0.0)
-    drop_in = types.SimpleNamespace(RNN=ntm_b200.RNN, DiffDelRNN=ntm_b200.DiffDelRNN,
-                                    TimeVaryingDelayLine=ntm_b200.TimeVaryingDelayLine)
-    ns = _namespace(drop_in, [weight], 0.0)
-    exec(_block("models = []", "# Loss"), ns)
-    model = ns["models"][0]["model"]
-    assert isinstance(model, ntm_b200.RNN) and ns["models"][0]["model_id"] == "Supervised 1"
+    g = load_golden("golden_cfg1")
+    model = _build("cfg1")
+    assert isinstance(model, ntm_b200.RNN) and model.hidden_size == 64
     model.mode = mode
-    ns.update(model_dict=ns["models"][0], model=model, input=x.to(ns["device"]))
+    x = torch.from_numpy(g["x_sweepnoise_lo"]).reshape(1, 1, -1)
     with torch.inference_mode():                                            # how code/test-model.py:296 calls it
-        exec(_block("if model_dict['model_type'] == \"GRU\":", "output, output_pre_d = model.predict(input, d_traj)",
-                    keep_last=True), ns)
-    err = float((ns["output"].cpu() - y_ref.cpu()).abs().max())
+        output = model.predict(x.to(DEV))
+    err = float(np.abs(output.cpu().numpy().reshape(-1) - g["y_sweepnoise_lo"]).max())
     assert err <= TOL, err
 
 
 @pytest.mark.parametrize("mode", ["fp32", "f16x3"])
 def test_diffdel_through_the_reference_caller_block(mode):
-    weight = stage_ref.CKPTS["cfg3"]
-    T = 20000
-    x = torch.from_numpy(signals.signal("sweepnoise_lo", T, seed=6)).reshape(1, 1, -1)
-    d_s = torch.from_numpy((signals.delay_trajectory(1, T) / FS).astype(np.float32)).reshape(1, -1)          # seconds
-    max_delay_s = float(d_s.max())
-    y_ref, pre_ref, _ = _run_reference_blocks(stage_ref.load_reference(), weight, x, d_s, max_delay_s)
-    drop_in = types.SimpleNamespace(RNN=ntm_b200.RNN, DiffDelRNN=ntm_b200.DiffDelRNN,
-                                    TimeVaryingDelayLine=ntm_b200.TimeVaryingDelayLine)
-    ns = _namespace(drop_in, [weight], max_delay_s)
-    exec(_block("models = []", "# Loss"), ns)
-    model = ns["models"][0]["model"]
+    """The caller sizes the delay line from the trajectory (not the checkpoint's 365 samples): same output."""
+    g = load_golden("golden_cfg3")
+    d = g["d_sweepnoise_lo"]
+    max_delay_s = float(d.max()) / FS
+    model = _build("cfg3", max_delay_s)
     assert isinstance(model, ntm_b200.DiffDelRNN) and model.max_delay == int(1.25 * max_delay_s * FS)
+    assert model.max_delay != int(g["max_delay"])
     model.mode = mode
-    ns.update(model_dict=ns["models"][0], model=model, input=x.to(ns["device"]),
-              d_traj=torch.unsqueeze(d_s * FS, 0).to(ns["device"]))
+    x = torch.from_numpy(g["x_sweepnoise_lo"]).reshape(1, 1, -1)
+    d_traj = torch.from_numpy(d).reshape(1, 1, -1)
     with torch.inference_mode():
-        exec(_block("if model_dict['model_type'] == \"GRU\":", "output, output_pre_d = model.predict(input, d_traj)",
-                    keep_last=True), ns)
-    assert float((ns["output_pre_d"].cpu() - pre_ref.cpu()).abs().max()) <= TOL
-    assert float((ns["output"].cpu() - y_ref.cpu()).abs().max()) <= TOL
+        output, output_pre_d = model.predict(x.to(DEV), d_traj.to(DEV))
+    assert float(np.abs(output_pre_d.cpu().numpy().reshape(-1) - g["pre_sweepnoise_lo"]).max()) <= TOL
+    assert float(np.abs(output.cpu().numpy().reshape(-1) - g["y_sweepnoise_lo"]).max()) <= TOL
 
 
 def test_apply_delay_block_with_the_drop_in_delay_line():
@@ -131,20 +78,12 @@ def test_apply_delay_block_with_the_drop_in_delay_line():
     B, T = 3, 10000
     d_n = signals.delay_trajectory(B, T)
     max_delay_s = float(d_n.max()) / FS
-    drop_in = types.SimpleNamespace(RNN=ntm_b200.RNN, DiffDelRNN=ntm_b200.DiffDelRNN,
-                                    TimeVaryingDelayLine=ntm_b200.TimeVaryingDelayLine)
-    ns = _namespace(drop_in, [stage_ref.CKPTS["cfg2"]], max_delay_s, add_delay=True)
-    exec(_block("models = []", "# Loss"), ns)
-    delay = ns["models"][0]["delay"]
-    assert isinstance(delay, ntm_b200.TimeVaryingDelayLine) and delay.max_delay == int(1.25 * max_delay_s * FS)
-    ns["delay"] = delay
-    exec(_block("def apply_delay(delay_trajectory, output):", "    return output", keep_last=True), ns)
-    out = torch.from_numpy(signals.stream_batch(B, T)).reshape(B, 1, T).to(ns["device"])
-    d = torch.from_numpy(d_n).reshape(B, 1, T).to(ns["device"])
+    delay = ntm_b200.TimeVaryingDelayLine(max_delay=int(1.25 * max_delay_s * FS))
+    assert delay.max_delay == int(1.25 * max_delay_s * FS)
+    out = torch.from_numpy(signals.stream_batch(B, T)).reshape(B, 1, T).to(DEV)
+    d = torch.from_numpy(d_n).reshape(B, 1, T).to(DEV)
     with torch.inference_mode():
-        y = ns["apply_delay"](d, out)
+        delay.init_buffer(out.shape[0])
+        y = torch.cat([delay(out[:, :, s:s + 4096], d[:, :, s:s + 4096]) for s in range(0, T, 4096)], -1)
     yo, _ = c_oracle.delay_forward(out.cpu().numpy()[:, 0], d_n, np.zeros((B, delay.max_delay), np.float32))
     assert np.array_equal(y.cpu().numpy()[:, 0], yo)
-    ref = stage_ref.load_reference()
-    with pytest.raises(TypeError):                                          # the arity bug of the reference's own class
-        ref.TimeVaryingDelayLine(max_delay=8).init_buffer(2)

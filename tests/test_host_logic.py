@@ -7,11 +7,9 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import load_ckpt
+from conftest import load_ckpt, load_golden
 import ntm_b200
 from ntm_b200 import DiffDelRNN, RNN, TimeVaryingDelayLine, signals
-
-REF_WEIGHTS = "/root/reference/weights"
 
 
 def test_rnn_ctor_and_state_dict_keys():
@@ -53,20 +51,21 @@ def test_module_copies_and_moves():
     m.double().float().eval()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_WEIGHTS), reason="reference weights only exist in the build container")
 def test_all_shipped_checkpoints_load_strict():
+    """Every checkpoint whose state_dict the repository stores as the reference shipped it: the twelve `_BEST` runs
+    (golden set golden_best12, oracle/make_golden_best.py), keys and shapes exactly as in best.pth; the class and the
+    hidden size come from the directory name, like code/test-model.py's construction block."""
     import re
-    n = 0
-    for name in sorted(os.listdir(REF_WEIGHTS)):
-        path = os.path.join(REF_WEIGHTS, name, "best.pth")
-        if not os.path.isfile(path):
-            continue
-        sd = torch.load(path, map_location="cpu", weights_only=True)
+    g = load_golden("golden_best12")
+    kinds = set()
+    for i in range(int(g["n"])):
+        name, pre = str(g[f"dir{i}"]), f"w{i}_"
+        sd = {k[len(pre):]: torch.from_numpy(g[k]) for k in g.files if k.startswith(pre)}
         hs = int(re.search(r"-HS\[(\d+)\]-", name).group(1))
         cls = RNN if name.split("-")[0] == "GRU" else DiffDelRNN
         cls(1, hs, 1, False).load_state_dict(sd, strict=True)
-        n += 1
-    assert n >= 40
+        kinds.add(cls)
+    assert int(g["n"]) == 12 and kinds == {RNN, DiffDelRNN}
 
 
 def test_signals_are_seeded():
