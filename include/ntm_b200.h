@@ -180,11 +180,19 @@ int ntm_diffdel_predict_host(void* handle, int mode, const float* x_host, const 
 int ntm_esr_sums_rows(const float* out, int64_t ldo, const float* target, int64_t ldt, int64_t B, int64_t T,
                       const int64_t* first, const int64_t* count, int dc_pre, double* sums, int device, void* stream);
 
-/* Kernel-selection knob for experiments and tests (0, 0 = automatic dispatch).  fp32 kernel: streams per CTA / k-split.
- * Tensor-core modes, by the second argument: 3 warp-level mma.sync kernel (first = streams per CTA 4|8|16),
- * 4 stream-major tcgen05 kernel (first = 128-stream tiles per CTA 1|2,
- * + 4 * (variant + 1) for kernel variants).  ntm_set_tuning sets the process-wide default (one atomic word, safe to
- * call concurrently with launches); ntm_handle_set_tuning overrides it for one handle (streams_per_cta = -1: follow the
+/* Kernel-selection knob for tests and benchmarks.  The pair (streams_per_cta, ksplit) means, by mode:
+ *   mode          pair                        runs
+ *   any           (0, 0)                      automatic dispatch
+ *   fp32          (s, ks), s in {0,1,2,4,8},  CUDA-core kernel, s streams per CTA, ks k-slices per hidden unit
+ *                 ks in {0,2,4}; ks = 2 only  (0 = automatic)
+ *                 with s = 1 or 2
+ *   tensor-core   (4, 3), (8, 3)              general warp-level mma.sync kernel, 4 or 8 streams per CTA
+ *   tensor-core   (4, 6)                      lean 4-stream mma.sync kernel (tf32 has no lean form: the general kernel with
+ *                                             automatic streams per CTA)
+ *   tensor-core   (t, 4), t in {1, 2}         stream-major tcgen05 kernel, t 128-stream tiles per CTA
+ *   tensor-core   (t + 4, 4)                  the same with the static schedule (one CTA per tile group, no job queue)
+ * Any other pair makes the launch return NTM_EINVAL.  ntm_set_tuning sets the process-wide default (one atomic word, safe
+ * to call concurrently with launches); ntm_handle_set_tuning overrides it for one handle (streams_per_cta = -1: follow the
  * default again).  ntm_handle_last_kernel: NTM_Q_LAST_KERNEL of that handle's last launch. */
 int ntm_set_tuning(int streams_per_cta, int ksplit);
 int ntm_handle_set_tuning(void* handle, int streams_per_cta, int ksplit);

@@ -17,18 +17,18 @@ namespace {
 
 constexpr unsigned HANDLE_MAGIC = 0x4e544d42u;   // "NTMB"
 thread_local int t_last_cuda = 0;
-// Kernel-selection knob (experiments / tests): a process-wide default (ntm_set_tuning) that a handle may override
-// (ntm_handle_set_tuning).  Packed into one atomic word so that concurrent launches from several threads read a
-// consistent pair; nothing on the launch path writes shared state except the two counters below.
+// Kernel-selection knob (tests, benchmarks; the pairs are tabled in include/ntm_b200.h): a process-wide default
+// (ntm_set_tuning) that a handle may override (ntm_handle_set_tuning).  Packed into one atomic word so that concurrent
+// launches from several threads read a consistent pair; nothing on the launch path writes shared state except the two
+// counters below.
 struct Tuning {
     int s = 0, ks = 0;
 };
 std::atomic<unsigned long long> g_tuning{0};
 unsigned long long pack_tuning(int s, int ks) { return ((unsigned long long)(unsigned)s << 32) | (unsigned)ks; }
 Tuning unpack_tuning(unsigned long long v) { return Tuning{(int)(v >> 32), (int)(v & 0xffffffffull)}; }
-// 0 fp32 CUDA-core, 1 warp-level mma.sync, 3 tcgen05 stream-major (NTM_Q_LAST_KERNEL; also kept per handle)
+// NTM_Q_LAST_KERNEL (also kept per handle)
 std::atomic<int> g_last_kernel{-1};
-constexpr long long TCS_MIN_STREAMS_PER_SM = 110;     // crossover mma.sync -> stream-major tcgen05 kernel (DESIGN.md 3.3)
 
 struct HostPipe {            // staging of the *_host entry points
     cudaStream_t s_in = nullptr, s_run = nullptr, s_out = nullptr;
@@ -93,53 +93,105 @@ constexpr int MODE_MASK = (1 << NTM_MODE_FP32) | (1 << NTM_MODE_TF32) | (1 << NT
 int mode_fmt(int mode) { return mode == NTM_MODE_TF32 ? 2 : mode == NTM_MODE_BF16 ? 1 : mode == NTM_MODE_F16X3 ? 3 : 0; }
 bool mode_supported(int mode) { return mode >= 0 && mode < 31 && ((MODE_MASK >> mode) & 1); }
 
+// Recurrent kernels, by their NTM_Q_LAST_KERNEL id
+enum Kernel { K_FP32 = 0, K_MMA = 1, K_TCS = 3, K_MMA4 = 4 };
+
+// One launch's kernel and configuration, fully resolved: the launchers decide nothing.
+struct LaunchCfg {
+    int kernel = -1;
+    int fp32_streams = 0, fp32_ksplit = 0;   // K_FP32: streams per CTA (1, 2, 4, 8), k-slices per hidden unit (2, 4)
+    int mma_streams = 0;                     // K_MMA: streams per CTA (4, 8)
+    bool defer_head = false;                 // K_MMA, 4 streams per CTA: the deferred-head form
+    int tcs_tiles = 0;                       // K_TCS: 128-stream tiles per CTA (1, 2)
+    bool static_schedule = false;            // K_TCS: one CTA per tile group, no job queue
+};
+
+constexpr long long TCS_MIN_STREAMS_PER_SM = 110;     // crossover mma.sync -> stream-major tcgen05 kernel (DESIGN.md 3.3)
+
+// Every kernel-selection rule of the engine: (mode, batch, SMs, tuning pair) -> configuration, or NTM_EINVAL for a tuning
+// pair that has no meaning in this mode (the table in include/ntm_b200.h).
+int resolve_launch(int mode, long long B, int sm_count, Tuning tune, LaunchCfg* out)
+{
+    LaunchCfg c;
+    const int s = tune.s, ks = tune.ks;
+    const bool automatic = s == 0 && ks == 0;
+    if (mode == NTM_MODE_FP32) {
+        // (streams per CTA, k-split), 0 = automatic; the 2-way k-split exists for one and two streams per CTA
+        if ((s != 0 && s != 1 && s != 2 && s != 4 && s != 8) || (ks != 0 && ks != 2 && ks != 4)) return NTM_EINVAL;
+        if (ks == 2 && s != 1 && s != 2) return NTM_EINVAL;
+        c.kernel = K_FP32;
+        c.fp32_streams = s;
+        if (s == 0) {
+            // fill the SMs first (two CTAs per SM), then grow the streams per CTA
+            const long long per_cta = (B + 2ll * sm_count - 1) / (2ll * sm_count);
+            c.fp32_streams = 1;
+            while (c.fp32_streams < 8 && c.fp32_streams < per_cta) c.fp32_streams <<= 1;
+        }
+        // measured on B200 (tools/experiments/sweep_fp32.py): the 2-way k-split wins while a CTA owns <= 2 streams
+        c.fp32_ksplit = ks != 0 ? ks : c.fp32_streams <= 2 ? 2 : 4;
+        *out = c;
+        return NTM_OK;
+    }
+    const bool strict = mode == NTM_MODE_F16X3;
+    // four streams per CTA, 16-bit operands or the strict mode (cfg 2's width and below, GRU and DiffDelGRU): the lean form of
+    // gru_mma4.cu (same results, bit for bit: 194.5 vs 215 ns/step at 1024 streams, 162 vs 168 at batch 1).  The strict form
+    // only while every CTA has an SM of its own: with two CTAs per SM the general kernel's 4-stream form is faster, 361.7 vs
+    // 366.8 ns/step at 1024 streams.  f16 / bf16 up to THREE such CTAs per SM: 5.19 vs 5.03e9 samples/s at 1480 streams, 6.23 vs
+    // 6.04 at 1776 against the 8-stream form; beyond 12 streams per SM the 8-stream form wins: 6.96 vs 5.08 at 2048.
+    const bool lean_ok = mode != NTM_MODE_TF32;
+    const bool lean_auto = strict ? B <= 4ll * sm_count : B <= 12ll * sm_count;
+    if (automatic) {
+        // latency regime (few streams per SM): warp-level mma.sync kernels; throughput regime (>= one 128-stream tile per
+        // SM): stream-major tcgen05 kernel (every operand format; DiffDelRNN batches run the delay read as a second pass)
+        if (B >= (long long)sm_count * TCS_MIN_STREAMS_PER_SM) {
+            c.kernel = K_TCS;
+            // one tile per SM (time-multiplexed by the job queue) beats two resident tiles until ~190 streams per SM (measured)
+            c.tcs_tiles = B >= 190ll * sm_count ? 2 : 1;
+        } else {
+            c.kernel = lean_ok && lean_auto ? K_MMA4 : K_MMA;
+        }
+    } else if (ks == 3 && (s == 4 || s == 8)) {                 // general mma.sync kernel, s streams per CTA
+        c.kernel = K_MMA;
+        c.mma_streams = s;
+    } else if (ks == 6 && s == 4) {                             // lean 4-stream kernel (tf32 has none: general kernel)
+        c.kernel = lean_ok ? K_MMA4 : K_MMA;
+    } else if (ks == 4 && (s == 1 || s == 2 || s == 5 || s == 6)) {   // tcgen05, 1 or 2 tiles per CTA (+ 4: static schedule)
+        c.kernel = K_TCS;
+        c.tcs_tiles = s & 3;
+        c.static_schedule = s > 4;
+    } else {
+        return NTM_EINVAL;
+    }
+    if (c.kernel == K_MMA) {
+        // automatic: 4 streams per CTA (shorter dependent step) up to two such CTAs per SM -- measured 216 vs 243 ns/step at
+        // 1024 streams, 172 vs 238 at <= 592 (profiles/r02_mma_variants.txt); the strict form too since its 4-stream layout
+        // carries the state residual in the otherwise dead columns (two MMAs per product instead of three): 363 vs 394
+        // ns/step at 1024 streams, 264 vs 388 at batch 1 (profiles/r02_strict_paircol.txt)
+        if (c.mma_streams == 0) c.mma_streams = B <= 8ll * sm_count ? 4 : 8;
+        // the deferred head wins while every 4-stream CTA has an SM of its own (B <= 4 streams per SM; rounded modes)
+        c.defer_head = c.mma_streams == 4 && !strict && (B + 3) / 4 <= sm_count;
+    }
+    *out = c;
+    return NTM_OK;
+}
+
 int run_gru(Handle* hd, int mode, const ntm::GruArgs& a, cudaStream_t st)
 {
     if (!mode_supported(mode)) return NTM_EUNSUPPORTED;
     unsigned long long tv = hd->tuning.load(std::memory_order_relaxed);
     if (tv == ~0ull) tv = g_tuning.load(std::memory_order_relaxed);
-    const Tuning tune = unpack_tuning(tv);
-    int kernel;
-    if (mode == NTM_MODE_FP32) {
-        // fp32 kernel: (streams per CTA, k-split); bit 8 of the second value selects the MUFU-approx activations (experiment)
-        CU(ntm::launch_gru_fp32(a, hd->sm_count, tune.s, tune.ks & 0xff, (tune.ks >> 8) & 1, st));
-        kernel = 0;
-    } else {
-        const int fmt = mode_fmt(mode);
-        // latency regime (few streams per SM): warp-level mma.sync kernel; throughput regime (>= one 128-stream tile per
-        // SM): stream-major tcgen05 kernel (every operand format; DiffDelRNN batches run the delay read as a second pass).
-        // Tuning (n, 3) forces mma.sync with n = 4 | 8 | 16 streams per CTA, (tiles + 4 * (variant + 1), 4) the
-        // stream-major kernel with 1 or 2 tiles per CTA.
-        const int tg = tune.ks & 0xff;
-        const bool use_tcs = tg == 4 || (tg == 0 && a.B >= (long long)hd->sm_count * TCS_MIN_STREAMS_PER_SM);
-        if (use_tcs) {
-            CU(ntm::launch_gru_tcs(a, hd->tcs, fmt, hd->sm_count, tg == 4 ? (tune.s & 3) : 0, tg == 4 ? (tune.s >> 2) - 1 : -1, st));
-            kernel = 3;
-        } else {
-            // automatic: 4 streams per CTA (shorter dependent step) up to two such CTAs per SM -- measured 216 vs 243
-            // ns/step at 1024 streams, 172 vs 238 at <= 592 (profiles/r02_mma_variants.txt); the strict form too since its
-            // 4-stream layout carries the state residual in the otherwise dead columns (two MMAs per product instead of
-            // three): 363 vs 394 ns/step at 1024 streams, 264 vs 388 at batch 1 (profiles/r02_strict_paircol.txt)
-            int nt;
-            if (tune.s > 0 && tg == 3) nt = tune.s / 8;
-            else nt = a.B <= 8ll * hd->sm_count ? 0 : 1;
-            // four streams per CTA, 16-bit operands or the strict mode (cfg 2's width and below, GRU and DiffDelGRU): the lean
-            // form of gru_mma4.cu (same results, bit for bit: 194.5 vs 215 ns/step at 1024 streams, 162 vs 168 at batch 1);
-            // forced with tuning (4, 6); (4, 3) keeps the general kernel
-            // (the strict form only while every CTA has an SM of its own: with two CTAs per SM the general kernel's 4-stream
-            // form is faster, 361.7 vs 366.8 ns/step at 1024 streams)
-            // (f16 / bf16 up to THREE such CTAs per SM: 5.19 vs 5.03e9 samples/s at 1480 streams, 6.23 vs 6.04 at 1776 against the 8-stream
-            // form; beyond 12 streams per SM the 8-stream form wins: 6.96 vs 5.08 at 2048)
-            const bool lean_ok = fmt == 0 || fmt == 1 || fmt == 3;
-            const bool lean_auto = fmt == 3 ? a.B <= 4ll * hd->sm_count : a.B <= 12ll * hd->sm_count;
-            const bool lean = lean_ok && (tg == 6 || (tg == 0 && lean_auto));
-            if (lean) CU(ntm::launch_gru_mma4(a, fmt, st));
-            else CU(ntm::launch_gru_mma(a, fmt, nt, st));
-            kernel = lean ? 4 : 1;
-        }
+    LaunchCfg c;
+    const int rc = resolve_launch(mode, a.B, hd->sm_count, unpack_tuning(tv), &c);
+    if (rc != NTM_OK) return rc;
+    const int fmt = mode_fmt(mode);
+    switch (c.kernel) {
+        case K_FP32: CU(ntm::launch_gru_fp32(a, c.fp32_streams, c.fp32_ksplit, st)); break;
+        case K_MMA: CU(ntm::launch_gru_mma(a, fmt, c.mma_streams, c.defer_head, st)); break;
+        case K_MMA4: CU(ntm::launch_gru_mma4(a, fmt, st)); break;
+        default: CU(ntm::launch_gru_tcs(a, hd->tcs, fmt, hd->sm_count, c.tcs_tiles, c.static_schedule, st)); break;
     }
-    hd->last_kernel.store(kernel, std::memory_order_relaxed);
-    g_last_kernel.store(kernel, std::memory_order_relaxed);
+    hd->last_kernel.store(c.kernel, std::memory_order_relaxed);
+    g_last_kernel.store(c.kernel, std::memory_order_relaxed);
     return NTM_OK;
 }
 

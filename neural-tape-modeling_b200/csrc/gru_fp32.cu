@@ -21,20 +21,8 @@ namespace ntm {
 
 namespace {
 
-// Activation flavours.  ACC: libm-grade expf / tanhf (<= 2 ulp) and IEEE division.  FAST: MUFU ex2.approx +
-// rcp.approx (each <= 2 ulp; ~1e-7 absolute on the gate values), 4-5 instructions per activation.
-template <bool FAST>
-__device__ __forceinline__ float sigmoid_f(float a)
-{
-    if (FAST) return rcp_approx(1.0f + ex2_approx(-1.4426950408889634f * a));
-    return 1.0f / (1.0f + expf(-a));
-}
-template <bool FAST>
-__device__ __forceinline__ float tanh_f(float a)
-{
-    if (FAST) return fmaf(-2.0f, rcp_approx(1.0f + ex2_approx(2.8853900817779268f * a)), 1.0f);
-    return tanhf(a);
-}
+// Activations: libm-grade expf / tanhf (<= 2 ulp) and IEEE division.
+__device__ __forceinline__ float sigmoid_f(float a) { return 1.0f / (1.0f + expf(-a)); }
 
 template <int KS, int SP>
 struct Transpose;   // combine the KS partial sums; lane q ends up owning streams i*KS + q
@@ -92,7 +80,7 @@ struct Cfg {
     static constexpr int SMEM_BYTES = SMEM_FLOATS * 4;
 };
 
-template <int KS, int S, bool FAST>
+template <int KS, int S>
 __global__ void __launch_bounds__(64 * KS, 2) gru_fp32_kernel(const GruArgs a)
 {
     using C = Cfg<KS, S>;
@@ -204,9 +192,9 @@ __global__ void __launch_bounds__(64 * KS, 2) gru_fp32_kernel(const GruArgs a)
                 const int s = i * KS + q;
                 const bool live = s < S;             // padded lanes compute garbage in lock-step, store nothing
                 const float xv = xcur[(live ? s : 0) * CH + tt];
-                const float r = sigmoid_f<FAST>(fmaf(wir, xv, br) + own[0][i]);
-                const float z = sigmoid_f<FAST>(fmaf(wiz, xv, bz) + own[1][i]);
-                const float nn = tanh_f<FAST>(fmaf(r, own[2][i] + bhn, fmaf(win, xv, bin)));
+                const float r = sigmoid_f(fmaf(wir, xv, br) + own[0][i]);
+                const float z = sigmoid_f(fmaf(wiz, xv, bz) + own[1][i]);
+                const float nn = tanhf(fmaf(r, own[2][i] + bhn, fmaf(win, xv, bin)));
                 const float hn = fmaf(hown[i] - nn, z, nn);      // (h - n) * z + n
                 hown[i] = hn;
                 if (live) hnext[s * HS + j] = hn;
@@ -280,54 +268,41 @@ __global__ void __launch_bounds__(64 * KS, 2) gru_fp32_kernel(const GruArgs a)
     }
 }
 
-template <int KS, int S, bool FAST>
+template <int KS, int S>
 cudaError_t launch_one(const GruArgs& a, cudaStream_t st)
 {
     using C = Cfg<KS, S>;
     static OncePerDevice once;
     cudaError_t e = once.run([] {
-        return cudaFuncSetAttribute(gru_fp32_kernel<KS, S, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
+        return cudaFuncSetAttribute(gru_fp32_kernel<KS, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
     });
     if (e != cudaSuccess) return e;
     const long long grid = (a.B + S - 1) / S;
-    gru_fp32_kernel<KS, S, FAST><<<(unsigned)grid, C::NT, C::SMEM_BYTES, st>>>(a);
+    gru_fp32_kernel<KS, S><<<(unsigned)grid, C::NT, C::SMEM_BYTES, st>>>(a);
     ++g_launches;
     return cudaGetLastError();
 }
 
-template <bool FAST>
-cudaError_t launch_cfg(const GruArgs& a, int s, int ks, cudaStream_t st)
-{
-    if (ks == 2) {
-        if (s <= 1) return launch_one<2, 1, FAST>(a, st);
-        return launch_one<2, 2, FAST>(a, st);
-    }
-    switch (s) {
-        case 1: return launch_one<4, 1, FAST>(a, st);
-        case 2: return launch_one<4, 2, FAST>(a, st);
-        case 4: return launch_one<4, 4, FAST>(a, st);
-        default: return launch_one<4, 8, FAST>(a, st);
-    }
-}
-
 }  // namespace
 
-cudaError_t launch_gru_fp32(const GruArgs& a, int sm_count, int tune_s, int tune_ks, int fast_act, cudaStream_t st)
+// streams: streams per CTA (1, 2, 4 or 8); ksplit: k-slices per hidden unit (2 with <= 2 streams per CTA, or 4)
+cudaError_t launch_gru_fp32(const GruArgs& a, int streams, int ksplit, cudaStream_t st)
 {
     if (a.B <= 0 || a.T <= 0) return cudaSuccess;
-    int s = tune_s;
-    if (s <= 0) {
-        // fill the SMs first (two CTAs per SM), then grow the streams per CTA
-        const long long per_cta = (a.B + 2 * sm_count - 1) / (2 * sm_count);
-        s = 1;
-        while (s < 8 && s < per_cta) s <<= 1;
+    if (ksplit == 2) {
+        switch (streams) {
+            case 1: return launch_one<2, 1>(a, st);
+            case 2: return launch_one<2, 2>(a, st);
+        }
+    } else if (ksplit == 4) {
+        switch (streams) {
+            case 1: return launch_one<4, 1>(a, st);
+            case 2: return launch_one<4, 2>(a, st);
+            case 4: return launch_one<4, 4>(a, st);
+            case 8: return launch_one<4, 8>(a, st);
+        }
     }
-    if (s != 1 && s != 2 && s != 4) s = 8;
-    // measured on B200 (tools/experiments/sweep_fp32.py): the 2-way k-split wins while a CTA owns <= 2 streams
-    int ks = tune_ks > 0 ? tune_ks : (s <= 2 ? 2 : 4);
-    if (ks != 2) ks = 4;
-    if (ks == 2 && s > 2) ks = 4;
-    return fast_act ? launch_cfg<true>(a, s, ks, st) : launch_cfg<false>(a, s, ks, st);
+    return cudaErrorInvalidValue;
 }
 
 }  // namespace ntm

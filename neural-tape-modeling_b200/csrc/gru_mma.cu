@@ -11,7 +11,7 @@
 // RNN.forward / DiffDelRNN.forward (code/model.py:81-82, :412-413; torch rnn.py:1221-1224) and the delay read
 // of code/model.py:422.
 //
-// One CTA = 4 warps owns 8*NT streams for all T steps.  Warp w owns hidden units [16w, 16w+16): three m16 tiles
+// One CTA = 4 warps owns 8 streams (one n8 tile) for all T steps.  Warp w owns hidden units [16w, 16w+16): three m16 tiles
 //   tile A rows 0-7: r of units 16w+0..7, rows 8-15: z of the same units      -> c0,c1 = r   c2,c3 = z   (unit u0)
 //   tile B the same for units 16w+8..15                                          -> c0,c1 = r   c2,c3 = z   (unit u1)
 //   tile C rows 0-7: n of units 16w+0..7, rows 8-15: n of units 16w+8..15        -> c0,c1 = n(u0) c2,c3 = n(u1)
@@ -33,9 +33,9 @@ namespace {
 
 constexpr float LOG2E_F = 1.4426950408889634f;
 
-template <int FMT, int NT, bool SPLIT = false>
+template <int FMT, bool SPLIT = false>
 struct MmaCfg {
-    static constexpr int S = 8 * NT;                 // streams per CTA
+    static constexpr int S = 8;                      // columns of the state tile (streams per CTA of the 8-stream form)
     static constexpr int CH = 128;                   // steps per staged chunk (measured at 1024 streams: 32 -> 232.7 ns/step, 64 -> 238, 128 -> 221.7, 256 -> 220.1)
     static constexpr int YP_LD = S + 2;              // even: float2 stores of the head partials
     static constexpr int HB_BYTES = S * Frag<FMT, SPLIT>::ROW_BYTES;
@@ -46,7 +46,7 @@ struct MmaCfg {
     static constexpr int SMEM_BYTES = OFF_DS + 2 * CH * S * 4;                    // + the pre_d ring, sized at launch
 };
 
-// HALF (NT == 1 only): the CTA owns 4 streams, placed in the EVEN columns of its n8 tile (stream s <-> column 2s), and
+// HALF: the CTA owns 4 streams, placed in the EVEN columns of its n8 tile (stream s <-> column 2s), and
 // skips the gate math, state stores and outputs of the odd columns: half the MUFU / FMA work per step for the same
 // MMAs -- the shorter dependent step wins whenever there are CTAs to spare (B <= 4 streams per SM: cfg 3, cfg 5).
 // RT (HALF only): resident real-time server -- the CTA stays on its SM, keeps weights, state and staging on chip and
@@ -54,14 +54,13 @@ struct MmaCfg {
 // costs two PCIe round trips instead of a kernel launch, a prologue and a stream synchronisation.
 // DEFER (HALF only): the output head's accumulators are consumed one iteration later (see the head block); wins when a
 // warp has its SM sub-partition to itself (one CTA per SM: cfg 3, cfg 5, the real-time server), loses otherwise.
-template <int FMT, int NT, bool HALF, bool RT = false, bool DEFER = RT, bool SPLIT = false>
+template <int FMT, bool HALF, bool RT = false, bool DEFER = RT, bool SPLIT = false>
 // (HALF is only dispatched up to two CTAs per SM: the full register file removes its spills, 197 vs 204 ns/step; the
 // strict form keeps two sets of weight fragments in registers)
 __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 4) gru_mma_kernel(const GruArgs a)
 {
-    static_assert(!HALF || NT == 1, "HALF needs a single n8 tile");
     static_assert(!RT || HALF, "the real-time server uses the 4-streams-per-CTA form");
-    static_assert(!SPLIT || (FMT == FMT_F16 && NT == 1 && !DEFER), "the strict form: f16 pairs, one n8 tile, immediate head");
+    static_assert(!SPLIT || (FMT == FMT_F16 && !DEFER), "the strict form: f16 pairs, immediate head");
     constexpr int NP = SPLIT ? 2 : 1;                // operand parts (hi, lo')
     constexpr int SL = SPLIT ? 1 : 0;                // accumulators per tile: W_hi h_hi | (strict) W_hi h_lo' , W_lo' h_hi
     // PAIRCOL: strict form with four streams per CTA.  The odd column next to a stream's even column, dead in the rounded
@@ -70,10 +69,10 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
     // fragments, one head MMA (row 0 = w_hi, row 8 = w_lo': c0 + 2^-11 (c1 + c2)).  25 HMMAs per warp and step instead of 38.
     constexpr bool PAIRCOL = SPLIT && HALF;
     constexpr int NPB = PAIRCOL ? 1 : NP;            // parts of the state tile a thread loads B fragments from
-    constexpr int SC = HALF ? 4 : 8 * NT;            // streams per CTA
+    constexpr int SC = HALF ? 4 : 8;                 // streams per CTA
     constexpr int CS = HALF ? 2 : 1;                 // column stride of a stream
     constexpr int NE = HALF ? 1 : 2;                 // live columns per thread and n8 tile
-    using C = MmaCfg<FMT, NT, SPLIT>;
+    using C = MmaCfg<FMT, SPLIT>;
     using F = Frag<FMT, SPLIT>;
     constexpr int S = C::S, CH = C::CH, NK = F::NK, BW = F::BW;
     extern __shared__ __align__(128) uint8_t smem[];
@@ -199,9 +198,9 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
     // eight in registers (four SEL per step): 171.6 -> 168.1 ns/step at batch 1, cfg 3 181.7 -> 178.6.  With two CTAs per SM the
     // same change costs 8 % (215.7 -> 232.2 ns/step: one more shared-memory access per step in front of an HMMA), so the
     // immediate-head form keeps the selects (profiles/r02_mma_variants.txt).
-    auto head_mma_step = [&](const uint8_t* tile, int nt, const uint32_t (&bp)[NPB][BW], float (&c)[4]) {
+    auto head_mma_step = [&](const uint8_t* tile, const uint32_t (&bp)[NPB][BW], float (&c)[4]) {
         if (DEFER && HK == 1 && NPB == 1 && !SPLIT) {
-            const uint2 w2 = *reinterpret_cast<const uint2*>(tile + (nt * 8 + gid) * F::ROW_BYTES + tig * 32 + warp * 8);
+            const uint2 w2 = *reinterpret_cast<const uint2*>(tile + gid * F::ROW_BYTES + tig * 32 + warp * 8);
             c[0] = c[1] = c[2] = c[3] = 0.0f;
             mma_sync<FMT>(c, ahead[0], w2.x, w2.y);
         } else {
@@ -213,13 +212,13 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         if (PAIRCOL) return make_float2(fmaf(SPLIT_INV, c[1] + c[2], c[0]), 0.0f);
         return SPLIT ? make_float2(fmaf(SPLIT_INV, c[2], c[0]), fmaf(SPLIT_INV, c[3], c[1])) : make_float2(c[0] + c[2], c[1] + c[3]);
     };
-    auto load_bfrag = [&](const uint8_t* tile, int nt, uint32_t (&bp)[NPB][BW]) {
+    auto load_bfrag = [&](const uint8_t* tile, uint32_t (&bp)[NPB][BW]) {
         // f16/bf16: the thread's 16 elements are contiguous (2 vectors); tf32: vector q holds elements
         // q*16 + tig*4 .. +3 (4 vectors, a quarter-warp reads 64 contiguous bytes); strict form: the lo' part of the row
         // follows the hi part
 #pragma unroll
         for (int part = 0; part < NPB; ++part) {
-            const uint8_t* src = tile + (nt * 8 + gid) * F::ROW_BYTES + part * F::PART_BYTES + (FMT == FMT_TF32 ? tig * 16 : tig * 32);
+            const uint8_t* src = tile + gid * F::ROW_BYTES + part * F::PART_BYTES + (FMT == FMT_TF32 ? tig * 16 : tig * 32);
 #pragma unroll
             for (int q = 0; q < BW / 4; ++q) {
                 const uint4 v = *reinterpret_cast<const uint4*>(src + q * (FMT == FMT_TF32 ? 64 : 16));
@@ -282,21 +281,19 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         }
     }
 
-    // ---- initial state: fp32 in registers (hst[nt][unit][stream]), rounded copy into state tile 0 ---------------
-    float hst[NT][2][2];
+    // ---- initial state: fp32 in registers (hst[unit][stream]), rounded copy into state tile 0 ---------------------
+    float hst[2][2];
 #pragma unroll
-    for (int nt = 0; nt < NT; ++nt)
+    for (int e = 0; e < 2; ++e) {
+        const int col = 2 * tig + e, s = col / CS;
+        const bool live = col % CS == 0 && s < ns;
 #pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            const int col = nt * 8 + 2 * tig + e, s = col / CS;
-            const bool live = col % CS == 0 && s < ns;
-#pragma unroll
-            for (int u = 0; u < 2; ++u) hst[nt][u][e] = (live && a.h_in) ? a.h_in[(b0 + s) * 64 + u0 + u] : 0.0f;
-            if (!PAIRCOL || e == 0) {
-                put_state(hb, col, hst[nt][0][e], hst[nt][1][e]);
-                put_state(hb + C::HB_BYTES, col, 0.0f, 0.0f);                                    // dead columns stay finite
-            }
+        for (int u = 0; u < 2; ++u) hst[u][e] = (live && a.h_in) ? a.h_in[(b0 + s) * 64 + u0 + u] : 0.0f;
+        if (!PAIRCOL || e == 0) {
+            put_state(hb, col, hst[0][e], hst[1][e]);
+            put_state(hb + C::HB_BYTES, col, 0.0f, 0.0f);                                    // dead columns stay finite
         }
+    }
     const long long nchunks = (a.T + CH - 1) / CH;
     int cur = 0;
     unsigned rt_seen = 0;
@@ -349,36 +346,33 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
             if (use_ring) load_d(xb ^ 1, t0 + CH);
         }
 
-        float hpend[NT][4];
+        float hpend[4];
         for (int tt = 0; tt < n; ++tt) {
             const uint8_t* hcur = hb + cur * C::HB_BYTES;
             uint8_t* hnext = hb + (cur ^ 1) * C::HB_BYTES;
-            float acc[NT][3][4];
-            float accs[SPLIT ? NT : 1][3][SPLIT ? 2 : 1][4];      // strict form: W_hi h_lo' and W_lo' h_hi (scaled by 2^11)
-            uint32_t breg[NT][NPB][BW];
+            float acc[3][4];
+            float accs[3][SPLIT ? 2 : 1][4];      // strict form: W_hi h_lo' and W_lo' h_hi (scaled by 2^11)
+            uint32_t breg[NPB][BW];
+            load_bfrag(hcur, breg);
 #pragma unroll
-            for (int nt = 0; nt < NT; ++nt) {
-                load_bfrag(hcur, nt, breg[nt]);
+            for (int tile = 0; tile < 3; ++tile) {
+                acc[tile][0] = acc[tile][1] = acc[tile][2] = acc[tile][3] = 0.0f;
+                if (SPLIT)
 #pragma unroll
-                for (int tile = 0; tile < 3; ++tile) {
-                    acc[nt][tile][0] = acc[nt][tile][1] = acc[nt][tile][2] = acc[nt][tile][3] = 0.0f;
-                    if (SPLIT)
+                    for (int i = 0; i < 4; ++i) accs[tile][0][i] = accs[tile][SL][i] = 0.0f;
+            }
+            if (!HALF) {
+                // throughput form: input projection and biases enter through the accumulators (fewer FP32 instructions
+                // after the MMAs: 976 vs 1027 ns/step at 8192 streams; the 4-stream latency form measured slower with it)
+                const float2 xi = *reinterpret_cast<const float2*>(xcur + tt * S + 2 * tig);
 #pragma unroll
-                        for (int i = 0; i < 4; ++i) accs[nt][tile][0][i] = accs[nt][tile][SL][i] = 0.0f;
-                }
-                if (!HALF) {
-                    // throughput form: input projection and biases enter through the accumulators (fewer FP32 instructions
-                    // after the MMAs: 976 vs 1027 ns/step at 8192 streams; the 4-stream latency form measured slower with it)
-                    const float2 xi = *reinterpret_cast<const float2*>(xcur + tt * S + nt * 8 + 2 * tig);
+                for (int u = 0; u < 2; ++u)
 #pragma unroll
-                    for (int u = 0; u < 2; ++u)
-#pragma unroll
-                        for (int e = 0; e < NE; ++e) {
-                            acc[nt][0][2 * u + e] = fmaf(uc[u].cr_w, e ? xi.y : xi.x, uc[u].cr_b);
-                            acc[nt][1][2 * u + e] = fmaf(uc[u].cz_w, e ? xi.y : xi.x, uc[u].cz_b);
-                            acc[nt][2][2 * u + e] = uc[u].ch_b;
-                        }
-                }
+                    for (int e = 0; e < NE; ++e) {
+                        acc[0][2 * u + e] = fmaf(uc[u].cr_w, e ? xi.y : xi.x, uc[u].cr_b);
+                        acc[1][2 * u + e] = fmaf(uc[u].cz_w, e ? xi.y : xi.x, uc[u].cz_b);
+                        acc[2][2 * u + e] = uc[u].ch_b;
+                    }
             }
             // critical path first: r -> n -> h' is the dependent chain of the step, z only enters the final blend.  The r and
             // n tiles alternate (two dependent accumulator chains keep the pipe busy), the z tile follows and overlaps r's
@@ -387,14 +381,11 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
             // Strict form: three independent accumulator chains per tile (hi.hi, hi.lo', lo'.hi), issued r, n, then z; the
             // scaled chains are folded into the main accumulator once all MMAs are in flight.
             auto tile_mmas = [&](int tile, int ks) {
-#pragma unroll
-                for (int nt = 0; nt < NT; ++nt) {
-                    mma_sync<FMT>(acc[nt][tile], areg[0][tile][ks], breg[nt][0][2 * ks], breg[nt][0][2 * ks + 1]);
-                    if (SPLIT) {
-                        if (!PAIRCOL)
-                            mma_sync<FMT>(accs[nt][tile][0], areg[0][tile][ks], breg[nt][NPB - 1][2 * ks], breg[nt][NPB - 1][2 * ks + 1]);
-                        mma_sync<FMT>(accs[nt][tile][SL], areg[NP - 1][tile][ks], breg[nt][0][2 * ks], breg[nt][0][2 * ks + 1]);
-                    }
+                mma_sync<FMT>(acc[tile], areg[0][tile][ks], breg[0][2 * ks], breg[0][2 * ks + 1]);
+                if (SPLIT) {
+                    if (!PAIRCOL)
+                        mma_sync<FMT>(accs[tile][0], areg[0][tile][ks], breg[NPB - 1][2 * ks], breg[NPB - 1][2 * ks + 1]);
+                    mma_sync<FMT>(accs[tile][SL], areg[NP - 1][tile][ks], breg[0][2 * ks], breg[0][2 * ks + 1]);
                 }
             };
             {
@@ -413,103 +404,94 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
             // per SM sub-partition.  With two or more warps per sub-partition that stall is hidden by the other warps and
             // the compact 12-HMMA burst of the deferred form collides on the tensor pipe instead (221 -> 232 ns/step at
             // 1024 streams, 948 -> 1000 at 8192), so the immediate form stays there.
-#pragma unroll
-            for (int nt = 0; nt < NT; ++nt) {
-                if (DEFER) {
-                    if (tt > 1 && gid == 0)
-                        *reinterpret_cast<float2*>(yp + (warp * CH + tt - 2) * C::YP_LD + nt * 8 + 2 * tig) = head_value(hpend[nt]);
-                    head_mma_step(hcur, nt, breg[nt], hpend[nt]);
-                } else {
-                    float ch[4];
-                    head_mma_step(hcur, nt, breg[nt], ch);
-                    if (tt > 0 && gid == 0)
-                        *reinterpret_cast<float2*>(yp + (warp * CH + tt - 1) * C::YP_LD + nt * 8 + 2 * tig) = head_value(ch);
-                }
+            if (DEFER) {
+                if (tt > 1 && gid == 0)
+                    *reinterpret_cast<float2*>(yp + (warp * CH + tt - 2) * C::YP_LD + 2 * tig) = head_value(hpend);
+                head_mma_step(hcur, breg, hpend);
+            } else {
+                float ch[4];
+                head_mma_step(hcur, breg, ch);
+                if (tt > 0 && gid == 0)
+                    *reinterpret_cast<float2*>(yp + (warp * CH + tt - 1) * C::YP_LD + 2 * tig) = head_value(ch);
             }
             // ---- gates, state blend, rounded state for the next step, head partials ------------------------------
+            const float2 xv = *reinterpret_cast<const float2*>(xcur + tt * S + 2 * tig);
+            float z[2][2], dn[2][2], hn[2][2];
+            if (SPLIT) {                       // fold the scaled chains: W h = hi.hi + 2^-11 (hi.lo' + lo'.hi)
 #pragma unroll
-            for (int nt = 0; nt < NT; ++nt) {
-                const float2 xv = *reinterpret_cast<const float2*>(xcur + tt * S + nt * 8 + 2 * tig);
-                float z[2][2], dn[2][2], hn[2][2];
-                if (SPLIT) {                       // fold the scaled chains: W h = hi.hi + 2^-11 (hi.lo' + lo'.hi)
+                for (int tile = 0; tile < 3; ++tile)
 #pragma unroll
-                    for (int tile = 0; tile < 3; ++tile)
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-                            if (PAIRCOL) {             // W_hi h_lo' sits in the odd column of the main accumulator
-                                if ((i & 1) == 0)
-                                    acc[nt][tile][i] = fmaf(SPLIT_INV, acc[nt][tile][i + 1] + accs[nt][tile][SL][i], acc[nt][tile][i]);
-                            } else if (!HALF || (i & 1) == 0) {
-                                acc[nt][tile][i] = fmaf(SPLIT_INV, accs[nt][tile][0][i] + accs[nt][tile][SL][i], acc[nt][tile][i]);
-                            }
-                }
-                if (SPLIT) {                       // strict activations (gates.cuh), nothing shared between pairs
-#pragma unroll
-                    for (int u = 0; u < 2; ++u)
-#pragma unroll
-                        for (int e = 0; e < NE; ++e) {
-                            const float xx = e ? xv.y : xv.x;
-                            float pr = acc[nt][0][2 * u + e], pz = acc[nt][1][2 * u + e], ahn = acc[nt][2][2 * u + e];
-                            if (HALF) {            // (non-HALF: the accumulators already hold W_i x + b for r, z and b_hn for n)
-                                pr += fmaf(uc[u].cr_w, xx, uc[u].cr_b);
-                                pz += fmaf(uc[u].cz_w, xx, uc[u].cz_b);
-                                ahn += uc[u].ch_b;
-                            }
-                            hn[u][e] = gates_strict(pr, pz, ahn, fmaf(uc[u].cn_w, xx, uc[u].cn_b), hst[nt][u][e]);
+                    for (int i = 0; i < 4; ++i)
+                        if (PAIRCOL) {             // W_hi h_lo' sits in the odd column of the main accumulator
+                            if ((i & 1) == 0)
+                                acc[tile][i] = fmaf(SPLIT_INV, acc[tile][i + 1] + accs[tile][SL][i], acc[tile][i]);
+                        } else if (!HALF || (i & 1) == 0) {
+                            acc[tile][i] = fmaf(SPLIT_INV, accs[tile][0][i] + accs[tile][SL][i], acc[tile][i]);
                         }
-                }
+            }
+            if (SPLIT) {                       // strict activations (gates.cuh), nothing shared between pairs
 #pragma unroll
                 for (int u = 0; u < 2; ++u)
 #pragma unroll
-                    for (int e = 0; e < (SPLIT ? 0 : NE); ++e) {
-                        // r has its own reciprocal at every width: sharing 1/(d_r d_z) (4.5 instead of 5.5 MUFU per pair)
-                        // measured slower even in the throughput regime (1052 vs 1030 ns/step at 8192 streams)
+                    for (int e = 0; e < NE; ++e) {
                         const float xx = e ? xv.y : xv.x;
-                        if (HALF) {
-                            gates_rz_dn_fast_r(uc[u], acc[nt][0][2 * u + e], acc[nt][1][2 * u + e], acc[nt][2][2 * u + e], xx,
-                                               z[u][e], dn[u][e]);
-                        } else {                   // accumulators already hold W_i x + b (r, z) and b_hn (n)
-                            const float r = rcp_approx(1.0f + ex2_approx(acc[nt][0][2 * u + e]));
-                            dn[u][e] = 1.0f + ex2_approx(fminf(fmaf(r, acc[nt][2][2 * u + e], fmaf(uc[u].cn_w, xx, uc[u].cn_b)), EX2_CLAMP));
-                            z[u][e] = rcp_approx(1.0f + ex2_approx(acc[nt][1][2 * u + e]));
+                        float pr = acc[0][2 * u + e], pz = acc[1][2 * u + e], ahn = acc[2][2 * u + e];
+                        if (HALF) {            // (non-HALF: the accumulators already hold W_i x + b for r, z and b_hn for n)
+                            pr += fmaf(uc[u].cr_w, xx, uc[u].cr_b);
+                            pz += fmaf(uc[u].cz_w, xx, uc[u].cz_b);
+                            ahn += uc[u].ch_b;
                         }
+                        hn[u][e] = gates_strict(pr, pz, ahn, fmaf(uc[u].cn_w, xx, uc[u].cn_b), hst[u][e]);
                     }
+            }
+#pragma unroll
+            for (int u = 0; u < 2; ++u)
 #pragma unroll
                 for (int e = 0; e < (SPLIT ? 0 : NE); ++e) {
-                    if (HALF) {                    // own n-gate reciprocals, shorter dependent chain (sharing them between the two
-                                                   // units measured 227.3 vs 221.5 ns/step even with two CTAs per SM)
-                        // `_late`: everything that does not depend on the n gate's reciprocal is evaluated in front of it, one
-                        // FMA behind the step's last MUFU instead of three (221.7 -> 215.6 ns/step at 1024 streams, 176.9 ->
-                        // 171.6 at batch 1, profiles/r02_mma_variants.txt)
-                        hn[0][e] = gates_blend1_late(z[0][e], dn[0][e], hst[nt][0][e]);
-                        hn[1][e] = gates_blend1_late(z[1][e], dn[1][e], hst[nt][1][e]);
-                    } else {                       // the two hidden units of one stream share the n-gate reciprocal
-                        gates_blend2(z[0][e], dn[0][e], hst[nt][0][e], z[1][e], dn[1][e], hst[nt][1][e], hn[0][e], hn[1][e]);
+                    // r has its own reciprocal at every width: sharing 1/(d_r d_z) (4.5 instead of 5.5 MUFU per pair)
+                    // measured slower even in the throughput regime (1052 vs 1030 ns/step at 8192 streams)
+                    const float xx = e ? xv.y : xv.x;
+                    if (HALF) {
+                        gates_rz_dn_fast_r(uc[u], acc[0][2 * u + e], acc[1][2 * u + e], acc[2][2 * u + e], xx,
+                                           z[u][e], dn[u][e]);
+                    } else {                   // accumulators already hold W_i x + b (r, z) and b_hn (n)
+                        const float r = rcp_approx(1.0f + ex2_approx(acc[0][2 * u + e]));
+                        dn[u][e] = 1.0f + ex2_approx(fminf(fmaf(r, acc[2][2 * u + e], fmaf(uc[u].cn_w, xx, uc[u].cn_b)), EX2_CLAMP));
+                        z[u][e] = rcp_approx(1.0f + ex2_approx(acc[1][2 * u + e]));
                     }
                 }
 #pragma unroll
-                for (int e = 0; e < NE; ++e) {
-                    hst[nt][0][e] = hn[0][e];
-                    hst[nt][1][e] = hn[1][e];
-                    put_state(hnext, nt * 8 + 2 * tig + e, hn[0][e], hn[1][e]);
+            for (int e = 0; e < (SPLIT ? 0 : NE); ++e) {
+                if (HALF) {                    // own n-gate reciprocals, shorter dependent chain (sharing them between the two
+                                               // units measured 227.3 vs 221.5 ns/step even with two CTAs per SM)
+                    // `_late`: everything that does not depend on the n gate's reciprocal is evaluated in front of it, one
+                    // FMA behind the step's last MUFU instead of three (221.7 -> 215.6 ns/step at 1024 streams, 176.9 ->
+                    // 171.6 at batch 1, profiles/r02_mma_variants.txt)
+                    hn[0][e] = gates_blend1_late(z[0][e], dn[0][e], hst[0][e]);
+                    hn[1][e] = gates_blend1_late(z[1][e], dn[1][e], hst[1][e]);
+                } else {                       // the two hidden units of one stream share the n-gate reciprocal
+                    gates_blend2(z[0][e], dn[0][e], hst[0][e], z[1][e], dn[1][e], hst[1][e], hn[0][e], hn[1][e]);
                 }
+            }
+#pragma unroll
+            for (int e = 0; e < NE; ++e) {
+                hst[0][e] = hn[0][e];
+                hst[1][e] = hn[1][e];
+                put_state(hnext, 2 * tig + e, hn[0][e], hn[1][e]);
             }
             cur ^= 1;
             __syncthreads();                   // next state tile published; all reads of the old one are done
         }
 
         if (n > 0) {                           // head of the chunk's last step: one more MMA on the final state tile
-#pragma unroll
-            for (int nt = 0; nt < NT; ++nt) {
-                if (DEFER && n > 1 && gid == 0) // (the pending head of the step before it)
-                    *reinterpret_cast<float2*>(yp + (warp * CH + n - 2) * C::YP_LD + nt * 8 + 2 * tig) = head_value(hpend[nt]);
-                uint32_t bfin[NPB][BW];
-                float ch[4];
-                load_bfrag(hb + cur * C::HB_BYTES, nt, bfin);
-                head_mma(bfin, ch);
-                if (gid == 0)
-                    *reinterpret_cast<float2*>(yp + (warp * CH + n - 1) * C::YP_LD + nt * 8 + 2 * tig) = head_value(ch);
-            }
+            if (DEFER && n > 1 && gid == 0)    // (the pending head of the step before it)
+                *reinterpret_cast<float2*>(yp + (warp * CH + n - 2) * C::YP_LD + 2 * tig) = head_value(hpend);
+            uint32_t bfin[NPB][BW];
+            float ch[4];
+            load_bfrag(hb + cur * C::HB_BYTES, bfin);
+            head_mma(bfin, ch);
+            if (gid == 0)
+                *reinterpret_cast<float2*>(yp + (warp * CH + n - 1) * C::YP_LD + 2 * tig) = head_value(ch);
             __syncthreads();
         }
         // ---- flush the chunk: y = sum of the four warps' partials + bias (+ x) ------------------------------------
@@ -570,14 +552,12 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
 
     // ---- final state; rolled delay history (code/model.py:314-315) -------------------------------------------------
 #pragma unroll
-    for (int nt = 0; nt < NT; ++nt)
+    for (int u = 0; u < 2; ++u)
 #pragma unroll
-        for (int u = 0; u < 2; ++u)
-#pragma unroll
-            for (int e = 0; e < NE; ++e) {
-                const int s = (nt * 8 + 2 * tig + e) / CS;
-                if (s < ns) a.h_out[(b0 + s) * 64 + u0 + u] = hst[nt][u][e];
-            }
+        for (int e = 0; e < NE; ++e) {
+            const int s = (2 * tig + e) / CS;
+            if (s < ns) a.h_out[(b0 + s) * 64 + u0 + u] = hst[u][e];
+        }
     if (delay) {
         __syncthreads();
         for (long long idx = tid; idx < (long long)ns * a.D; idx += 128) {
@@ -590,16 +570,13 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
     }
 }
 
-template <int FMT, int NT, bool HALF, bool DEFER = false, bool SPLIT = false>
+template <int FMT, bool HALF, bool DEFER = false, bool SPLIT = false>
 cudaError_t launch_mma_one(const GruArgs& a, cudaStream_t st)
 {
-    if (HALF && !DEFER && !SPLIT) {        // one CTA per SM at most: the deferred-head form
-        if (a.sm_count > 0 && (a.B + 3) / 4 <= a.sm_count) return launch_mma_one<FMT, NT, HALF, HALF>(a, st);
-    }
-    using C = MmaCfg<FMT, NT, SPLIT>;
+    using C = MmaCfg<FMT, SPLIT>;
     static OncePerDevice once;
     cudaError_t e = once.run([] {
-        return cudaFuncSetAttribute(gru_mma_kernel<FMT, NT, HALF, false, DEFER, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        return cudaFuncSetAttribute(gru_mma_kernel<FMT, HALF, false, DEFER, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     C::SMEM_BYTES + 48 * 1024);
     });
     if (e != cudaSuccess) return e;
@@ -618,7 +595,7 @@ cudaError_t launch_mma_one(const GruArgs& a, cudaStream_t st)
             smem_bytes += (int)(rl * SC * 4);
         }
     }
-    gru_mma_kernel<FMT, NT, HALF, false, DEFER, SPLIT><<<(unsigned)grid, 128, smem_bytes, st>>>(b);
+    gru_mma_kernel<FMT, HALF, false, DEFER, SPLIT><<<(unsigned)grid, 128, smem_bytes, st>>>(b);
     ++g_launches;
     return cudaGetLastError();
 }
@@ -626,37 +603,37 @@ cudaError_t launch_mma_one(const GruArgs& a, cudaStream_t st)
 template <int FMT, bool SPLIT = false>
 cudaError_t launch_mma_rt_fmt(const GruArgs& a, cudaStream_t st)
 {
-    using C = MmaCfg<FMT, 1, SPLIT>;
-    cudaError_t e = cudaFuncSetAttribute(gru_mma_kernel<FMT, 1, true, true, !SPLIT, SPLIT>,
+    using C = MmaCfg<FMT, SPLIT>;
+    cudaError_t e = cudaFuncSetAttribute(gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
     if (e != cudaSuccess) return e;
-    gru_mma_kernel<FMT, 1, true, true, !SPLIT, SPLIT><<<1, 128, C::SMEM_BYTES, st>>>(a);
+    gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT><<<1, 128, C::SMEM_BYTES, st>>>(a);
     ++g_launches;
     return cudaGetLastError();
 }
 
 template <int FMT>
-cudaError_t launch_mma_fmt(const GruArgs& a, int nt, cudaStream_t st)
+cudaError_t launch_mma_fmt(const GruArgs& a, int streams, bool defer_head, cudaStream_t st)
 {
-    if (nt >= 2) return launch_mma_one<FMT, 2, false>(a, st);
-    if (nt <= 0) return launch_mma_one<FMT, 1, true>(a, st);
-    return launch_mma_one<FMT, 1, false>(a, st);
+    if (streams == 8) return launch_mma_one<FMT, false>(a, st);
+    return defer_head ? launch_mma_one<FMT, true, true>(a, st) : launch_mma_one<FMT, true>(a, st);
 }
 
 }  // namespace
 
-// fmt: FMT_F16 / FMT_BF16 / FMT_TF32 / FMT_F16X3 (strict: f16 hi/lo pairs, three MMAs per product).  n_tiles: 8-stream
-// tiles per CTA (1 or 2; the strict form has 1); 0 = four streams per CTA (HALF).
-cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int n_tiles, cudaStream_t st)
+// fmt: FMT_F16 / FMT_BF16 / FMT_TF32 / FMT_F16X3 (strict: f16 hi/lo pairs, three MMAs per product).  streams: streams per CTA,
+// 4 (HALF) or 8.  defer_head: the deferred-head form of the 4-stream kernel (rounded modes only; see DEFER).
+cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_head, cudaStream_t st)
 {
     if (a.B <= 0 || a.T <= 0) return cudaSuccess;
+    if (streams != 4 && streams != 8) return cudaErrorInvalidValue;
     switch (fmt) {
         case FMT_F16X3:
-            return n_tiles <= 0 ? launch_mma_one<FMT_F16, 1, true, false, true>(a, st)
-                                : launch_mma_one<FMT_F16, 1, false, false, true>(a, st);
-        case FMT_TF32: return launch_mma_fmt<FMT_TF32>(a, n_tiles, st);
-        case FMT_BF16: return launch_mma_fmt<FMT_BF16>(a, n_tiles, st);
-        default: return launch_mma_fmt<FMT_F16>(a, n_tiles, st);
+            return streams == 4 ? launch_mma_one<FMT_F16, true, false, true>(a, st)
+                                : launch_mma_one<FMT_F16, false, false, true>(a, st);
+        case FMT_TF32: return launch_mma_fmt<FMT_TF32>(a, streams, defer_head, st);
+        case FMT_BF16: return launch_mma_fmt<FMT_BF16>(a, streams, defer_head, st);
+        default: return launch_mma_fmt<FMT_F16>(a, streams, defer_head, st);
     }
 }
 

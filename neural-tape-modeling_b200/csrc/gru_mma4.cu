@@ -35,23 +35,17 @@ using namespace mmaf;
 namespace {
 
 constexpr float LOG2E_F4 = 1.4426950408889634f;
-#ifndef NTM_MMA4_CH
-#define NTM_MMA4_CH 128          // steps per staged chunk (A/B knob, tools/ab_build.py)
-#endif
-#ifndef NTM_MMA4_XPAD
-#define NTM_MMA4_XPAD 8          // padding of a staged x row in floats (A/B knob)
-#endif
-#ifndef NTM_MMA4_YPAD
-#define NTM_MMA4_YPAD 4          // padding of a head-partial row in floats, >= 4 (A/B knob)
-#endif
+constexpr int MMA4_CH = 128;         // steps per staged chunk
+constexpr int MMA4_XPAD = 8;         // padding of a staged x row in floats
+constexpr int MMA4_YPAD = 4;         // padding of a head-partial row in floats, >= 4
 
 template <int FMT>
 struct Mma4Cfg {
     using F = Frag<FMT, false>;
     static constexpr int SC = 4;                     // streams per CTA (columns 0, 2, 4, 6 of the n8 tile)
-    static constexpr int CH = NTM_MMA4_CH;           // steps per staged chunk
-    static constexpr int XLD = CH + NTM_MMA4_XPAD;   // staged x row of one stream
-    static constexpr int YLD = CH + NTM_MMA4_YPAD;   // head partials of one (warp, stream): position p holds sample p - 1
+    static constexpr int CH = MMA4_CH;               // steps per staged chunk
+    static constexpr int XLD = CH + MMA4_XPAD;       // staged x row of one stream
+    static constexpr int YLD = CH + MMA4_YPAD;       // head partials of one (warp, stream): position p holds sample p - 1
     static constexpr int TILE_BYTES = 8 * F::ROW_BYTES;
     static constexpr int OFF_HB = 0;                                         // [2][8][ROW_BYTES]
     static constexpr int OFF_XS = (2 * TILE_BYTES + 127) / 128 * 128;        // [2][SC][CH] floats

@@ -51,14 +51,6 @@ constexpr uint32_t TS_SBO = 128, TS_LBO = (TS_N / 8) * 128;       // K-major, no
 constexpr int TS_UG = 8;                   // hidden units per TMEM load group
 constexpr int TS_UW = 2;                   // threads per stream
 constexpr float TS_LO_SCALE = 256.0f;      // strict form: h_lo' = (h - h_hi) * 2^8
-#ifndef NTM_TCS_STRICT_OWN_RCP
-// strict form: 1 = every gate its own reciprocal, 0 = r/z of a unit and n of two units share one.  Measured (profiles/
-// r02_strict_tcs_variants.txt): own reciprocals change NOTHING in the achieved error (cfg-1 pulse train, the one chaotic
-// golden signal: 3.3e-5 either way) and cost 16 % (9.18 vs 10.96 Gsamples/s at 37 888 streams) -- sharing stays.
-#define NTM_TCS_STRICT_OWN_RCP 0
-#endif
-constexpr int TCS_DEFAULT_VAR = 15;        // staggered tiles + r/z reciprocal shared by two units + packed fp32 arithmetic + n reciprocal
-                                           // shared by four units (the last only where the K augmentation exists: f16, bf16)
 
 template <int FMT>
 struct TsFmt {
@@ -74,18 +66,6 @@ struct TsFmt {
     static constexpr uint32_t OFF_YP = OFF_BAR + 64;           // [2 tiles][2][128] floats
     static constexpr uint32_t SMEM_BYTES = OFF_YP + 2 * 2 * 128 * 4;
 };
-
-#ifdef NTM_TCS_TRACE
-// debug build only (NTM_EXTRA_NVCC_FLAGS=-DNTM_TCS_TRACE): per-step clock stamps of CTA 0, [tile][step][start, mid, end]
-__device__ long long g_tcs_trace[2 * 256 * 3];
-#define TCS_STAMP(slot)                                                                          \
-    do {                                                                                         \
-        if (blockIdx.x == 0 && lane == 0 && wq == 0 && UH == 0 && t >= 64 && t < 64 + 256)       \
-            g_tcs_trace[(tile * 256 + (int)(t - 64)) * 3 + (slot)] = clock64();                  \
-    } while (0)
-#else
-#define TCS_STAMP(slot) do {} while (0)
-#endif
 
 // dynamic schedule of one launch (all null / 0: static)
 struct TcsSched {
@@ -124,102 +104,59 @@ __device__ __forceinline__ void tmem_st2(uint32_t taddr, uint32_t r0, uint32_t r
 // New states of the two hidden units (j, j + 1) of one stream from their accumulator values.
 //   AUG formats: ar, az are complete scaled pre-activations, an = W_hn h + b_hn.
 //   others:      ar, az, an = (gain x) W_h* h; input projection and biases are added here in fp32.
-// SHARE4: one reciprocal serves r and z of BOTH units (4.0 MUFU per unit-step; ex2 arguments of r, z clamped to 30 so the
-// product of four denominators stays finite: sigmoid saturates at 2^-30); STRICT: Newton-refined reciprocals.
-template <int FMT, bool SHARE4, bool PACK2>
+// Non-strict formats: one reciprocal serves r and z of BOTH units (4.0 MUFU per unit-step; ex2 arguments of r, z clamped to
+// 30 so the product of four denominators stays finite: sigmoid saturates at 2^-30).  STRICT: Newton-refined reciprocals, one
+// shared only between the r and z gate of ONE unit (a product of four denominators carries three more roundings into every
+// gate value); every gate its own reciprocal changed nothing in the achieved error and cost 16 % (9.18 vs 10.96 Gsamples/s at
+// 37 888 streams, profiles/r02_strict_tcs_variants.txt).  The n gates of the pair share one reciprocal in every format.
+template <int FMT>
 __device__ __forceinline__ void tcs_gate_pair(const TcsConsts& kc, int j, float x, float ar0, float ar1, float az0, float az1,
                                               float an0, float an1, float& h0, float& h1, float& ys)
 {
     using F = TsFmt<FMT>;
+    constexpr bool SHARE4 = !F::STRICT;
     constexpr float C = SHARE4 ? 30.0f : EX2_CLAMP;
     auto rcp_f = [](float d) { return F::STRICT ? rcp_strict(d) : rcp_approx(d); };
-    if (PACK2) {
-        const f32x2 one = pk(1.0f, 1.0f), x2 = pk(x, x);
-        f32x2 pr = pk(ar0, ar1), pz = pk(az0, az1), ahn = pk(an0, an1);
-        if (!F::AUG) {
-            const f32x2 gi = pk(kc.gain_inv, kc.gain_inv);
-            const f32x2 ir = fma2(pk(kc.cr_w[j], kc.cr_w[j + 1]), x2, pk(kc.cr_b[j], kc.cr_b[j + 1]));
-            const f32x2 iz = fma2(pk(kc.cz_w[j], kc.cz_w[j + 1]), x2, pk(kc.cz_b[j], kc.cz_b[j + 1]));
-            const f32x2 hb = pk(kc.ch_b[j], kc.ch_b[j + 1]);
-            if (F::STRICT) { pr = fma2(pr, gi, ir); pz = fma2(pz, gi, iz); ahn = fma2(ahn, gi, hb); }
-            else { pr = add2(pr, ir); pz = add2(pz, iz); ahn = add2(ahn, hb); }
-        }
-        float r0, r1, z0, z1;
-        upk(pr, r0, r1);
-        upk(pz, z0, z1);
-        const f32x2 dr = add2(pk(ex2_approx(fminf(r0, C)), ex2_approx(fminf(r1, C))), one);
-        const f32x2 dz = add2(pk(ex2_approx(fminf(z0, C)), ex2_approx(fminf(z1, C))), one);
-        const f32x2 p = mul2(dr, dz);
-        float p0, p1;
-        upk(p, p0, p1);
-        f32x2 r, z;
-        if (F::STRICT && NTM_TCS_STRICT_OWN_RCP) {       // every gate its own Newton-refined reciprocal (as gates_strict)
-            float a0, a1, b0, b1;
-            upk(dr, a0, a1);
-            upk(dz, b0, b1);
-            r = pk(rcp_f(a0), rcp_f(a1));
-            z = pk(rcp_f(b0), rcp_f(b1));
-        } else {
-            f32x2 inv;
-            if (SHARE4) {
-                const float q = rcp_f(p0 * p1);
-                inv = mul2(pk(p1, p0), pk(q, q));
-            } else {
-                inv = pk(rcp_f(p0), rcp_f(p1));
-            }
-            r = mul2(dz, inv);
-            z = mul2(dr, inv);
-        }
-        const f32x2 gin = fma2(pk(kc.cn_w[j], kc.cn_w[j + 1]), x2, pk(kc.cn_b[j], kc.cn_b[j + 1]));
-        float a0, a1;
-        upk(fma2(r, ahn, gin), a0, a1);
-        const f32x2 dn = add2(pk(ex2_approx(fminf(a0, EX2_CLAMP)), ex2_approx(fminf(a1, EX2_CLAMP))), one);
-        float d0, d1;
-        upk(dn, d0, d1);
-        f32x2 n;
-        if (F::STRICT && NTM_TCS_STRICT_OWN_RCP) {
-            n = fma2(pk(rcp_f(d0), rcp_f(d1)), pk(-2.0f, -2.0f), one);
-        } else {
-            const float qn = rcp_f(d0 * d1);
-            n = fma2(mul2(pk(d1, d0), pk(qn, qn)), pk(-2.0f, -2.0f), one);          // 1 - 2 / dn
-        }
-        const f32x2 h = pk(h0, h1);
-        const f32x2 hn = fma2(z, fma2(n, pk(-1.0f, -1.0f), h), n);                          // n + z (h - n)
-        upk(hn, h0, h1);
-        ys = fmaf(kc.wo[j], h0, ys);
-        ys = fmaf(kc.wo[j + 1], h1, ys);
-    } else {
-        if (!F::AUG) {
-            const float gi = F::STRICT ? kc.gain_inv : 1.0f;
-            ar0 = fmaf(ar0, gi, fmaf(kc.cr_w[j], x, kc.cr_b[j]));
-            ar1 = fmaf(ar1, gi, fmaf(kc.cr_w[j + 1], x, kc.cr_b[j + 1]));
-            az0 = fmaf(az0, gi, fmaf(kc.cz_w[j], x, kc.cz_b[j]));
-            az1 = fmaf(az1, gi, fmaf(kc.cz_w[j + 1], x, kc.cz_b[j + 1]));
-            an0 = fmaf(an0, gi, kc.ch_b[j]);
-            an1 = fmaf(an1, gi, kc.ch_b[j + 1]);
-        }
-        const float dr0 = 1.0f + ex2_approx(fminf(ar0, C)), dr1 = 1.0f + ex2_approx(fminf(ar1, C));
-        const float dz0 = 1.0f + ex2_approx(fminf(az0, C)), dz1 = 1.0f + ex2_approx(fminf(az1, C));
-        float r0, z0, r1, z1;
-        const float p0 = dr0 * dz0, p1 = dr1 * dz1;
-        if (SHARE4) {
-            const float q = rcp_f(p0 * p1);
-            const float i0 = p1 * q, i1 = p0 * q;
-            r0 = dz0 * i0; z0 = dr0 * i0; r1 = dz1 * i1; z1 = dr1 * i1;
-        } else {
-            const float i0 = rcp_f(p0), i1 = rcp_f(p1);
-            r0 = dz0 * i0; z0 = dr0 * i0; r1 = dz1 * i1; z1 = dr1 * i1;
-        }
-        const float g0 = fmaf(kc.cn_w[j], x, kc.cn_b[j]), g1 = fmaf(kc.cn_w[j + 1], x, kc.cn_b[j + 1]);
-        const float dn0 = 1.0f + ex2_approx(fminf(fmaf(r0, an0, g0), EX2_CLAMP));
-        const float dn1 = 1.0f + ex2_approx(fminf(fmaf(r1, an1, g1), EX2_CLAMP));
-        const float qn = rcp_f(dn0 * dn1);
-        const float n0 = fmaf(-2.0f, dn1 * qn, 1.0f), n1 = fmaf(-2.0f, dn0 * qn, 1.0f);
-        h0 = fmaf(z0, h0 - n0, n0);
-        h1 = fmaf(z1, h1 - n1, n1);
-        ys = fmaf(kc.wo[j], h0, ys);
-        ys = fmaf(kc.wo[j + 1], h1, ys);
+    const f32x2 one = pk(1.0f, 1.0f), x2 = pk(x, x);
+    f32x2 pr = pk(ar0, ar1), pz = pk(az0, az1), ahn = pk(an0, an1);
+    if (!F::AUG) {
+        const f32x2 gi = pk(kc.gain_inv, kc.gain_inv);
+        const f32x2 ir = fma2(pk(kc.cr_w[j], kc.cr_w[j + 1]), x2, pk(kc.cr_b[j], kc.cr_b[j + 1]));
+        const f32x2 iz = fma2(pk(kc.cz_w[j], kc.cz_w[j + 1]), x2, pk(kc.cz_b[j], kc.cz_b[j + 1]));
+        const f32x2 hb = pk(kc.ch_b[j], kc.ch_b[j + 1]);
+        if (F::STRICT) { pr = fma2(pr, gi, ir); pz = fma2(pz, gi, iz); ahn = fma2(ahn, gi, hb); }
+        else { pr = add2(pr, ir); pz = add2(pz, iz); ahn = add2(ahn, hb); }
     }
+    float r0, r1, z0, z1;
+    upk(pr, r0, r1);
+    upk(pz, z0, z1);
+    const f32x2 dr = add2(pk(ex2_approx(fminf(r0, C)), ex2_approx(fminf(r1, C))), one);
+    const f32x2 dz = add2(pk(ex2_approx(fminf(z0, C)), ex2_approx(fminf(z1, C))), one);
+    const f32x2 p = mul2(dr, dz);
+    float p0, p1;
+    upk(p, p0, p1);
+    f32x2 inv;
+    if (SHARE4) {
+        const float q = rcp_f(p0 * p1);
+        inv = mul2(pk(p1, p0), pk(q, q));
+    } else {
+        inv = pk(rcp_f(p0), rcp_f(p1));
+    }
+    const f32x2 r = mul2(dz, inv);
+    const f32x2 z = mul2(dr, inv);
+    const f32x2 gin = fma2(pk(kc.cn_w[j], kc.cn_w[j + 1]), x2, pk(kc.cn_b[j], kc.cn_b[j + 1]));
+    float a0, a1;
+    upk(fma2(r, ahn, gin), a0, a1);
+    const f32x2 dn = add2(pk(ex2_approx(fminf(a0, EX2_CLAMP)), ex2_approx(fminf(a1, EX2_CLAMP))), one);
+    float d0, d1;
+    upk(dn, d0, d1);
+    const float qn = rcp_f(d0 * d1);
+    const f32x2 n = fma2(mul2(pk(d1, d0), pk(qn, qn)), pk(-2.0f, -2.0f), one);          // 1 - 2 / dn
+    const f32x2 h = pk(h0, h1);
+    const f32x2 hn = fma2(z, fma2(n, pk(-1.0f, -1.0f), h), n);                          // n + z (h - n)
+    upk(hn, h0, h1);
+    ys = fmaf(kc.wo[j], h0, ys);
+    ys = fmaf(kc.wo[j + 1], h1, ys);
 }
 
 // FOUR hidden units (j .. j+3) of one stream, AUG formats, packed arithmetic: r and z of each pair share a reciprocal (as in
@@ -299,17 +236,17 @@ __device__ __forceinline__ void tcs_store_state(uint32_t t_op, int u0, int jl, c
 }
 
 // Gate math of one tile: one thread = one 32-unit slice (UH = 0, 1) of one stream.
-template <int FMT, int TILES, int VAR, int UH>
+template <int FMT, int TILES, int UH>
 __device__ __forceinline__ void tcs_epilogue(const GruArgs& a, const TcsConsts& kc, int tile, int wq, int lane, uint32_t tmem,
                                              uint64_t* bars, float* ypart, long long group, long long t0, int nsteps,
                                              long long base)
 {
     using F = TsFmt<FMT>;
-    // (the strict form shares a reciprocal only between the r and z gate of ONE unit: a product of four denominators
-    // carries three more roundings into every gate value)
-    constexpr bool STAGGER = (VAR & 1) != 0 && TILES == 2, SHARE4 = (VAR & 2) != 0 && !F::STRICT, PACK2 = (VAR & 4) != 0;
-    // bit 3: the n gates of four units share one reciprocal (3.75 MUFU per unit-step; formats with the K augmentation only)
-    constexpr bool QUAD = (VAR & 8) != 0 && F::AUG && SHARE4 && PACK2;
+    // two tiles per CTA run staggered: a tile may start a step's gate math only after the other tile passed the middle of its
+    // own -- keeps the two tiles of a CTA in anti-phase, see DESIGN.md 3.3
+    constexpr bool STAGGER = TILES == 2;
+    // the n gates of four units share one reciprocal (3.75 MUFU per unit-step; formats with the K augmentation only)
+    constexpr bool QUAD = F::AUG;
     constexpr int NU = 64 / TS_UW;               // hidden units per thread
     constexpr int NG = NU / TS_UG;               // TMEM load groups per thread and step
     constexpr int u0 = UH * NU;
@@ -360,7 +297,6 @@ __device__ __forceinline__ void tcs_epilogue(const GruArgs& a, const TcsConsts& 
         if (stagger && (tile == 1 || gt > 0)) mbar_wait_sleep(&bars[4 + (tile ^ 1)], (uint32_t)((gt - (tile == 0)) & 1));
         mbar_wait_sleep(&bars[2 + tile], (uint32_t)(gt & 1));
         tc_fence_after();
-        TCS_STAMP(0);
         if (UH == 0 && t > 0) {
             // the partner's head partial of the previous step (published before its h_ready arrive, which
             // happens-before the commit this thread just observed)
@@ -402,12 +338,11 @@ __device__ __forceinline__ void tcs_epilogue(const GruArgs& a, const TcsConsts& 
 #pragma unroll
             for (int p = 0; p < TS_UG / 2; ++p) {
                 const int jl = g * TS_UG + 2 * p;                      // local unit index; global = u0 + jl (static per UH)
-                tcs_gate_pair<FMT, SHARE4, PACK2>(kc, u0 + jl, x0, pre[0][2 * p], pre[0][2 * p + 1], pre[1][2 * p],
+                tcs_gate_pair<FMT>(kc, u0 + jl, x0, pre[0][2 * p], pre[0][2 * p + 1], pre[1][2 * p],
                                                   pre[1][2 * p + 1], pre[2][2 * p], pre[2][2 * p + 1], h[jl], h[jl + 1], ys[p & 1]);
             }
             }
             tcs_store_state<FMT>(t_op, u0, g * TS_UG, h);
-            if (g == NG / 2 - 1) TCS_STAMP(1);
             if (stagger && g == NG / 2 - 1) {
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&bars[4 + tile]);
@@ -424,7 +359,6 @@ __device__ __forceinline__ void tcs_epilogue(const GruArgs& a, const TcsConsts& 
         tc_fence_before();
         __syncwarp();
         if (lane == 0 && t + 1 < nsteps) mbar_arrive(&bars[tile]);
-        TCS_STAMP(2);
 
         yprev = v;                   // UH == 0: completed by the partner's partial at the next step
         xprev = x0;
@@ -443,10 +377,7 @@ __device__ __forceinline__ void tcs_epilogue(const GruArgs& a, const TcsConsts& 
     }
 }
 
-// VAR bit 0: staggered tiles (a tile may start a step's gate math only after the other tile passed the middle of its
-//            own -- keeps the two tiles of a CTA in anti-phase, see DESIGN.md 3.3); bit 1: reciprocal shared by two
-//            units (4.0 MUFU per unit-step); bit 2: packed fp32 arithmetic (FFMA2 / FMUL2 / FADD2).
-template <int FMT, int TILES, int VAR>
+template <int FMT, int TILES>
 __global__ void __launch_bounds__(32 * (4 * TS_UW + 1) * TILES, 1) gru_tcs_kernel(const GruArgs a, const __grid_constant__ TcsConsts kc, const TcsSched sc)
 {
     using F = TsFmt<FMT>;
@@ -555,9 +486,9 @@ __global__ void __launch_bounds__(32 * (4 * TS_UW + 1) * TILES, 1) gru_tcs_kerne
             const int tile = warp / (4 * TS_UW);
             const int wq = warp & 3;                 // TMEM lane quarter (== warp id % 4)
             if (((warp >> 2) & 1) == 0)
-                tcs_epilogue<FMT, TILES, VAR, 0>(a, kc, tile, wq, lane, tmem, bars, ypart, group, t0, nsteps, base);
+                tcs_epilogue<FMT, TILES, 0>(a, kc, tile, wq, lane, tmem, bars, ypart, group, t0, nsteps, base);
             else
-                tcs_epilogue<FMT, TILES, VAR, 1>(a, kc, tile, wq, lane, tmem, bars, ypart, group, t0, nsteps, base);
+                tcs_epilogue<FMT, TILES, 1>(a, kc, tile, wq, lane, tmem, bars, ypart, group, t0, nsteps, base);
         }
         base += nsteps;
 
@@ -577,23 +508,24 @@ __global__ void __launch_bounds__(32 * (4 * TS_UW + 1) * TILES, 1) gru_tcs_kerne
     if (warp == EPI_WARPS) tmem_dealloc(tmem, TMEM_COLS);
 }
 
-template <int FMT, int TILES, int VAR>
-cudaError_t launch_tcs_one(const GruArgs& a, const TcsConsts& kc, int sm_count, bool dynamic, cudaStream_t st)
+template <int FMT, int TILES>
+cudaError_t launch_tcs_one(const GruArgs& a, const TcsConsts& kc, int sm_count, bool static_schedule, cudaStream_t st)
 {
     using F = TsFmt<FMT>;
     static OncePerDevice once;
     cudaError_t e = once.run([] {
-        return cudaFuncSetAttribute(gru_tcs_kernel<FMT, TILES, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F::SMEM_BYTES);
+        return cudaFuncSetAttribute(gru_tcs_kernel<FMT, TILES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F::SMEM_BYTES);
     });
     if (e != cudaSuccess) return e;
     const long long per_group = (long long)TS_M * TILES;
     const long long groups = (a.B + per_group - 1) / per_group;
     TcsSched sc{};
     long long grid = groups;
-    // More groups than SMs and a partial last wave: pull (group, time chunk) jobs dynamically.  Chunk length: a job
+    // More groups than SMs and a partial last wave: pull (group, time chunk) jobs dynamically (unless the caller asks for the
+    // static schedule, the bit-exact reference of this one).  Chunk length: a job
     // costs ~7 steps of overhead (state round trip through L2, pipeline fill/drain; measured) and the tail idles half a
     // job per SM on average, so ct ~ sqrt(2 * 7 * T * groups / SMs), as a power of two in 64 .. 1024.
-    if (groups > sm_count && groups % sm_count != 0 && groups < (1ll << 30) && dynamic) {
+    if (groups > sm_count && groups % sm_count != 0 && groups < (1ll << 30) && !static_schedule) {
         const double ct = sqrt(14.0 * (double)a.T * (double)groups / (double)sm_count);
         long long p2 = 64;
         while (p2 * 1.41 <= ct && p2 < 1024) p2 *= 2;
@@ -611,7 +543,7 @@ cudaError_t launch_tcs_one(const GruArgs& a, const TcsConsts& kc, int sm_count, 
             grid = sm_count;
         }
     }
-    gru_tcs_kernel<FMT, TILES, VAR><<<(unsigned)grid, 32 * (4 * TS_UW + 1) * TILES, F::SMEM_BYTES, st>>>(a, kc, sc);
+    gru_tcs_kernel<FMT, TILES><<<(unsigned)grid, 32 * (4 * TS_UW + 1) * TILES, F::SMEM_BYTES, st>>>(a, kc, sc);
     ++g_launches;
     e = cudaGetLastError();
     if (sc.counter) {
@@ -622,13 +554,6 @@ cudaError_t launch_tcs_one(const GruArgs& a, const TcsConsts& kc, int sm_count, 
 }
 
 }  // namespace
-
-#ifdef NTM_TCS_TRACE
-extern "C" __attribute__((visibility("default"))) int ntm_debug_tcs_trace(long long* dst)
-{
-    return (int)cudaMemcpyFromSymbol(dst, g_tcs_trace, sizeof(long long) * 2 * 256 * 3);
-}
-#endif
 
 // host: the warp-uniform per-unit constants of the stream-major kernel, from the fp32 part of the blob
 void fill_tcs_consts(const float* blob_host, TcsConsts* kc)
@@ -721,28 +646,13 @@ void pack_tc_images(float* blob_host)
     }
 }
 
-namespace {
-
-template <int FMT, int TILES>
-cudaError_t launch_tcs_var(const GruArgs& a, const TcsConsts& kc, int var, int sm_count, cudaStream_t st)
-{
-    const bool dynamic = var < 0 || (var & 32) == 0;
-    if (var >= 0) var &= 31;
-    switch (var) {      // experiments: (var & 15) = VAR bits, (var & 32) = static schedule
-        case 3: return launch_tcs_one<FMT, TILES, 3>(a, kc, sm_count, dynamic, st);
-        case 7: if (FMT < 2) return launch_tcs_one<FMT < 2 ? FMT : 0, TILES, 7>(a, kc, sm_count, dynamic, st);      // (elsewhere 7 == 15)
-        default: return launch_tcs_one<FMT, TILES, TCS_DEFAULT_VAR>(a, kc, sm_count, dynamic, st);
-    }
-}
-
-}  // namespace
-
-// fmt: FMT_F16 / FMT_BF16 / FMT_TF32 / FMT_F16X3.  tiles: 128-stream tiles per CTA (1 or 2; 0 = automatic); var: kernel
-// variant (experiments; -1 = default).  DiffDelRNN batches (a.d != nullptr): the GRU + head pass writes pre_d, the delay
-// read runs as a second, HBM-bound pass over it (csrc/delay.cu: 12 bytes per sample at ~4.7 TB/s against ~75 ps per
-// sample of recurrent work: +3 %) -- the taps reach up to D samples back into other time chunks' output, which the
-// job-queue schedule of this kernel may still be producing on another SM.
-cudaError_t launch_gru_tcs(const GruArgs& a0, const TcsConsts& kc, int fmt, int sm_count, int tiles, int var, cudaStream_t st)
+// fmt: FMT_F16 / FMT_BF16 / FMT_TF32 / FMT_F16X3.  tiles: 128-stream tiles per CTA (1 or 2).  static_schedule: one CTA per
+// tile group for all T steps even where the job queue would run.  DiffDelRNN batches (a.d != nullptr): the GRU + head pass
+// writes pre_d, the delay read runs as a second, HBM-bound pass over it (csrc/delay.cu: 12 bytes per sample at ~4.7 TB/s
+// against ~75 ps per sample of recurrent work: +3 %) -- the taps reach up to D samples back into other time chunks' output,
+// which the job-queue schedule of this kernel may still be producing on another SM.
+cudaError_t launch_gru_tcs(const GruArgs& a0, const TcsConsts& kc, int fmt, int sm_count, int tiles, bool static_schedule,
+                           cudaStream_t st)
 {
     if (a0.B <= 0 || a0.T <= 0) return cudaSuccess;
     GruArgs a = a0;
@@ -751,14 +661,14 @@ cudaError_t launch_gru_tcs(const GruArgs& a0, const TcsConsts& kc, int fmt, int 
         a.y = a0.pre; a.ldy = a0.ldp;
         a.d = nullptr; a.pre = nullptr;
     }
-    // one tile per SM (time-multiplexed by the job queue) beats two resident tiles until ~190 streams per SM (measured)
-    if (tiles <= 0) tiles = a.B >= 190ll * sm_count ? 2 : 1;
+    const bool two = tiles == 2;
+    const bool ss = static_schedule;
     cudaError_t e;
     switch (fmt) {
-        case FMT_BF16: e = tiles >= 2 ? launch_tcs_var<FMT_BF16, 2>(a, kc, var, sm_count, st) : launch_tcs_var<FMT_BF16, 1>(a, kc, var, sm_count, st); break;
-        case FMT_TF32: e = tiles >= 2 ? launch_tcs_var<FMT_TF32, 2>(a, kc, var, sm_count, st) : launch_tcs_var<FMT_TF32, 1>(a, kc, var, sm_count, st); break;
-        case FMT_F16X3: e = tiles >= 2 ? launch_tcs_var<FMT_F16X3, 2>(a, kc, var, sm_count, st) : launch_tcs_var<FMT_F16X3, 1>(a, kc, var, sm_count, st); break;
-        default: e = tiles >= 2 ? launch_tcs_var<FMT_F16, 2>(a, kc, var, sm_count, st) : launch_tcs_var<FMT_F16, 1>(a, kc, var, sm_count, st); break;
+        case FMT_BF16: e = two ? launch_tcs_one<FMT_BF16, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_BF16, 1>(a, kc, sm_count, ss, st); break;
+        case FMT_TF32: e = two ? launch_tcs_one<FMT_TF32, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_TF32, 1>(a, kc, sm_count, ss, st); break;
+        case FMT_F16X3: e = two ? launch_tcs_one<FMT_F16X3, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_F16X3, 1>(a, kc, sm_count, ss, st); break;
+        default: e = two ? launch_tcs_one<FMT_F16, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_F16, 1>(a, kc, sm_count, ss, st); break;
     }
     if (e != cudaSuccess || !delay) return e;
     // pass 2: y = delay(pre_d, d) with the carried history (warm-up: y = pre_d, history still rolled)

@@ -88,10 +88,12 @@ struct TcsConsts {
 };
 
 // per-TU launchers -------------------------------------------------------------------------------
-cudaError_t launch_gru_fp32(const GruArgs& a, int sm_count, int tune_s, int tune_ks, int fast_act, cudaStream_t st);
-cudaError_t launch_gru_tcs(const GruArgs& a, const TcsConsts& kc, int fmt, int sm_count, int tiles, int var, cudaStream_t st);
+// The launchers run exactly the configuration they are given (capi.cu resolve_launch chooses it).
+cudaError_t launch_gru_fp32(const GruArgs& a, int streams, int ksplit, cudaStream_t st);
+cudaError_t launch_gru_tcs(const GruArgs& a, const TcsConsts& kc, int fmt, int sm_count, int tiles, bool static_schedule,
+                           cudaStream_t st);
 void fill_tcs_consts(const float* blob_host, TcsConsts* kc);
-cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int n_tiles, cudaStream_t st);
+cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_head, cudaStream_t st);
 cudaError_t launch_gru_mma4(const GruArgs& a, int fmt, cudaStream_t st);   // plain GRU, f16 / bf16, four streams per CTA, 4x unrolled
 cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st);    // resident real-time server, <= 4 streams
 void pack_tc_images(float* blob_host);   // host: fills BlobLayout::IMG_* from the fp32 part of the blob
@@ -154,23 +156,15 @@ __device__ __forceinline__ float delay_read(float dt, long long t, int D, LoadPa
 
 __device__ __forceinline__ float ex2_approx(float x)
 {
-#if NTM_DIAG_NOMUFU       // timing diagnostic only (wrong results): one FMA-pipe instruction in place of the MUFU one
-    return fmaf(x, 0.001f, 1.0f);
-#else
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
-#endif
 }
 __device__ __forceinline__ float rcp_approx(float x)
 {
-#if NTM_DIAG_NOMUFU
-    return fmaf(x, -0.001f, 1.0f);
-#else
     float y;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
-#endif
 }
 
 // ---- packed fp32 arithmetic (sm_100: add / mul / fma .f32x2 = FADD2 / FMUL2 / FFMA2): one issue slot for two lanes' worth of

@@ -126,7 +126,7 @@ def test_rnn_segmentation_invariance_bit_exact():
                 assert torch.equal(m.hidden, h_all)
 
 
-def test_rnn_streams_are_independent_bit_exact():
+def test_rnn_streams_are_independent_for_every_fp32_config():
     """Every stream of a batch equals its own batch-1 run, for every streams-per-CTA variant of the kernel."""
     m = make_rnn("cfg2")
     B, T = 37, 1500
@@ -134,7 +134,7 @@ def test_rnn_streams_are_independent_bit_exact():
     with torch.inference_mode():
         lib.load().ntm_set_tuning(1, 4)                # same k-split as the batched runs below
         singles = torch.cat([m.predict(x[b:b + 1]) for b in range(B)], 0)
-        for s in (0, 1, 2, 4, 8, 16):
+        for s in (0, 1, 2, 4, 8):
             lib.load().ntm_set_tuning(s, 4)
             assert torch.equal(m.predict(x), singles), f"streams_per_cta={s}"
         lib.load().ntm_set_tuning(2, 2)                # other k-split: different summation order

@@ -51,7 +51,7 @@ def test_mode_mask():
                                              torch.zeros(64, device=DEV).data_ptr(), 1, 8, 0, None))
 
 
-# kernel selectors (ntm_set_tuning): (n, 3) mma.sync kernel with n = 4, 8, 16 streams per CTA, (4, 6) its lean 4-stream form
+# kernel selectors (ntm_set_tuning): (n, 3) mma.sync kernel with n = 4, 8 streams per CTA, (4, 6) its lean 4-stream form
 # (gru_mma4.cu: what cfg 2 / 3 / 5 run; f16 / bf16 / strict -- tf32 falls through to the general kernel), (tiles, 4) stream-major
 # tcgen05 kernel
 KERNELS = [(8, 3), (4, 3), (4, 6), (1, 4), (2, 4)]
@@ -89,7 +89,7 @@ def test_bf16_is_finite_and_close():
 
 
 @pytest.mark.parametrize("mode", TC_MODES)
-def test_tc_batch_vs_oracle_and_launch_shapes(mode):
+def test_tc_batch_vs_oracle_and_kernel_selectors(mode):
     """64 mixed streams x 0.25 s against the torch restatement of the reference; every (streams per group,
     groups per CTA) variant of the kernel and a ragged batch give the same answer per stream."""
     m = make_rnn("cfg2", mode)
@@ -104,7 +104,7 @@ def test_tc_batch_vs_oracle_and_launch_shapes(mode):
         assert abs(c_oracle.esr(y0.cpu().numpy(), yr.numpy())) <= ESR_TOL
         # g = 3: warp-level mma.sync kernel with n streams per CTA; g = 4: stream-major tcgen05 kernel, n tiles per CTA
         fam = {}
-        for n, g in ((8, 3), (16, 3), (4, 3), (4, 6), (1, 4), (2, 4)):
+        for n, g in ((8, 3), (4, 3), (4, 6), (1, 4), (2, 4)):
             lib.load().ntm_set_tuning(n, g)
             y = m.predict(x)
             per_stream = ((y.cpu() - yr) ** 2).sum(2) / ((yr ** 2).sum(2) + 1e-5)
@@ -238,10 +238,10 @@ def test_stream_major_kernel_large_batch():
         assert float(((yb - y) ** 2).sum() / (y ** 2).sum()) <= 5e-2
 
 
-def test_stream_major_dynamic_schedule_is_exact():
+def test_stream_major_dynamic_schedule_equals_static_schedule():
     """More tile groups than SMs with a partial last wave: the kernel pulls (group, time chunk) jobs from a queue and a
     group's state migrates between SMs through h_out.  Results and final state must equal the static schedule's bit
-    for bit (tuning variant bit 32 forces the static schedule), for one and two tiles per CTA."""
+    for bit (tuning (tiles + 4, 4) forces the static schedule), for one and two tiles per CTA."""
     m = make_rnn("cfg2", "f16")
     sms = lib.query(lib.Q_SM_COUNT)
     with torch.inference_mode():
@@ -251,14 +251,40 @@ def test_stream_major_dynamic_schedule_is_exact():
         for tiles, B, T in ((2, sms * 256 + 300, 700), (1, sms * 128 + 1000, 900)):
             x = signals.stream_batch_device(B, T, DEV, dur=10.0).reshape(B, 1, T)
             outs = []
-            for var in (15, 47):                                  # default variant: dynamic, static (bit 32)
-                lib.load().ntm_set_tuning(tiles + 4 * (var + 1), 4)
+            for sel in (tiles, tiles + 4):                        # dynamic schedule, static schedule
+                lib.load().ntm_set_tuning(sel, 4)
                 m.hidden = hw.expand(1, B, 64).contiguous()
                 outs.append((m(x), m.hidden.clone()))
                 assert lib.query(lib.Q_LAST_KERNEL) == 3
             assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])
             assert bool(torch.isfinite(outs[0][0]).all())
             del x, outs
+
+
+def test_removed_kernel_selectors_are_rejected():
+    """A tuning pair outside the table of include/ntm_b200.h fails the launch with "invalid argument" instead of running some
+    other configuration; the pairs of the table still run the kernel they name."""
+    L = lib.load()
+    B, T = 8, 256
+    x = torch.from_numpy(signals.stream_batch(B, T)).to(DEV).reshape(B, 1, T)
+    cases = [("f16", (16, 3)),                          # 16 streams per CTA
+             ("f16", (1 + 4 * (3 + 1), 4)),             # tcgen05 kernel variant 3
+             ("fp32", (4, 0x104)),                      # MUFU activations of the fp32 kernel
+             ("f16", (4, 2)), ("fp32", (8, 3)), ("fp32", (4, 2)), ("f16", (3, 4))]
+    with torch.inference_mode():
+        for mode, sel in cases:
+            m = make_rnn("cfg2", mode)
+            L.ntm_set_tuning(*sel)
+            with pytest.raises(RuntimeError, match="invalid argument"):
+                m.predict(x)
+        kept = [("f16", (0, 0), 4), ("f16", (4, 3), 1), ("f16", (8, 3), 1), ("f16", (4, 6), 4), ("tf32", (4, 6), 1),
+                ("f16", (1, 4), 3), ("f16", (2, 4), 3), ("f16", (5, 4), 3), ("f16", (6, 4), 3),
+                ("fp32", (0, 0), 0), ("fp32", (8, 4), 0), ("fp32", (2, 2), 0), ("fp32", (0, 4), 0)]
+        for mode, sel, kernel in kept:
+            m = make_rnn("cfg2", mode)
+            L.ntm_set_tuning(*sel)
+            m.predict(x)
+            assert lib.query(lib.Q_LAST_KERNEL) == kernel, (mode, sel)
 
 
 def test_full_size_cfg2_properties():

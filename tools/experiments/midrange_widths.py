@@ -11,7 +11,7 @@ with torch.inference_mode():
     for B,T in ((2048,24000),(4096,12000),(4736,12000),(8192,12000),(9472,12000),(12000,6000),(16000,6000)):
         x=signals.stream_batch_device(B,T,dev,dur=10.0).reshape(B,1,T)
         row=[]
-        for tune in ((8,3),(16,3),(1,4),(0,0)):
+        for tune in ((8,3),(1,4),(0,0)):
             L.ntm_set_tuning(*tune)
             m.hidden=hw.expand(1,B,64).contiguous(); m(x[:,:,:1000])
             best=1e9

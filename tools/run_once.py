@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Dev tool (GPU box): one forward of B streams x T samples (for ncu captures).
-   usage: run_once.py B T [mode] [streams_per_cta] [ksplit|0x100 for fast activations] [diffdel]"""
+   usage: run_once.py B T [mode] [s] [ks] [diffdel]    ((s, ks): a kernel selector of ntm_set_tuning, include/ntm_b200.h)"""
 import os
 import sys
 
@@ -14,7 +14,7 @@ from ntm_b200 import lib, signals
 B, T = int(sys.argv[1]), int(sys.argv[2])
 mode = sys.argv[3] if len(sys.argv) > 3 else "fp32"
 s = int(sys.argv[4]) if len(sys.argv) > 4 else 0
-ks = int(sys.argv[5], 0) if len(sys.argv) > 5 else 0
+ks = int(sys.argv[5]) if len(sys.argv) > 5 else 0
 diffdel = len(sys.argv) > 6
 dev = torch.device("cuda:0")
 tag = "cfg3" if diffdel else "cfg2"

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Dev tool (GPU box): the stream-major tcgen05 kernel per operand format and kernel variant at throughput widths.
+"""Dev tool (GPU box): the stream-major tcgen05 kernel per operand format, job-queue and static schedule, at throughput widths.
 usage: tcs_speed.py [B T]..."""
 import os
 import sys
@@ -29,9 +29,9 @@ with torch.inference_mode():
         ref = None
         for mode in ("f16", "f16x3", "tf32", "bf16"):
             m.mode = mode
-            for var in ((15, 7, 3) if mode in ("f16", "bf16") else (15, 3)):
-                tiles = 2 if B >= 190 * sms else 1
-                L.ntm_set_tuning(tiles + 4 * (var + 1), 4)
+            tiles = 2 if B >= 190 * sms else 1
+            for sched in ("dynamic", "static"):
+                L.ntm_set_tuning(tiles + (4 if sched == "static" else 0), 4)
                 m.hidden = hw.expand(1, B, 64).contiguous(); m(x[:, :, :300])
                 best = 1e9
                 for _ in range(3):
@@ -46,7 +46,7 @@ with torch.inference_mode():
                     m.mode = mode
                 err = float((y[:512] - ref).abs().max())
                 esr = float(((y[:512] - ref) ** 2).sum() / (ref ** 2).sum())
-                print(f"B={B} T={T} {mode:6s} var={var} tiles={tiles}: {best:8.3f} ms {B*T/best/1e6:7.3f} Gs/s "
+                print(f"B={B} T={T} {mode:6s} {sched:7s} tiles={tiles}: {best:8.3f} ms {B*T/best/1e6:7.3f} Gs/s "
                       f"{best*1e-3*1.965e9*sms/(B*T):6.2f} clk/stream-step/SM | vs strict mma.sync (512 streams): max-abs {err:.2e} ESR {esr:.2e}",
                       flush=True)
 L.ntm_set_tuning(0, 0)
