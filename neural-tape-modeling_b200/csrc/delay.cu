@@ -18,18 +18,12 @@ namespace {
 //   + second tap reused from the neighbour sample 5.20        9 gathers per thread instead of 16: the gathers cost L1 passes
 //   + 32 groups per thread, next delays prefetched 6.38       few long-lived CTAs instead of one CTA per 2048 samples
 constexpr int DELAY_SPT = 8;
-#ifndef NTM_DELAY_REUSE
-#define NTM_DELAY_REUSE 1
-#endif
-#ifndef NTM_DELAY_ITER
-#define NTM_DELAY_ITER 32
-#endif
 // Few, long-lived CTAs: a thread walks over up to DELAY_ITER groups of its row (a grid stride apart) and loads the delays of its next
 // group before it gathers the taps of the current one -- one exposed HBM round trip per group instead of two dependent ones, and
 // no CTA launch per 2048 samples.  Measured at 1024 x 1 440 000, D = 365 (profiles/r02f_delay_line.txt): 4.63 TB/s with one group
 // per thread, 5.20 with the tap reuse below, 5.85 / 6.07 / 6.18 / 6.36 at 4 / 8 / 16 / 32 groups per thread.  Small problems keep one
 // group per thread (the launcher never drops below DELAY_MIN_CTAS_PER_SM CTAs per SM).
-constexpr int DELAY_ITER = NTM_DELAY_ITER;
+constexpr int DELAY_ITER = 32;
 constexpr int DELAY_MIN_CTAS_PER_SM = 12;
 
 template <bool VEC>
@@ -99,7 +93,7 @@ __global__ void __launch_bounds__(256, 3) delay_kernel(const float* __restrict__
                     p[0][1] = __ldg(xt + off[0][1]);
 #pragma unroll
                     for (int j = 1; j < DELAY_SPT; ++j)
-                        p[j][1] = (NTM_DELAY_REUSE && off[j][1] == off[j - 1][0]) ? p[j - 1][0] : __ldg(xt + off[j][1]);
+                        p[j][1] = off[j][1] == off[j - 1][0] ? p[j - 1][0] : __ldg(xt + off[j][1]);
                 } else {
                     const float* ht = hr + D + t;
 #pragma unroll

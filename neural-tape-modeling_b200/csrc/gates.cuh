@@ -5,16 +5,15 @@
 //     n = tanh(W_in x + b_in + r * (W_hn h + b_hn))   h' = (1 - z) * n + z * h
 // with every pre-activation pre-scaled on the way in (weights and constants by -log2 e for r, z and by 2 log2 e for n):
 //     sigmoid(a) = 1 / (1 + 2^(-a log2 e))            tanh(a) = 1 - 2 / (1 + 2^(2 a log2 e))
-// MUFU is the scarce pipe (16 lanes/clk/SM): reciprocals are shared -- 1/(d_r d_z) serves r and z of one pair,
-// 1/(d_n0 d_n1) serves the n gates of two pairs -- which brings a (unit, stream) pair from 6 to 4 MUFU operations.
-// Arguments of ex2 are clamped to 60 so that a product of two denominators stays below 2^121.
+// MUFU is the scarce pipe (16 lanes/clk/SM): the 8-stream form shares 1/(d_n0 d_n1) between the n gates of two units of one
+// stream (gates_blend2).  Arguments of ex2 are clamped to 60 so that a product of two denominators stays below 2^121.
 #pragma once
 #include "ntm_common.cuh"
 
 namespace ntm {
 
 struct UnitConst {
-    float cr_w, cr_b, cz_w, cz_b, cn_w, cn_b, ch_b, wo;
+    float cr_w, cr_b, cz_w, cz_b, cn_w, cn_b, ch_b;
 };
 
 __device__ __forceinline__ UnitConst load_unit_const(const float* __restrict__ blob, int j)
@@ -28,34 +27,10 @@ __device__ __forceinline__ UnitConst load_unit_const(const float* __restrict__ b
     c.cn_w = 2.0f * L * blob[BlobLayout::W_IH + 128 + j];
     c.cn_b = 2.0f * L * blob[BlobLayout::B_IH + 128 + j];
     c.ch_b = 2.0f * L * blob[BlobLayout::B_HH + 128 + j];
-    c.wo = blob[BlobLayout::W_OUT + j];
     return c;
 }
 
 constexpr float EX2_CLAMP = 60.0f;
-
-// r, z and the denominator of the n gate of one pair.  ar, az, an: scaled W_h* h products from the tensor core.
-__device__ __forceinline__ void gates_rz_dn(const UnitConst& c, float ar, float az, float an, float x, float& z, float& dn)
-{
-    const float dr = 1.0f + ex2_approx(fminf(ar + fmaf(c.cr_w, x, c.cr_b), EX2_CLAMP));
-    const float dz = 1.0f + ex2_approx(fminf(az + fmaf(c.cz_w, x, c.cz_b), EX2_CLAMP));
-    const float rinv = rcp_approx(dr * dz);
-    const float r = dz * rinv;
-    z = dr * rinv;
-    dn = 1.0f + ex2_approx(fminf(fmaf(r, an + c.ch_b, fmaf(c.cn_w, x, c.cn_b)), EX2_CLAMP));
-}
-
-// the same with complete pre-activations: ar, az already contain W_i x + b (K-augmented MMA), an = W_hn h + b_hn,
-// gin = W_in x + b_in (all scaled)
-__device__ __forceinline__ void gates_rz_dn_pre(float ar, float az, float an, float gin, float& z, float& dn)
-{
-    const float dr = 1.0f + ex2_approx(fminf(ar, EX2_CLAMP));
-    const float dz = 1.0f + ex2_approx(fminf(az, EX2_CLAMP));
-    const float rinv = rcp_approx(dr * dz);
-    const float r = dz * rinv;
-    z = dr * rinv;
-    dn = 1.0f + ex2_approx(fminf(fmaf(r, an, gin), EX2_CLAMP));
-}
 
 // Latency-regime form: r has its own reciprocal (r -> n -> h' is the step's critical path; sharing 1/(d_r d_z) makes r
 // wait for z's ex2 and two more multiplies), z's ex2 / rcp fill the MUFU pipe's idle slots.  5.5 MUFU per pair.
@@ -87,101 +62,25 @@ __device__ __forceinline__ float gates_blend1_late(float z, float dn, float h)
     const float a = fmaf(z, h - 1.0f, 1.0f), b = fmaf(2.0f, z, -2.0f);
     return fmaf(b, rcp_approx(dn), a);
 }
-// 2^x on the FMA/ALU pipes (no MUFU): round-to-nearest split x = i + f, f in [-0.5, 0.5], degree-5 minimax polynomial
-// (max relative error 2.4e-7 in fp32 Horner form = the accuracy class of ex2.approx), exponent inserted by an integer
-// add.  x must be <= 127 on entry (callers clamp to EX2_CLAMP); clamped below at -125 (result ~2^-125 instead of 0).
-__device__ __forceinline__ float ex2_poly(float x)
-{
-    x = fmaxf(x, -125.0f);
-    const float t = x + 12582912.0f;                 // 1.5 * 2^23: the integer part lands in the low mantissa bits
-    const float f = x - (t - 12582912.0f);
-    float p = 1.327647129e-03f;
-    p = fmaf(p, f, 9.675540961e-03f);
-    p = fmaf(p, f, 5.550713092e-02f);
-    p = fmaf(p, f, 2.402212024e-01f);
-    p = fmaf(p, f, 6.931469440e-01f);
-    p = fmaf(p, f, 1.000000119e+00f);
-    return __int_as_float(__float_as_int(p) + (__float_as_int(t) << 23));
-}
 
 // ---- strict (fp32-grade) activations ---------------------------------------------------------------------------------
 // MUFU ex2.approx / rcp.approx are accurate to ~2 ulp, but their error is SYSTEMATIC: a constant relative bias of 1 ulp in
 // the gate values moves the output of the cfg-2 checkpoint by 1.7e-5 (numpy emulation), a random +-2 ulp only by 2e-6 --
-// the recurrence integrates a bias.  The strict mode therefore evaluates 2^x with a degree-6 minimax polynomial on the FMA
-// pipe (max relative error 0.66 ulp, mean bias 0.002 ulp over the reduced range) and refines the reciprocal with one
-// Newton step (error <= 1 ulp, unbiased).
-__device__ __forceinline__ float ex2_strict(float x)
-{
-    x = fmaxf(x, -125.0f);
-    const float t = x + 12582912.0f;                 // 1.5 * 2^23: round-to-nearest integer part in the low mantissa bits
-    const float f = x - (t - 12582912.0f);           // [-0.5, 0.5]
-    float p = 1.534580806e-04f;
-    p = fmaf(p, f, 1.339993090e-03f);
-    p = fmaf(p, f, 9.618489072e-03f);
-    p = fmaf(p, f, 5.550328642e-02f);
-    p = fmaf(p, f, 2.402264625e-01f);
-    p = fmaf(p, f, 6.931471825e-01f);
-    p = fmaf(p, f, 1.0f);
-    return __int_as_float(__float_as_int(p) + (__float_as_int(t) << 23));
-}
+// the recurrence integrates a bias.  The strict mode therefore refines every reciprocal with one Newton step (error <= 1 ulp,
+// unbiased); 2^x stays on MUFU.
 __device__ __forceinline__ float rcp_strict(float d)
 {
     const float r = rcp_approx(d);
     return fmaf(r, fmaf(-d, r, 1.0f), r);
 }
-#ifndef NTM_STRICT_ACT
-#define NTM_STRICT_ACT 1          // 0: bare MUFU, 1: Newton reciprocal (the default, see below), 2: + polynomial 2^x
-#endif
-__device__ __forceinline__ float ex2_s(float x) { return NTM_STRICT_ACT >= 2 ? ex2_strict(x) : ex2_approx(x); }
-__device__ __forceinline__ float rcp_s(float d) { return NTM_STRICT_ACT >= 1 ? rcp_strict(d) : rcp_approx(d); }
-
 // One (unit, stream) pair in the strict mode: own reciprocals everywhere (nothing shared, no products of denominators).
 // pr, pz: complete scaled pre-activations of r and z; ahn = W_hn h + b_hn, gin = W_in x + b_in (scaled); returns the new state.
 __device__ __forceinline__ float gates_strict(float pr, float pz, float ahn, float gin, float h)
 {
-    const float r = rcp_s(1.0f + ex2_s(fminf(pr, EX2_CLAMP)));
-    const float dn = 1.0f + ex2_s(fminf(fmaf(r, ahn, gin), EX2_CLAMP));
-    const float z = rcp_s(1.0f + ex2_s(fminf(pz, EX2_CLAMP)));
-    const float n = fmaf(-2.0f, rcp_s(dn), 1.0f);
-    return fmaf(z, h - n, n);
-}
-
-// Two hidden units (0, 1) of ONE stream, complete pre-activations (see gates_rz_dn_pre), new states out.
-//   SHARE4: one reciprocal serves r and z of BOTH units (4.0 MUFU per unit-step instead of 4.5); the ex2 arguments of
-//           r, z are then clamped to 30 so that the product of four denominators stays below 2^121 (sigmoid saturates
-//           at 2^-30 instead of 2^-60: absolute error < 1e-9).
-//   NPOLY:  how many of the six ex2 of the two units run on the FMA pipe (ex2_poly) instead of MUFU: 0, 1 (z of unit 1)
-//           or 2 (z of both units) -- the z gates are off the r -> n dependency chain.
-template <bool SHARE4, int NPOLY>
-__device__ __forceinline__ void gates_unit_pair(float ar0, float az0, float an0, float gin0, float ar1, float az1, float an1,
-                                                float gin1, float h0, float h1, float& hn0, float& hn1)
-{
-    constexpr float C = SHARE4 ? 30.0f : EX2_CLAMP;
-    const float dr0 = 1.0f + ex2_approx(fminf(ar0, C));
-    const float dr1 = 1.0f + ex2_approx(fminf(ar1, C));
-    const float dz0 = 1.0f + (NPOLY >= 2 ? ex2_poly(fminf(az0, C)) : ex2_approx(fminf(az0, C)));
-    const float dz1 = 1.0f + (NPOLY >= 1 ? ex2_poly(fminf(az1, C)) : ex2_approx(fminf(az1, C)));
-    float r0, z0, r1, z1;
-    if (SHARE4) {
-        const float p0 = dr0 * dz0, p1 = dr1 * dz1;
-        const float q = rcp_approx(p0 * p1);
-        const float i0 = p1 * q, i1 = p0 * q;
-        r0 = dz0 * i0; z0 = dr0 * i0;
-        r1 = dz1 * i1; z1 = dr1 * i1;
-    } else {
-        const float i0 = rcp_approx(dr0 * dz0), i1 = rcp_approx(dr1 * dz1);
-        r0 = dz0 * i0; z0 = dr0 * i0;
-        r1 = dz1 * i1; z1 = dr1 * i1;
-    }
-    const float dn0 = 1.0f + ex2_approx(fminf(fmaf(r0, an0, gin0), EX2_CLAMP));
-    const float dn1 = 1.0f + ex2_approx(fminf(fmaf(r1, an1, gin1), EX2_CLAMP));
-    gates_blend2(z0, dn0, h0, z1, dn1, h1, hn0, hn1);
-}
-
-// new state of one pair (own reciprocal: keeps a stream's arithmetic independent of its neighbours)
-__device__ __forceinline__ float gates_blend1(float z, float dn, float h)
-{
-    const float n = fmaf(-2.0f, rcp_approx(dn), 1.0f);
+    const float r = rcp_strict(1.0f + ex2_approx(fminf(pr, EX2_CLAMP)));
+    const float dn = 1.0f + ex2_approx(fminf(fmaf(r, ahn, gin), EX2_CLAMP));
+    const float z = rcp_strict(1.0f + ex2_approx(fminf(pz, EX2_CLAMP)));
+    const float n = fmaf(-2.0f, rcp_strict(dn), 1.0f);
     return fmaf(z, h - n, n);
 }
 

@@ -577,24 +577,13 @@ cudaError_t launch_mma_one(const GruArgs& a, cudaStream_t st)
     static OncePerDevice once;
     cudaError_t e = once.run([] {
         return cudaFuncSetAttribute(gru_mma_kernel<FMT, HALF, false, DEFER, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    C::SMEM_BYTES + 48 * 1024);
+                                    C::SMEM_BYTES + DELAY_RING_BUDGET);
     });
     if (e != cudaSuccess) return e;
     constexpr int SC = HALF ? 4 : C::S;
     const long long grid = (a.B + SC - 1) / SC;
-    // DiffDelRNN: keep the last D + CH samples of pre_d per stream on chip if they fit (<= 48 KB of ring per CTA, so that
-    // four CTAs still share an SM); longer histories read their taps back through L2
     GruArgs b = a;
-    b.ring_len = 0;
-    int smem_bytes = C::SMEM_BYTES;
-    if (a.d != nullptr && !a.warmup) {
-        long long rl = 64;
-        while (rl < (long long)a.D + C::CH + 1) rl *= 2;
-        if (rl * SC * 4 <= 48 * 1024) {
-            b.ring_len = (int)rl;
-            smem_bytes += (int)(rl * SC * 4);
-        }
-    }
+    const int smem_bytes = C::SMEM_BYTES + size_delay_ring(b, SC, C::CH);
     gru_mma_kernel<FMT, HALF, false, DEFER, SPLIT><<<(unsigned)grid, 128, smem_bytes, st>>>(b);
     ++g_launches;
     return cudaGetLastError();

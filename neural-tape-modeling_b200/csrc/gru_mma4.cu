@@ -361,22 +361,12 @@ cudaError_t launch_mma4_one(const GruArgs& a, cudaStream_t st)
     using C = Mma4Cfg<FMT>;
     static OncePerDevice once;
     cudaError_t e = once.run([] {
-        return cudaFuncSetAttribute(gru_mma4_kernel<FMT, STRICT>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES + 48 * 1024);
+        return cudaFuncSetAttribute(gru_mma4_kernel<FMT, STRICT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    C::SMEM_BYTES + DELAY_RING_BUDGET);
     });
     if (e != cudaSuccess) return e;
-    // DiffDelRNN: keep the last D + CH samples of pre_d per stream on chip if they fit (<= 48 KB of ring per CTA); longer
-    // histories read their taps back through L2
     GruArgs b = a;
-    b.ring_len = 0;
-    int smem_bytes = C::SMEM_BYTES;
-    if (a.d != nullptr && !a.warmup) {
-        long long rl = 64;
-        while (rl < (long long)a.D + C::CH + 1) rl *= 2;
-        if (rl * C::SC * 4 <= 48 * 1024) {
-            b.ring_len = (int)rl;
-            smem_bytes += (int)(rl * C::SC * 4);
-        }
-    }
+    const int smem_bytes = C::SMEM_BYTES + size_delay_ring(b, C::SC, C::CH);
     gru_mma4_kernel<FMT, STRICT><<<(unsigned)((a.B + C::SC - 1) / C::SC), 128, smem_bytes, st>>>(b);
     ++g_launches;
     return cudaGetLastError();

@@ -1,4 +1,4 @@
-// Fragment helpers shared by the warp-level mma.sync kernels (gru_mma.cu, gru_mma2.cu): operand formats, the MMA itself,
+// Fragment helpers shared by the warp-level mma.sync kernels (gru_mma.cu, gru_mma4.cu): operand formats, the MMA itself,
 // the rounded-state tile.  Internal to the engine.
 #pragma once
 #include <cuda_fp16.h>

@@ -66,8 +66,8 @@ struct GruArgs {
     int D;
     int warmup;
     int skip;
-    int ring_len;                   // mma.sync kernel, DiffDelRNN: samples of pre_d kept per stream in shared memory
-                                    // (power of two >= D + chunk; 0: read the delay taps back through L2)
+    int ring_len;                   // DiffDelRNN, mma.sync kernels: samples of pre_d kept per stream in shared memory (power
+                                    // of two >= D + chunk + 1, size_delay_ring; 0: read the delay taps back through L2)
     int sm_count;                   // SMs of the handle's device (host-side dispatch only)
     RtMailbox* rt;                  // real-time server form only (x, y point into it)
     unsigned long long rt_idle_ns;  // the server leaves after this long without a block
@@ -94,7 +94,8 @@ cudaError_t launch_gru_tcs(const GruArgs& a, const TcsConsts& kc, int fmt, int s
                            cudaStream_t st);
 void fill_tcs_consts(const float* blob_host, TcsConsts* kc);
 cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_head, cudaStream_t st);
-cudaError_t launch_gru_mma4(const GruArgs& a, int fmt, cudaStream_t st);   // plain GRU, f16 / bf16, four streams per CTA, 4x unrolled
+cudaError_t launch_gru_mma4(const GruArgs& a, int fmt, cudaStream_t st);   // GRU and DiffDelGRU, f16 / bf16 / strict f16x3, four
+                                                                             // streams per CTA, 4x unrolled
 cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st);    // resident real-time server, <= 4 streams
 void pack_tc_images(float* blob_host);   // host: fills BlobLayout::IMG_* from the fp32 part of the blob
 cudaError_t launch_delay(const float* x, long long ldx, const float* d, long long ldd, float* y, long long ldy,
@@ -152,6 +153,22 @@ __device__ __forceinline__ float delay_read(float dt, long long t, int D, LoadPa
         }
     }
     return acc;
+}
+
+// On-chip pre_d ring of a DiffDelRNN launch of the mma.sync kernels (gru_mma.cu, gru_mma4.cu) with `streams` streams per CTA
+// and chunks of `chunk` steps: the last ring_len samples of pre_d per stream, ring_len the smallest power of two (>= 64)
+// that is >= D + chunk + 1, stay in shared memory if they fit in DELAY_RING_BUDGET bytes per CTA (so that four CTAs still
+// share an SM); longer histories read their taps back through L2.  Sets b.ring_len (0: no ring) and returns the ring's bytes.
+constexpr int DELAY_RING_BUDGET = 48 * 1024;
+inline int size_delay_ring(GruArgs& b, int streams, int chunk)
+{
+    b.ring_len = 0;
+    if (b.d == nullptr || b.warmup) return 0;
+    long long rl = 64;
+    while (rl < (long long)b.D + chunk + 1) rl *= 2;
+    if (rl * streams * 4 > DELAY_RING_BUDGET) return 0;
+    b.ring_len = (int)rl;
+    return (int)(rl * streams * 4);
 }
 
 __device__ __forceinline__ float ex2_approx(float x)

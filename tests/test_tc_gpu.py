@@ -314,14 +314,19 @@ def test_full_size_cfg2_properties():
         assert float(per_stream.max()) <= ESR_TOL
 
 
-@pytest.mark.parametrize("max_delay", [100, 364, 2000, 6000])
-def test_tc_diffdel_delay_read_paths_bit_exact(max_delay):
-    """The fused delay read of the mma.sync kernel keeps the last D + 32 samples of pre_d per stream in shared memory
-    when they fit (D <= ~3000 for four streams per CTA) and reads its taps back through L2 otherwise: both paths must
-    reproduce the oracle's delay line bit for bit on the engine's own pre_d and warm history, across segment boundaries."""
+@pytest.mark.parametrize("max_delay", [100, 364, 1000, 2000, 6000])
+@pytest.mark.parametrize("mode,tuning,kernel", [("f16", (0, 0), 4), ("f16x3", (0, 0), 4), ("f16", (4, 3), 1),
+                                                ("f16", (8, 3), 1), ("tf32", (0, 0), 1), ("fp32", (0, 0), 0)])
+def test_tc_diffdel_delay_read_paths_bit_exact(mode, tuning, kernel, max_delay):
+    """The fused delay read of the mma.sync kernels keeps the last D + 129 samples of pre_d per stream (D = max_delay + 1)
+    in shared memory when they fit (D <= 1919 at four streams per CTA, D <= 895 at eight: max_delay = 1000 takes the ring
+    in one and L2 in the other) and reads its taps back through L2 otherwise, as the fp32 kernel always does.  Every
+    kernel and path must reproduce the oracle's delay line bit for bit on the engine's own pre_d and warm history, across
+    segment boundaries; a warm-up segment returns pre_d itself and still rolls the history."""
+    lib.load().ntm_set_tuning(*tuning)
     m = DiffDelRNN(input_size=1, hidden_size=64, output_size=1, skip=False, max_delay=max_delay).to(DEV)
     m.load_state_dict(load_ckpt("cfg3"))
-    m.mode = "f16"
+    m.mode = mode
     B, T = 6, 9000
     rng = np.random.default_rng(max_delay)
     x = dev(signals.stream_batch(B, T)).reshape(B, 1, T)
@@ -336,12 +341,19 @@ def test_tc_diffdel_delay_read_paths_bit_exact(max_delay):
         m.hidden = m.hidden.expand(1, B, 64).contiguous()
         m.diffdel.buffer = m.diffdel.buffer.expand(B, 1, -1).contiguous()
         ys, ps, s = [], [], 0
-        for n in (31, 4000, 1, 4968):
-            yy, pp = m(x[:, :, s:s + n], d[:, :, s:s + n])
+        warm = slice(4032, 4532)                            # the warm-up segment
+        for n in (31, 4000, 1, 500, 4468):
+            yy, pp = m(x[:, :, s:s + n], d[:, :, s:s + n], warmup=s == warm.start)
+            assert lib.query(lib.Q_LAST_KERNEL) == kernel
             ys.append(yy)
             ps.append(pp)
             s += n
+        assert s == T
         y, pre = torch.cat(ys, 2).cpu().numpy().reshape(B, T), torch.cat(ps, 2).cpu().numpy().reshape(B, T)
-        yo, _ = c_oracle.delay_forward(pre, dn, np.repeat(hist_w, B, 0))
+        assert np.array_equal(y[:, warm], pre[:, warm])
+        # the oracle runs over all of pre_d: the segments after the warm-up one read the history it rolled
+        yo, ho = c_oracle.delay_forward(pre, dn, np.repeat(hist_w, B, 0))
+        yo[:, warm] = pre[:, warm]
         assert np.array_equal(yo, y)
+        assert np.array_equal(ho.reshape(B, -1), m.diffdel.buffer.cpu().numpy().reshape(B, -1))
         assert np.all(np.isfinite(y))
