@@ -250,7 +250,7 @@ __global__ void __launch_bounds__(64 * KS, 2) gru_fp32_kernel(const GruArgs a)
         }
     }
 
-    // ---- final state; rolled delay history (code/model.py:314-315) -------------------------------
+    // ---- final state; rolled delay history ------------------------------------------------------
 #pragma unroll
     for (int i = 0; i < SO; ++i) {
         const int s = i * KS + q;
@@ -258,13 +258,7 @@ __global__ void __launch_bounds__(64 * KS, 2) gru_fp32_kernel(const GruArgs a)
     }
     if (delay) {
         __syncthreads();
-        for (long long idx = tid; idx < (long long)ns * a.D; idx += NT) {
-            const int s = (int)(idx / a.D);
-            const long long i = idx % a.D;
-            const long long src = a.T - a.D + i;
-            a.hist_out[(b0 + s) * (long long)a.D + i] =
-                src >= 0 ? __ldcg(a.pre + (b0 + s) * a.ldp + src) : a.hist_in[(b0 + s) * (long long)a.D + a.D + src];
-        }
+        delay_roll_history<NT>(a, b0, ns, tid);
     }
 }
 

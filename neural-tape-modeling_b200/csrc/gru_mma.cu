@@ -273,13 +273,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         }
         cp_async_commit();
     };
-    if (use_ring) {                                          // carried history -> ring positions -D .. -1
-        for (long long idx = tid; idx < (long long)ns * a.D; idx += 128) {
-            const int s = (int)(idx / a.D);
-            const int i = (int)(idx % a.D);
-            ring[s * a.ring_len + ((i - a.D) & rmask)] = a.hist_in[(b0 + s) * (long long)a.D + i];
-        }
-    }
+    if (use_ring) delay_ring_prefill<128>(a, b0, ns, tid, ring);
 
     // ---- initial state: fp32 in registers (hst[unit][stream]), rounded copy into state tile 0 ---------------------
     float hst[2][2];
@@ -523,17 +517,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
             }
         } else if (delay && !a.warmup) {
             __syncthreads();                   // this chunk's pre_d is visible CTA-wide (L2 reads below)
-            for (int idx = tid; idx < SC * CH; idx += 128) {
-                const int s = idx / CH, tt = idx % CH;
-                if (s < ns && tt < n) {
-                    const long long tg = t0 + tt;
-                    const float* prow = a.pre + (b0 + s) * a.ldp;
-                    const float* hrow = a.hist_in + (b0 + s) * (long long)a.D;
-                    a.y[(b0 + s) * a.ldy + tg] =
-                        delay_read(a.d[(b0 + s) * a.ldd + tg], tg, a.D,
-                                   [&](long long i) { return i >= 0 ? __ldcg(prow + i) : hrow[a.D + i]; });
-                }
-            }
+            delay_chunk_l2<128, SC, CH>(a, b0, ns, tid, t0, n);
         }
     }
 
@@ -550,7 +534,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
     }
     } while (RT);
 
-    // ---- final state; rolled delay history (code/model.py:314-315) -------------------------------------------------
+    // ---- final state; rolled delay history --------------------------------------------------------------------------
 #pragma unroll
     for (int u = 0; u < 2; ++u)
 #pragma unroll
@@ -560,13 +544,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         }
     if (delay) {
         __syncthreads();
-        for (long long idx = tid; idx < (long long)ns * a.D; idx += 128) {
-            const int s = (int)(idx / a.D);
-            const long long i = idx % a.D;
-            const long long src = a.T - a.D + i;
-            a.hist_out[(b0 + s) * (long long)a.D + i] =
-                src >= 0 ? __ldcg(a.pre + (b0 + s) * a.ldp + src) : a.hist_in[(b0 + s) * (long long)a.D + a.D + src];
-        }
+        delay_roll_history<128>(a, b0, ns, tid);
     }
 }
 

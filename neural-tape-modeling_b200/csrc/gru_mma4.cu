@@ -165,13 +165,7 @@ __global__ void __launch_bounds__(128, 2) gru_mma4_kernel(const GruArgs a)
         }
         cp_async_commit();
     };
-    if (use_ring) {                                          // carried history -> ring positions -D .. -1
-        for (long long idx = tid; idx < (long long)ns * a.D; idx += 128) {
-            const int s = (int)(idx / a.D);
-            const int i = (int)(idx % a.D);
-            ring[s * a.ring_len + ((i - a.D) & rmask)] = a.hist_in[(b0 + s) * (long long)a.D + i];
-        }
-    }
+    if (use_ring) delay_ring_prefill<128>(a, b0, ns, tid, ring);
 
     // ---- initial state: fp32 in registers, rounded copy into state tile 0; the odd (dead) columns of both tiles stay zero ----
     float hst[2] = {0.0f, 0.0f};
@@ -330,28 +324,13 @@ __global__ void __launch_bounds__(128, 2) gru_mma4_kernel(const GruArgs a)
             }
         } else if (delay && !a.warmup) {
             __syncthreads();                   // this chunk's pre_d is visible CTA-wide (L2 reads below)
-            for (int idx = tid; idx < SC * CH; idx += 128) {
-                const int s = idx / CH, t = idx % CH;
-                if (s < ns && t < n) {
-                    const long long tg = t0 + t;
-                    const float* prow = a.pre + (b0 + s) * a.ldp;
-                    const float* hrow = a.hist_in + (b0 + s) * (long long)a.D;
-                    a.y[(b0 + s) * a.ldy + tg] = delay_read(a.d[(b0 + s) * a.ldd + tg], tg, a.D,
-                                                            [&](long long i) { return i >= 0 ? __ldcg(prow + i) : hrow[a.D + i]; });
-                }
-            }
+            delay_chunk_l2<128, SC, CH>(a, b0, ns, tid, t0, n);
         }
     }
     if (tig < ns) { a.h_out[(b0 + tig) * 64 + u0] = hst[0]; a.h_out[(b0 + tig) * 64 + u1] = hst[1]; }
-    if (delay) {                               // rolled delay history (code/model.py:314-315)
+    if (delay) {
         __syncthreads();
-        for (long long idx = tid; idx < (long long)ns * a.D; idx += 128) {
-            const int s = (int)(idx / a.D);
-            const long long i = idx % a.D;
-            const long long src = a.T - a.D + i;
-            a.hist_out[(b0 + s) * (long long)a.D + i] =
-                src >= 0 ? __ldcg(a.pre + (b0 + s) * a.ldp + src) : a.hist_in[(b0 + s) * (long long)a.D + a.D + src];
-        }
+        delay_roll_history<128>(a, b0, ns, tid);
     }
 }
 

@@ -171,6 +171,56 @@ inline int size_delay_ring(GruArgs& b, int streams, int chunk)
     return (int)(rl * streams * 4);
 }
 
+// DiffDelRNN delay tail of the fused recurrent kernels (gru_fp32.cu, gru_mma.cu, gru_mma4.cu), for a CTA of NT threads that owns
+// the ns streams from b0 on.  hist_in and hist_out hold each stream's last D samples of pre_d, oldest first.  ptxas
+// reschedules the kernels' step loops when the shape of this code changes, so compare their SASS after editing it.  The ring
+// delay pass of the mma.sync kernels and gru_fp32.cu's delay pass (warm-up store inside) stay in their kernels: every shared
+// form of them tried did that.
+
+// Carried history -> positions -D .. -1 of the pre_d ring (mma.sync kernels, a.ring_len > 0).
+template <int NT>
+__device__ __forceinline__ void delay_ring_prefill(const GruArgs& a, long long b0, int ns, int tid, float* ring)
+{
+    const int rmask = a.ring_len - 1;
+    for (long long idx = tid; idx < (long long)ns * a.D; idx += NT) {
+        const int s = (int)(idx / a.D);
+        const int i = (int)(idx % a.D);
+        ring[s * a.ring_len + ((i - a.D) & rmask)] = a.hist_in[(b0 + s) * (long long)a.D + i];
+    }
+}
+
+// y of samples [t0, t0 + n) of the chunk (CH steps, SC streams per CTA), the taps read back through L2: from the pre_d this
+// CTA has just written (__ldcg) and from hist_in.
+template <int NT, int SC, int CH>
+__device__ __forceinline__ void delay_chunk_l2(const GruArgs& a, long long b0, int ns, int tid, long long t0, int n)
+{
+    for (int idx = tid; idx < SC * CH; idx += NT) {
+        const int s = idx / CH, tt = idx % CH;
+        if (s < ns && tt < n) {
+            const long long tg = t0 + tt;
+            const float* prow = a.pre + (b0 + s) * a.ldp;
+            const float* hrow = a.hist_in + (b0 + s) * (long long)a.D;
+            a.y[(b0 + s) * a.ldy + tg] =
+                delay_read(a.d[(b0 + s) * a.ldd + tg], tg, a.D,
+                           [&](long long i) { return i >= 0 ? __ldcg(prow + i) : hrow[a.D + i]; });
+        }
+    }
+}
+
+// Rolled delay history (code/model.py:314-315): hist_out = the last D samples of (hist_in || pre_d), once the CTA has
+// written all of pre_d.
+template <int NT>
+__device__ __forceinline__ void delay_roll_history(const GruArgs& a, long long b0, int ns, int tid)
+{
+    for (long long idx = tid; idx < (long long)ns * a.D; idx += NT) {
+        const int s = (int)(idx / a.D);
+        const long long i = idx % a.D;
+        const long long src = a.T - a.D + i;
+        a.hist_out[(b0 + s) * (long long)a.D + i] =
+            src >= 0 ? __ldcg(a.pre + (b0 + s) * a.ldp + src) : a.hist_in[(b0 + s) * (long long)a.D + a.D + src];
+    }
+}
+
 __device__ __forceinline__ float ex2_approx(float x)
 {
     float y;
