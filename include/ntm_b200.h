@@ -180,6 +180,26 @@ int ntm_diffdel_predict_host(void* handle, int mode, const float* x_host, const 
 int ntm_esr_sums_rows(const float* out, int64_t ldo, const float* target, int64_t ldt, int64_t B, int64_t T,
                       const int64_t* first, const int64_t* count, int dc_pre, double* sums, int device, void* stream);
 
+/*
+ * Multi-resolution STFT loss (the third loss of the reference's evaluation loop, code/test-model.py:253).
+ * Replaces: auraloss MultiResolutionSTFTLoss (auraloss/freq.py) with its defaults: per resolution r, torch.stft(x, N_r,
+ * hop_r, win_r, hann_window(win_r)) with center=True and reflect padding by N_r/2 (F = 1 + n/hop_r frames, N_r/2 + 1 bins)
+ * and the clamped magnitudes |X| = sqrt(max(|STFT|^2, 1e-8)) of out (X) and target (Y).
+ *   out, target: B rows of T samples (row strides ldo, ldt); row b is evaluated over its own window
+ *   [first[b], first[b] + count[b]) (DEVICE int64 arrays of B values; NULL = 0 / T), clipped to the row, and the
+ *   reflection is relative to that window (the INIT_LEN cut, code/test-model.py:367-370).
+ *   fft_sizes / hop_sizes / win_lengths: HOST arrays of n_res values; N a power of two in [256, 4096], 1 <= win <= N,
+ *   hop >= 1.
+ *   sums (DEVICE, B x n_res x 4 doubles, written asynchronously): sum (|Y|-|X|)^2, sum |Y|^2, sum |ln|X| - ln|Y||,
+ *   sum ||X| - |Y||.  SC = sqrt(s0)/sqrt(s1) (one ratio over all rows for a batch), LogMag = s2/(F (N/2+1)),
+ *   LinMag = s3/(F (N/2+1)).  A (row, resolution) whose window has count <= N/2 samples gets NaN sums (torch.stft
+ *   raises there).  One memset and one kernel launch per resolution; no allocation, no synchronisation.
+ */
+int ntm_mrstft_sums_rows(const float* out, int64_t ldo, const float* target, int64_t ldt, int64_t B, int64_t T,
+                         const int64_t* first, const int64_t* count, int n_res, const int* fft_sizes,
+                         const int* hop_sizes, const int* win_lengths, double* sums /* device, B x n_res x 4 */,
+                         int device, void* stream);
+
 /* Kernel-selection knob for tests and benchmarks.  The pair (streams_per_cta, ksplit) means, by mode:
  *   mode          pair                        runs
  *   any           (0, 0)                      automatic dispatch

@@ -1,7 +1,7 @@
 """ntm_b200 -- B200-native engine for the recurrent forward pass of neural-tape-modeling
 (GRU-HS[64] tape nonlinearity, DiffDelGRU delay line).  See DESIGN.md."""
 from . import driver, lib, sharding, signals  # noqa: F401
-from .losses import DCPreESR, ESRLoss  # noqa: F401
+from .losses import DCPreESR, ESRLoss, MultiResolutionSTFTLoss  # noqa: F401
 from .model import RNN, BlockStream, DiffDelRNN, RealtimeStream, TimeVaryingDelayLine  # noqa: F401
 
-__all__ = ["RNN", "BlockStream", "RealtimeStream", "DiffDelRNN", "TimeVaryingDelayLine", "ESRLoss", "DCPreESR", "driver", "lib", "sharding", "signals"]
+__all__ = ["RNN", "BlockStream", "RealtimeStream", "DiffDelRNN", "TimeVaryingDelayLine", "ESRLoss", "DCPreESR", "MultiResolutionSTFTLoss", "driver", "lib", "sharding", "signals"]

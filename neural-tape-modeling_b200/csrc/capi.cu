@@ -719,6 +719,28 @@ int ntm_esr_sums_rows(const float* out, int64_t ldo, const float* target, int64_
     return NTM_OK;
 }
 
+int ntm_mrstft_sums_rows(const float* out, int64_t ldo, const float* target, int64_t ldt, int64_t B, int64_t T,
+                         const int64_t* first, const int64_t* count, int n_res, const int* fft_sizes,
+                         const int* hop_sizes, const int* win_lengths, double* sums, int device, void* stream)
+{
+    if (B < 0 || T < 0 || n_res < 1 || !fft_sizes || !hop_sizes || !win_lengths || (B > 0 && !sums)) return NTM_EINVAL;
+    if (B > 0 && T > 0 && (!out || !target || ldo < T || ldt < T)) return NTM_EINVAL;
+    for (int r = 0; r < n_res; ++r) {
+        const int n = fft_sizes[r];
+        if (n < 256 || n > 4096 || (n & (n - 1)) || hop_sizes[r] < 1 || win_lengths[r] < 1 || win_lengths[r] > n)
+            return NTM_EINVAL;
+    }
+    if (B == 0) return NTM_OK;
+    DeviceGuard g(device);
+    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice);
+    int sms = 0;
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+    CU(ntm::launch_stft_loss(out, ldo, target, ldt, B, T, reinterpret_cast<const long long*>(first),
+                             reinterpret_cast<const long long*>(count), n_res, fft_sizes, hop_sizes, win_lengths, sums, sms,
+                             (cudaStream_t)stream));
+    return NTM_OK;
+}
+
 int ntm_gru_predict_host(void* handle, int mode, const float* x_host, float* y_host, float* h_host, int64_t B,
                          int64_t T, int skip, int64_t chunk_T)
 {

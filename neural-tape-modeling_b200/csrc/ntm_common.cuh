@@ -114,6 +114,12 @@ cudaError_t launch_esr(const float* out, long long ldo, const float* tgt, long l
                        int dc_pre, double* sums, int sm_count, cudaStream_t st, const long long* first = nullptr,
                        const long long* count = nullptr, int per_row = 0);
 
+// Multi-resolution STFT loss (stft.cu): sums[B][n_res][4], one memset and one launch per resolution; row b over samples
+// [first[b], first[b] + count[b]) as launch_esr.  fft_sizes / hop_sizes / win_lengths: HOST arrays, validated by the caller.
+cudaError_t launch_stft_loss(const float* out, long long ldo, const float* tgt, long long ldt, long long B, long long T,
+                             const long long* first, const long long* count, int n_res, const int* fft_sizes,
+                             const int* hop_sizes, const int* win_lengths, double* sums, int sm_count, cudaStream_t st);
+
 extern std::atomic<unsigned long long> g_launches;   // engine kernels launched by this process (ntm_query)
 
 // One-time per-device kernel configuration (cudaFuncSetAttribute) without mutable statics that race when several host

@@ -11,12 +11,14 @@
 //   ntm::diffdel_forward                   DiffDelRNN.forward, code/model.py:393-424
 //   ntm::delay_forward, ntm::delay_check   TimeVaryingDelayLine.forward, code/model.py:269-320 (assert :283)
 //   ntm::esr_sums, ntm::esr_sums_rows      ESRLoss / DCPreESR, CoreAudioML/training.py:5-16, GreyBoxDRC/loss_funcs.py:6-52
+//   ntm::mrstft_sums_rows                  auraloss MultiResolutionSTFTLoss (auraloss/freq.py), code/test-model.py:253
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
 #include <torch/library.h>
 #include <torch/types.h>
 
 #include <tuple>
+#include <vector>
 
 #include "../../include/ntm_b200.h"
 
@@ -170,6 +172,16 @@ Tensor esr_sums(const Tensor& out, const Tensor& target, bool dc_pre)
     return sums;
 }
 
+// first / count of the per-row ops: a contiguous int64 tensor of B values on the device of `like`, or None (nullptr)
+const int64_t* row_index(const c10::optional<Tensor>& v, int64_t B, const Tensor& like, const char* name)
+{
+    if (!v.has_value()) return nullptr;
+    TORCH_CHECK(v->is_cuda() && v->device() == like.device() && v->scalar_type() == at::kLong && v->is_contiguous() &&
+                    v->numel() == B,
+                "ntm_b200: ", name, " must be a contiguous int64 tensor of ", B, " values on ", like.device());
+    return v->data_ptr<int64_t>();
+}
+
 // per-row sums over samples [first[b], first[b] + count[b]) of row b (int64 CUDA tensors of B values, or None = whole rows)
 Tensor esr_sums_rows(const Tensor& out, const Tensor& target, const c10::optional<Tensor>& first,
                      const c10::optional<Tensor>& count, bool dc_pre)
@@ -177,18 +189,43 @@ Tensor esr_sums_rows(const Tensor& out, const Tensor& target, const c10::optiona
     const Rows o = rows(out, "output"), t = rows(target, "target");
     TORCH_CHECK(o.B == t.B && o.T == t.T && out.device() == target.device(), "ntm_b200: output ", out.sizes(), " and target ",
                 target.sizes(), " differ");
-    auto idx = [&](const c10::optional<Tensor>& v, const char* name) -> const int64_t* {
-        if (!v.has_value()) return nullptr;
-        TORCH_CHECK(v->is_cuda() && v->device() == out.device() && v->scalar_type() == at::kLong && v->is_contiguous() &&
-                        v->numel() == o.B,
-                    "ntm_b200: ", name, " must be a contiguous int64 tensor of ", o.B, " values on ", out.device());
-        return v->data_ptr<int64_t>();
-    };
     Tensor sums = at::empty({o.B, 2}, out.options().dtype(at::kDouble));
     const c10::cuda::CUDAGuard guard(out.device());
-    check_rc(ntm_esr_sums_rows(o.p, o.ld, t.p, t.ld, o.B, o.T, idx(first, "first"), idx(count, "count"), dc_pre ? 1 : 0,
-                               sums.data_ptr<double>(), out.get_device(), cur_stream(out)),
+    check_rc(ntm_esr_sums_rows(o.p, o.ld, t.p, t.ld, o.B, o.T, row_index(first, o.B, out, "first"),
+                               row_index(count, o.B, out, "count"), dc_pre ? 1 : 0, sums.data_ptr<double>(),
+                               out.get_device(), cur_stream(out)),
              "esr_sums_rows");
+    return sums;
+}
+
+// per-row, per-resolution sums of the multi-resolution STFT loss: (B, n_res, 4) doubles, windows as esr_sums_rows
+Tensor mrstft_sums_rows(const Tensor& out, const Tensor& target, const c10::optional<Tensor>& first,
+                        const c10::optional<Tensor>& count, at::IntArrayRef fft_sizes, at::IntArrayRef hop_sizes,
+                        at::IntArrayRef win_lengths)
+{
+    const Rows o = rows(out, "output"), t = rows(target, "target");
+    TORCH_CHECK(o.B == t.B && o.T == t.T && out.device() == target.device(), "ntm_b200: output ", out.sizes(), " and target ",
+                target.sizes(), " differ");
+    const size_t n = fft_sizes.size();
+    TORCH_CHECK(n > 0 && hop_sizes.size() == n && win_lengths.size() == n,
+                "ntm_b200: fft_sizes, hop_sizes and win_lengths must have the same non-zero length");
+    std::vector<int> fft(n), hop(n), win(n);
+    for (size_t r = 0; r < n; ++r) {
+        TORCH_CHECK(fft_sizes[r] >= 256 && fft_sizes[r] <= 4096 && (fft_sizes[r] & (fft_sizes[r] - 1)) == 0,
+                    "ntm_b200: fft sizes must be powers of two from 256 to 4096, got ", fft_sizes[r]);
+        TORCH_CHECK(win_lengths[r] >= 1 && win_lengths[r] <= fft_sizes[r], "ntm_b200: win_length ", win_lengths[r],
+                    " must be in [1, fft_size = ", fft_sizes[r], "]");
+        TORCH_CHECK(hop_sizes[r] >= 1 && hop_sizes[r] <= INT32_MAX, "ntm_b200: hop sizes must be >= 1, got ", hop_sizes[r]);
+        fft[r] = (int)fft_sizes[r];
+        hop[r] = (int)hop_sizes[r];
+        win[r] = (int)win_lengths[r];
+    }
+    Tensor sums = at::empty({o.B, (int64_t)n, 4}, out.options().dtype(at::kDouble));
+    const c10::cuda::CUDAGuard guard(out.device());
+    check_rc(ntm_mrstft_sums_rows(o.p, o.ld, t.p, t.ld, o.B, o.T, row_index(first, o.B, out, "first"),
+                                  row_index(count, o.B, out, "count"), (int)n, fft.data(), hop.data(), win.data(),
+                                  sums.data_ptr<double>(), out.get_device(), cur_stream(out)),
+             "mrstft_sums_rows");
     return sums;
 }
 
@@ -208,4 +245,7 @@ TORCH_LIBRARY(ntm, m)
     m.def("delay_check(Tensor d, int max_delay) -> bool", &delay_check);
     m.def("esr_sums(Tensor output, Tensor target, bool dc_pre) -> Tensor", &esr_sums);
     m.def("esr_sums_rows(Tensor output, Tensor target, Tensor? first, Tensor? count, bool dc_pre) -> Tensor", &esr_sums_rows);
+    m.def("mrstft_sums_rows(Tensor output, Tensor target, Tensor? first, Tensor? count, int[] fft_sizes, int[] hop_sizes, "
+          "int[] win_lengths) -> Tensor",
+          &mrstft_sums_rows);
 }

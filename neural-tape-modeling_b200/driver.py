@@ -4,9 +4,9 @@ Replaces the per-file loop of the reference's evaluation flow (code/test-model.p
 losses, :882-893 .wav output) and the segment reads of code/dataset.py:348-379 (`torchaudio.load(file, num_frames=length,
 frame_offset=offset, normalize=False)`): examples are packed into one zero-padded (B, 1, T_max) batch -- the model is
 causal, so trailing padding never changes a real sample --, predicted with predict() semantics per stream (zero state,
-1024-sample warm start), cut by INIT_LEN, scored on the device (ESR / DCPreESR) and optionally written back as float32
-.wav files.  The on-disk format is the reference's: float32 (or PCM) RIFF/WAVE, channel 0 = audio, channel 1 (if any) =
-the 100 Hz pulse track (SURVEY.md section 8f rank 4).  No soundfile / torchaudio needed.
+1024-sample warm start), cut by INIT_LEN, scored on the device (ESR / DCPreESR, optionally MR-STFT) and optionally
+written back as float32 .wav files.  The on-disk format is the reference's: float32 (or PCM) RIFF/WAVE, channel 0 = audio,
+channel 1 (if any) = the 100 Hz pulse track (SURVEY.md section 8f rank 4).  No soundfile / torchaudio needed.
 
 All three prediction modes of the reference's loss loop (code/test-model.py:346-368) are covered: plain GRU, DiffDelGRU
 with the example's delay trajectory (`meta['delay_trajectory'] * fs`, :349-352), and GRU followed by the stand-alone delay
@@ -19,7 +19,7 @@ import struct
 import numpy as np
 import torch
 
-from .losses import DCPreESR, ESRLoss
+from .losses import DCPreESR, ESRLoss, MultiResolutionSTFTLoss
 
 _PCM, _FLOAT, _EXTENSIBLE = 1, 3, 0xFFFE
 
@@ -111,7 +111,7 @@ def read_trajectory(path, offset=0, length=-1):
     return a[int(offset):end]
 
 
-def mean_losses(results, keys=("ESR", "DCPreESR")):
+def mean_losses(results, keys=("ESR", "DCPreESR", "MR-STFT")):
     """Dataset mean of the per-example losses = the reference's `results_dict[key] / num_batches` with batch size 1
     (code/test-model.py:385-397)."""
     return {k: float(np.mean([r[k] for r in results])) for k in keys if results and all(k in r for r in results)}
@@ -126,15 +126,18 @@ class BatchedEvaluator:
     (`trajectory_*.npy`, sliced with the example's offset / length).
     `model` is an ntm_b200.RNN or DiffDelRNN on a CUDA device; `delay` is an optional stand-alone
     ntm_b200.TimeVaryingDelayLine applied after a plain RNN (the reference's ADD_DELAY); `max_streams` examples are
-    packed per launch."""
+    packed per launch.  `mrstft=True` adds the reference's third loss, auraloss `MultiResolutionSTFTLoss()`
+    (code/test-model.py:253), as r['MR-STFT'], over the same window and in the same per-group pass."""
 
-    def __init__(self, model, max_streams=1024, delay=None):
+    def __init__(self, model, max_streams=1024, delay=None, mrstft=False):
         from .model import DiffDelRNN
         self.model, self.max_streams, self.delay = model, int(max_streams), delay
         self.diffdel = isinstance(model, DiffDelRNN)
         if self.diffdel and delay is not None:
             raise ValueError("ADD_DELAY applies to the plain GRU only (code/test-model.py:354)")
         self.losses = {"ESR": ESRLoss(), "DCPreESR": DCPreESR(dc_pre=True)}
+        if mrstft:
+            self.losses["MR-STFT"] = MultiResolutionSTFTLoss()
 
     @staticmethod
     def _load(ex, key):
@@ -163,7 +166,7 @@ class BatchedEvaluator:
         return self.delay(y, d)
 
     def run(self, examples, out_dir=None, init_len=0, write_pre_d=False):
-        """-> one dict per example: {'input_name', 'frames', 'fs', ['ESR', 'DCPreESR',] ['output_file']}; losses are
+        """-> one dict per example: {'input_name', 'frames', 'fs', ['ESR', 'DCPreESR', ['MR-STFT',]] ['output_file']}; losses are
         computed after cutting the first `init_len` samples (INIT_LEN, code/test-model.py:323-325,367-370)."""
         dev = self.model._device()
         need_d = self.diffdel or self.delay is not None

@@ -50,6 +50,7 @@ SIGNATURES = {
     "ntm_rt_process": (_int, [_vp, _vp, _vp]),
     "ntm_rt_close": (_int, [_vp, _vp]),
     "ntm_esr_sums": (_int, [_vp, _i64, _vp, _i64, _i64, _i64, _int, _vp, _int, _vp]),
+    "ntm_mrstft_sums_rows": (_int, [_vp, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _int, _vp, _vp, _vp, _vp, _int, _vp]),
 }
 
 _lib = None
