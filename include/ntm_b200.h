@@ -38,7 +38,7 @@ extern "C" {
 #define NTM_ENOMEM       (-3)
 #define NTM_ECUDA        (-4)   /* a CUDA runtime call failed: see ntm_last_cuda_error() */
 #define NTM_EDELAY       (-5)   /* a delay value exceeds the history length D (the reference's assert,
-                                   code/model.py:283) -- only returned by ntm_delay_check */
+                                   code/model.py:283) -- returned by ntm_delay_check and ntm_rt_diffdel_process */
 #define NTM_ENODEVICE    (-6)   /* no CUDA device / not an sm_100 device */
 #define NTM_ECLOSED      (-7)   /* real-time stream: the resident kernel has left (closed or idle timeout) */
 
@@ -135,6 +135,23 @@ int ntm_rt_open(void* handle, int mode, const float* h_host, int64_t B, int64_t 
                 int idle_timeout_ms, void** rt);
 int ntm_rt_process(void* rt, const float* x_host, float* y_host);
 int ntm_rt_close(void* rt, float* h_host_out);
+
+/*
+ * The same resident server for the full tape model (DiffDelRNN.forward, code/model.py:393-424, on consecutive blocks with
+ * self.hidden and the delay history carried): GRU, head and the wow/flutter delay line in one persistent CTA.  The last
+ * D + 128 or more samples of pre_d stay in an on-chip ring across blocks, so each block's y and pre_d are bit-identical to
+ * one long ntm_diffdel_forward call over the concatenated signal.  hist_host: B x D initial delay history
+ * (TimeVaryingDelayLine.buffer) or NULL (zeros).  The ring must fit on chip: D <= 32639 for one stream, <= 16255 for two,
+ * <= 8063 for three or four (NTM_EUNSUPPORTED beyond).  check_delay != 0: ntm_rt_diffdel_process checks the block's
+ * delays on the host first, and a block with any d > D or NaN returns NTM_EDELAY without being handed over (state and
+ * history unchanged).  x_host, d_host, y_host, pre_d_host (NULL: not returned): B x block_len contiguous HOST floats.
+ * ntm_rt_diffdel_close stops the kernel and returns the final state (B x 64) and the rolled history (B x D), either NULL to
+ * skip.  Limits, modes, idle timeout and handle reference as ntm_rt_open.
+ */
+int ntm_rt_diffdel_open(void* handle, int mode, const float* h_host, const float* hist_host, int64_t B,
+                        int64_t block_len, int64_t D, int skip, int check_delay, int idle_timeout_ms, void** rt);
+int ntm_rt_diffdel_process(void* rt, const float* x_host, const float* d_host, float* y_host, float* pre_d_host);
+int ntm_rt_diffdel_close(void* rt, float* h_host_out, float* hist_host_out);
 
 /*
  * Evaluation losses on the device (the step right after the recurrent path, code/test-model.py:250-253,386-388).

@@ -2,6 +2,7 @@
 (GRU-HS[64] tape nonlinearity, DiffDelGRU delay line).  See DESIGN.md."""
 from . import driver, lib, sharding, signals  # noqa: F401
 from .losses import DCPreESR, ESRLoss, MultiResolutionSTFTLoss  # noqa: F401
-from .model import RNN, BlockStream, DiffDelRNN, RealtimeStream, TimeVaryingDelayLine  # noqa: F401
+from .model import (RNN, BlockStream, DelayBlockStream, DiffDelRNN, RealtimeDelayStream, RealtimeStream,  # noqa: F401
+                    TimeVaryingDelayLine)
 
-__all__ = ["RNN", "BlockStream", "RealtimeStream", "DiffDelRNN", "TimeVaryingDelayLine", "ESRLoss", "DCPreESR", "MultiResolutionSTFTLoss", "driver", "lib", "sharding", "signals"]
+__all__ = ["RNN", "BlockStream", "RealtimeStream", "DiffDelRNN", "DelayBlockStream", "RealtimeDelayStream", "TimeVaryingDelayLine", "ESRLoss", "DCPreESR", "MultiResolutionSTFTLoss", "driver", "lib", "sharding", "signals"]

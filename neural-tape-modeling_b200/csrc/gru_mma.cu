@@ -54,12 +54,17 @@ struct MmaCfg {
 // costs two PCIe round trips instead of a kernel launch, a prologue and a stream synchronisation.
 // DEFER (HALF only): the output head's accumulators are consumed one iteration later (see the head block); wins when a
 // warp has its SM sub-partition to itself (one CTA per SM: cfg 3, cfg 5, the real-time server), loses otherwise.
-template <int FMT, bool HALF, bool RT = false, bool DEFER = RT, bool SPLIT = false>
+// RTD (RT only): the DiffDelRNN server (a.rtd, RtDelayMailbox) -- each block also brings its delay trajectory and returns
+// pre_d next to y.  The pre_d ring persists across blocks on the time axis of a 64-bit sample counter since open (the
+// carried history at -D .. -1), so every block's y is the one long fused call's, bit for bit; the rolled history is read
+// back from the ring when the server leaves.
+template <int FMT, bool HALF, bool RT = false, bool DEFER = RT, bool SPLIT = false, bool RTD = false>
 // (HALF is only dispatched up to two CTAs per SM: the full register file removes its spills, 197 vs 204 ns/step; the
 // strict form keeps two sets of weight fragments in registers)
 __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 4) gru_mma_kernel(const GruArgs a)
 {
     static_assert(!RT || HALF, "the real-time server uses the 4-streams-per-CTA form");
+    static_assert(!RTD || RT, "the DiffDelRNN server is a form of the real-time server");
     static_assert(!SPLIT || (FMT == FMT_F16 && !DEFER), "the strict form: f16 pairs, immediate head");
     constexpr int NP = SPLIT ? 2 : 1;                // operand parts (hi, lo')
     constexpr int SL = SPLIT ? 1 : 0;                // accumulators per tile: W_hi h_hi | (strict) W_hi h_lo' , W_lo' h_hi
@@ -242,7 +247,11 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
 
     __shared__ __align__(16) float rt_xblk[RT ? RT_MAXSTREAMS * RT_MAXBLK : 4];   // server form: one block of x ...
     __shared__ __align__(16) float rt_yblk[RT ? RT_MAXSTREAMS * RT_MAXBLK : 4];   // ... and of y, staged on chip
-    const bool delay = a.d != nullptr;
+    // DiffDelRNN server: the block's d and pre_d stage in the trajectory staging `ds`, which this form does not use otherwise
+    static_assert(2 * RT_MAXSTREAMS * RT_MAXBLK <= 2 * CH * S, "the server's d and pre_d blocks fit in ds");
+    float* const rt_dblk = ds;
+    float* const rt_pblk = ds + RT_MAXSTREAMS * RT_MAXBLK;
+    const bool delay = RTD || a.d != nullptr;
     float* __restrict__ head_out = delay ? a.pre : a.y;
     const long long ldo = delay ? a.ldp : a.ldy;
 
@@ -263,7 +272,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
     };
 
     const int rmask = a.ring_len - 1;
-    const bool use_ring = delay && !a.warmup && a.ring_len > 0;
+    const bool use_ring = RTD || (delay && !a.warmup && a.ring_len > 0);
     auto load_d = [&](int buf, long long t0) {               // the chunk's delay trajectory, staged like x
         const int n = (int)((a.T - t0) < (long long)CH ? (a.T - t0) : (long long)CH);
         float* dstb = ds + buf * CH * S;
@@ -291,6 +300,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
     const long long nchunks = (a.T + CH - 1) / CH;
     int cur = 0;
     unsigned rt_seen = 0;
+    long long rt_pos = 0;                      // DiffDelRNN server: samples since open, the ring's time axis
     __shared__ unsigned rt_flag;
     do {
     if (RT) {
@@ -299,7 +309,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
             unsigned long long t_wait;
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_wait));
             unsigned sq;
-            while ((sq = a.rt->seq_in) == rt_seen) {
+            while ((sq = RTD ? a.rtd->seq_in : a.rt->seq_in) == rt_seen) {
                 unsigned long long now;
                 asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
                 if (now - t_wait > a.rt_idle_ns) { sq = RT_STOP; break; }
@@ -310,7 +320,24 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         if (rt_flag == RT_STOP) break;
         rt_seen = rt_flag;
         // fetch the block: every thread keeps up to 8 uncached loads of mapped host memory in flight (one round trip)
-        {
+        if (RTD) {                             // (x and d: 16 loads in the same round trip)
+            const int total = ns * (int)a.T;
+            float v[8], w[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const int idx = tid + 128 * i;
+                v[i] = idx < total ? __ldcv(a.x + (idx / (int)a.T) * a.ldx + idx % (int)a.T) : 0.0f;
+                w[i] = idx < total ? __ldcv(a.d + (idx / (int)a.T) * a.ldd + idx % (int)a.T) : 0.0f;
+            }
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const int idx = tid + 128 * i;
+                if (idx < total) {
+                    rt_xblk[(idx / (int)a.T) * RT_MAXBLK + idx % (int)a.T] = v[i];
+                    rt_dblk[(idx / (int)a.T) * RT_MAXBLK + idx % (int)a.T] = w[i];
+                }
+            }
+        } else {
             const int total = ns * (int)a.T;
             float v[8];
 #pragma unroll
@@ -327,7 +354,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         __syncthreads();
     }
     load_x(0, 0);
-    if (use_ring) load_d(0, 0);
+    if (use_ring && !RTD) load_d(0, 0);
     for (long long c = 0; c < nchunks; ++c) {
         const long long t0 = c * CH;
         const int n = (int)((a.T - t0) < (long long)CH ? (a.T - t0) : (long long)CH);
@@ -337,7 +364,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         __syncthreads();                       // xs[xb] landed; state tile `cur` complete; previous flush done
         if (c + 1 < nchunks) {
             load_x(xb ^ 1, t0 + CH);
-            if (use_ring) load_d(xb ^ 1, t0 + CH);
+            if (use_ring && !RTD) load_d(xb ^ 1, t0 + CH);
         }
 
         float hpend[4];
@@ -495,13 +522,29 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
                 float v = yp[tt * C::YP_LD + col] + yp[(CH + tt) * C::YP_LD + col] + yp[(2 * CH + tt) * C::YP_LD + col] +
                           yp[(3 * CH + tt) * C::YP_LD + col] + bo;
                 if (a.skip) v += xcur[tt * S + col];
+                if (RTD) {
+                    rt_pblk[s * RT_MAXBLK + t0 + tt] = v;
+                    ring[s * a.ring_len + ((int)(rt_pos + t0 + tt) & rmask)] = v;
+                    continue;
+                }
                 if (RT) rt_yblk[s * RT_MAXBLK + t0 + tt] = v;
                 else head_out[(b0 + s) * ldo + t0 + tt] = v;
                 if (delay && a.warmup) a.y[(b0 + s) * a.ldy + t0 + tt] = v;
                 if (use_ring) ring[s * a.ring_len + ((int)(t0 + tt) & rmask)] = v;
             }
         }
-        if (use_ring) {
+        if (RTD) {
+            // the same delay read on the server's time axis; the block's y stages next to x
+            __syncthreads();
+            for (int idx = tid; idx < SC * CH; idx += 128) {
+                const int s = idx / CH, tt = idx % CH;
+                if (s < ns && tt < n) {
+                    const float* rrow = ring + s * a.ring_len;
+                    rt_yblk[s * RT_MAXBLK + t0 + tt] = delay_read(rt_dblk[s * RT_MAXBLK + t0 + tt], rt_pos + t0 + tt, a.D,
+                                                                  [&](long long i) { return rrow[(int)i & rmask]; });
+                }
+            }
+        } else if (use_ring) {
             // delay taps from the on-chip ring (the last ring_len >= D + CH samples of pre_d, history included) and the
             // staged trajectory: no L2 round trip of the samples this CTA has just produced
             __syncthreads();
@@ -526,11 +569,19 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         // the block's output goes out in full 128-byte lines (a warp writes 32 consecutive samples of one stream)
         for (int idx = tid; idx < ns * RT_MAXBLK; idx += 128) {
             const int sidx = idx / RT_MAXBLK, t = idx % RT_MAXBLK;
-            if (t < (int)a.T) a.y[sidx * a.ldy + t] = rt_yblk[sidx * RT_MAXBLK + t];
+            if (t < (int)a.T) {
+                a.y[sidx * a.ldy + t] = rt_yblk[sidx * RT_MAXBLK + t];
+                if (RTD) a.pre[sidx * a.ldp + t] = rt_pblk[sidx * RT_MAXBLK + t];
+            }
         }
-        __threadfence_system();                // this block's y is visible to the host ...
+        __threadfence_system();                // this block's y (and pre_d) is visible to the host ...
         __syncthreads();
-        if (tid == 0) a.rt->seq_out = rt_seen; // ... before its sequence number is
+        if (RTD) {                             // ... before its sequence number is
+            if (tid == 0) a.rtd->seq_out = rt_seen;
+            rt_pos += a.T;
+        } else {
+            if (tid == 0) a.rt->seq_out = rt_seen;
+        }
     }
     } while (RT);
 
@@ -542,7 +593,13 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
             const int s = (2 * tig + e) / CS;
             if (s < ns) a.h_out[(b0 + s) * 64 + u0 + u] = hst[u][e];
         }
-    if (delay) {
+    if (RTD) {                                 // rolled history: ring positions rt_pos - D .. rt_pos - 1
+        __syncthreads();
+        for (long long idx = tid; idx < (long long)ns * a.D; idx += 128) {
+            const int s = (int)(idx / a.D), i = (int)(idx % a.D);
+            a.hist_out[(b0 + s) * (long long)a.D + i] = ring[s * a.ring_len + ((int)(rt_pos - a.D + i) & rmask)];
+        }
+    } else if (delay) {
         __syncthreads();
         delay_roll_history<128>(a, b0, ns, tid);
     }
@@ -567,14 +624,19 @@ cudaError_t launch_mma_one(const GruArgs& a, cudaStream_t st)
     return cudaGetLastError();
 }
 
-template <int FMT, bool SPLIT = false>
+template <int FMT, bool SPLIT = false, bool RTD = false>
 cudaError_t launch_mma_rt_fmt(const GruArgs& a, cudaStream_t st)
 {
     using C = MmaCfg<FMT, SPLIT>;
-    cudaError_t e = cudaFuncSetAttribute(gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
+    GruArgs b = a;
+    b.ring_len = RTD ? rt_delay_ring_len(a.B, a.D) : 0;
+    if (RTD && b.ring_len == 0) return cudaErrorInvalidValue;
+    const int ring_bytes = (int)(b.B * b.ring_len * 4);
+    cudaError_t e = cudaFuncSetAttribute(gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT, RTD>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         C::SMEM_BYTES + (RTD ? RT_RING_BUDGET : 0));
     if (e != cudaSuccess) return e;
-    gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT><<<1, 128, C::SMEM_BYTES, st>>>(a);
+    gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT, RTD><<<1, 128, C::SMEM_BYTES + ring_bytes, st>>>(b);
     ++g_launches;
     return cudaGetLastError();
 }
@@ -613,6 +675,26 @@ cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st)
         case FMT_TF32: return launch_mma_rt_fmt<FMT_TF32>(a, st);
         case FMT_BF16: return launch_mma_rt_fmt<FMT_BF16>(a, st);
         default: return launch_mma_rt_fmt<FMT_F16>(a, st);
+    }
+}
+
+int rt_delay_ring_len(long long B, long long D)
+{
+    const long long rl = delay_ring_len(D, MmaCfg<FMT_F16>::CH);
+    return B * rl * 4 <= RT_RING_BUDGET ? (int)rl : 0;
+}
+
+// The DiffDelRNN server (a.rtd; a.x, a.d, a.y, a.pre point into it; hist_in / hist_out: B x D, may alias).
+cudaError_t launch_gru_mma_rt_delay(const GruArgs& a, int fmt, cudaStream_t st)
+{
+    if (a.B <= 0 || a.B > RT_MAXSTREAMS || a.T <= 0 || a.T > RT_MAXBLK || !a.rtd || !a.d || !a.pre || a.warmup || a.D < 0 ||
+        (a.D > 0 && (!a.hist_in || !a.hist_out)))
+        return cudaErrorInvalidValue;
+    switch (fmt) {
+        case FMT_F16X3: return launch_mma_rt_fmt<FMT_F16, true, true>(a, st);
+        case FMT_TF32: return launch_mma_rt_fmt<FMT_TF32, false, true>(a, st);
+        case FMT_BF16: return launch_mma_rt_fmt<FMT_BF16, false, true>(a, st);
+        default: return launch_mma_rt_fmt<FMT_F16, false, true>(a, st);
     }
 }
 

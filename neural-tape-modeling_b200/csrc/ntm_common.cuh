@@ -51,6 +51,19 @@ struct RtMailbox {
     float y[RT_MAXSTREAMS][RT_MAXBLK];
 };
 
+// Mailbox of a real-time DiffDelRNN stream (ntm_rt_diffdel_*; gru_mma.cu, RT + delay form): the same handshake, with the
+// block's delay trajectory d next to x and the head output before the delay (pre) next to y.
+struct RtDelayMailbox {
+    volatile unsigned seq_in;
+    unsigned pad0[31];
+    float x[RT_MAXSTREAMS][RT_MAXBLK];
+    float d[RT_MAXSTREAMS][RT_MAXBLK];
+    volatile unsigned seq_out;
+    unsigned pad1[31];
+    float y[RT_MAXSTREAMS][RT_MAXBLK];
+    float pre[RT_MAXSTREAMS][RT_MAXBLK];
+};
+
 // Arguments of one recurrent launch; d == nullptr selects the plain RNN.forward path.
 struct GruArgs {
     const float* blob;
@@ -69,7 +82,10 @@ struct GruArgs {
     int ring_len;                   // DiffDelRNN, mma.sync kernels: samples of pre_d kept per stream in shared memory (power
                                     // of two >= D + chunk + 1, size_delay_ring; 0: read the delay taps back through L2)
     int sm_count;                   // SMs of the handle's device (host-side dispatch only)
-    RtMailbox* rt;                  // real-time server form only (x, y point into it)
+    union {                         // real-time server forms only:
+        RtMailbox* rt;              //   RNN (x, y point into it)
+        RtDelayMailbox* rtd;        //   DiffDelRNN (x, d, y, pre point into it)
+    };
     unsigned long long rt_idle_ns;  // the server leaves after this long without a block
 };
 
@@ -97,6 +113,10 @@ cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_he
 cudaError_t launch_gru_mma4(const GruArgs& a, int fmt, cudaStream_t st);   // GRU and DiffDelGRU, f16 / bf16 / strict f16x3, four
                                                                              // streams per CTA, 4x unrolled
 cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st);    // resident real-time server, <= 4 streams
+// The same server for DiffDelRNN (a.rtd).  rt_delay_ring_len: its pre_d ring per stream for B streams and history length D, or
+// 0 if the ring does not fit RT_RING_BUDGET (the launcher then refuses the launch).
+cudaError_t launch_gru_mma_rt_delay(const GruArgs& a, int fmt, cudaStream_t st);
+int rt_delay_ring_len(long long B, long long D);
 void pack_tc_images(float* blob_host);   // host: fills BlobLayout::IMG_* from the fp32 part of the blob
 cudaError_t launch_delay(const float* x, long long ldx, const float* d, long long ldd, float* y, long long ldy,
                          const float* hist_in, float* hist_out, long long B, long long T, long long D, int warmup,
@@ -165,13 +185,22 @@ __device__ __forceinline__ float delay_read(float dt, long long t, int D, LoadPa
 // and chunks of `chunk` steps: the last ring_len samples of pre_d per stream, ring_len the smallest power of two (>= 64)
 // that is >= D + chunk + 1, stay in shared memory if they fit in DELAY_RING_BUDGET bytes per CTA (so that four CTAs still
 // share an SM); longer histories read their taps back through L2.  Sets b.ring_len (0: no ring) and returns the ring's bytes.
+// The real-time DiffDelRNN server is one CTA on an SM of its own and keeps its ring across blocks in up to RT_RING_BUDGET
+// bytes: with its 128-step chunks, ring_len 32768 (D <= 32639) for one stream, 16384 (D <= 16255) for two, 8192 (D <= 8063)
+// for three or four.  Its total shared memory stays under the 227 KB a CTA may opt into.
 constexpr int DELAY_RING_BUDGET = 48 * 1024;
+constexpr int RT_RING_BUDGET = 128 * 1024;
+inline long long delay_ring_len(long long D, int chunk)
+{
+    long long rl = 64;
+    while (rl < D + chunk + 1) rl *= 2;
+    return rl;
+}
 inline int size_delay_ring(GruArgs& b, int streams, int chunk)
 {
     b.ring_len = 0;
     if (b.d == nullptr || b.warmup) return 0;
-    long long rl = 64;
-    while (rl < (long long)b.D + chunk + 1) rl *= 2;
+    const long long rl = delay_ring_len(b.D, chunk);
     if (rl * streams * 4 > DELAY_RING_BUDGET) return 0;
     b.ring_len = (int)rl;
     return (int)(rl * streams * 4);

@@ -49,6 +49,9 @@ SIGNATURES = {
     "ntm_rt_open": (_int, [_vp, _int, _vp, _i64, _i64, _int, _int, ctypes.POINTER(_vp)]),
     "ntm_rt_process": (_int, [_vp, _vp, _vp]),
     "ntm_rt_close": (_int, [_vp, _vp]),
+    "ntm_rt_diffdel_open": (_int, [_vp, _int, _vp, _vp, _i64, _i64, _i64, _int, _int, _int, ctypes.POINTER(_vp)]),
+    "ntm_rt_diffdel_process": (_int, [_vp, _vp, _vp, _vp, _vp]),
+    "ntm_rt_diffdel_close": (_int, [_vp, _vp, _vp]),
     "ntm_esr_sums": (_int, [_vp, _i64, _vp, _i64, _i64, _i64, _int, _vp, _int, _vp]),
     "ntm_mrstft_sums_rows": (_int, [_vp, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _int, _vp, _vp, _vp, _vp, _int, _vp]),
 }

@@ -528,3 +528,172 @@ class DiffDelRNN(RNN):
         self.hidden = self._from_engine(h.reshape(1, B, ENGINE_H)).to(dev)
         self.diffdel.buffer = hist.reshape(B, 1, D).to(dev)
         return y, pre
+
+    def block_stream(self, n_streams=1, block_len=64):
+        """Real-time block mode of the full tape model: consecutive `forward(x, d)` calls on short blocks with state and
+        delay history carried on the device, one C call per block -- see DelayBlockStream."""
+        return DelayBlockStream(self, n_streams, block_len)
+
+    def realtime_stream(self, n_streams=1, block_len=64, idle_timeout_ms=5000):
+        """Real-time block mode of the full tape model with a resident kernel (host blocks in, host blocks out) -- see
+        RealtimeDelayStream."""
+        return RealtimeDelayStream(self, n_streams, block_len, idle_timeout_ms)
+
+
+class DelayBlockStream:
+    """Block-by-block DiffDelRNN processing of `n_streams` streams with the state and the delay history carried on the
+    device.
+
+    Semantically identical to calling `model(x_block, d_block)` repeatedly (code/model.py:393-424 with `self.hidden` and
+    `self.diffdel.buffer` carried): both start from the model (`initialize_hidden(B, max_D)`, `warm_start()` and a
+    broadcast to B streams first give `predict()` semantics) and are written back by `close()`.  Buffers, raw pointers, the
+    handle and the CUDA stream are resolved once, so a block costs one ctypes call + one kernel launch; the history
+    alternates between two device buffers because the kernel's hist_out must not alias its hist_in.  When
+    `model.diffdel.check_delay` is set (the default), every block first runs the reference's delay assert, which
+    synchronises the stream once per block; a refused block raises AssertionError and changes nothing."""
+
+    def __init__(self, model, n_streams, block_len):
+        dev = model._device()
+        if dev.type != "cuda":
+            raise RuntimeError("ntm_b200 has no CPU path; move the model to a CUDA device")
+        self.model, self.B, self.T, self.device = model, int(n_streams), int(block_len), dev
+        self._handle = ctypes.c_void_p(model._handle(dev))
+        self._generation = model._engine.generation
+        self._mode = _lib.MODES[model.mode]
+        self._skip = int(bool(model.skip))
+        self.D = int(model.diffdel.max_delay)
+        h = model._hidden_in(self.B, dev)
+        self.h = torch.zeros((1, self.B, ENGINE_H), dtype=torch.float32, device=dev) if h is None else h.clone()
+        hist = model.diffdel._history(self.B, dev)
+        self.hist = (hist.clone(), torch.empty_like(hist))
+        self._cur = 0                                       # self.hist[_cur] holds the carried history
+        self.y = torch.empty((self.B, 1, self.T), dtype=torch.float32, device=dev)
+        self.pre_d = torch.empty((self.B, 1, self.T), dtype=torch.float32, device=dev)
+        L = _lib.load()
+        self._fn, self._check = L.ntm_diffdel_forward, L.ntm_delay_check
+        self._hp = ctypes.c_void_p(self.h.data_ptr())
+        self._histp = tuple(ctypes.c_void_p(t.data_ptr()) for t in self.hist)
+        self._st = _stream(dev)
+
+    def process(self, x, d, out=None, out_pre_d=None):
+        """x, d (n_streams, 1, block_len) float32 on the model's device -> (y, pre_d): the internal buffers, overwritten
+        by the next call, or `out` / `out_pre_d`.  Asynchronous on the stream that was current when the stream was
+        created, except for the delay check."""
+        for t, name in ((x, "x"), (d, "d")):
+            if t.dtype != torch.float32 or not t.is_cuda or t.dim() != 3 or t.shape[0] != self.B or t.shape[1] != 1 \
+                    or t.shape[2] > self.T or t.stride(2) != 1:
+                raise RuntimeError(f"{name}: expected a float32 CUDA block of shape ({self.B}, 1, <= {self.T})")
+        if d.shape != x.shape:
+            raise RuntimeError(f"x {tuple(x.shape)} and d {tuple(d.shape)} must have the same shape")
+        T = x.shape[2]
+
+        def ld(t):
+            return t.stride(0) if self.B > 1 else max(T, 1)
+        if self._generation != self.model._engine.generation:     # parameters were re-packed: the old handle is gone
+            self._handle = ctypes.c_void_p(self.model._handle(self.device))
+            self._generation = self.model._engine.generation
+        dp = ctypes.c_void_p(d.data_ptr())
+        if self.model.diffdel.check_delay and T > 0:
+            rc = self._check(dp, ld(d), self.B, T, self.D, self.device.index, self._st)
+            if rc:
+                _lib.check(rc)
+        y = self.y if out is None else out
+        pre = self.pre_d if out_pre_d is None else out_pre_d
+        rc = self._fn(self._handle, self._mode, ctypes.c_void_p(x.data_ptr()), ld(x), dp, ld(d),
+                      ctypes.c_void_p(y.data_ptr()), ld(y), ctypes.c_void_p(pre.data_ptr()), ld(pre), self._hp, self._hp,
+                      self._histp[self._cur], self._histp[self._cur ^ 1], self.B, T, self.D, 0, self._skip, self._st)
+        if rc:
+            _lib.check(rc)
+        self._cur ^= 1
+        if T != y.shape[2]:
+            y, pre = y[:, :, :T], pre[:, :, :T]
+        return y, pre
+
+    def close(self):
+        """Hand the carried state and delay history back to the model (`model.hidden`, `model.diffdel.buffer`)."""
+        self.model.hidden = self.model._from_engine(self.h)
+        self.model.diffdel.buffer = self.hist[self._cur]
+        return self.model.hidden, self.model.diffdel.buffer
+
+
+class RealtimeDelayStream:
+    """Block-by-block DiffDelRNN processing of up to 4 streams through a RESIDENT server kernel (ntm_rt_diffdel_*,
+    csrc/gru_mma.cu RT + delay form).
+
+    Same semantics as DelayBlockStream / repeated `model(x_block, d_block)` calls with `self.hidden` and
+    `self.diffdel.buffer` carried (code/model.py:393-424), with the blocks in HOST memory like RealtimeStream: the GRU,
+    the head and the wow/flutter delay line run in one persistent CTA that keeps the last samples of pre_d on chip across
+    blocks.  `process(x, d)` takes float32 host tensors or numpy arrays of shape (n_streams, block_len) [or (n_streams, 1,
+    block_len)] and returns host (y, pre_d) of the same shape.  State and history start from the model and are handed back
+    by `close()`.  The history length D = `model.diffdel.max_delay` must fit the on-chip ring: D <= 32639 for one stream,
+    16255 for two, 8063 for three or four.  The delay assert (`model.diffdel.check_delay`, read at open) runs on the host
+    copy of each block, without a device synchronisation; a refused block raises AssertionError and changes nothing.
+    Tensor-core modes only.  While the stream is open do not synchronise the whole device: the resident kernel only ends
+    at `close()` or after `idle_timeout_ms` without a block."""
+
+    def __init__(self, model, n_streams=1, block_len=64, idle_timeout_ms=5000):
+        dev = model._device()
+        if dev.type != "cuda":
+            raise RuntimeError("ntm_b200 has no CPU path; move the model to a CUDA device")
+        self.model, self.B, self.T, self.device = model, int(n_streams), int(block_len), dev
+        self.D = int(model.diffdel.max_delay)
+        h = model._hidden_in(self.B, dev)
+        h_host = None if h is None else h.reshape(self.B, ENGINE_H).to("cpu", torch.float32).contiguous()
+        hist_host = model.diffdel._history(self.B, dev).reshape(self.B, self.D).to("cpu").contiguous()
+        torch.cuda.current_stream(dev).synchronize()         # state and history are final before the server reads them
+        self._rt = ctypes.c_void_p()
+        rc = _lib.load().ntm_rt_diffdel_open(model._handle(dev), _lib.MODES[model.mode], _ptr(h_host), _ptr(hist_host),
+                                             self.B, self.T, self.D, int(bool(model.skip)),
+                                             int(bool(model.diffdel.check_delay)), int(idle_timeout_ms),
+                                             ctypes.byref(self._rt))
+        _lib.check(rc)
+        self._y = torch.empty((self.B, self.T), dtype=torch.float32)
+        self._pre = torch.empty((self.B, self.T), dtype=torch.float32)
+        self._fn = _lib.load().ntm_rt_diffdel_process
+        self._yp = ctypes.c_void_p(self._y.data_ptr())
+        self._pp = ctypes.c_void_p(self._pre.data_ptr())
+        self.x_in = torch.zeros((self.B, self.T), dtype=torch.float32)       # optional fixed input blocks for step()
+        self.d_in = torch.zeros((self.B, self.T), dtype=torch.float32)
+        self._xp = ctypes.c_void_p(self.x_in.data_ptr())
+        self._dp = ctypes.c_void_p(self.d_in.data_ptr())
+
+    def step(self):
+        """Lowest-overhead form: process the blocks the caller wrote into `self.x_in` / `self.d_in`; returns the internal
+        (y, pre_d) blocks (overwritten by the next call)."""
+        rc = self._fn(self._rt, self._xp, self._dp, self._yp, self._pp)
+        if rc:
+            _lib.check(rc)
+        return self._y, self._pre
+
+    def process(self, x, d):
+        if self._rt is None:
+            raise RuntimeError("ntm_b200: real-time stream is closed")
+        xt, dt = torch.as_tensor(x), torch.as_tensor(d)
+        for t in (xt, dt):
+            if t.is_cuda or t.dtype != torch.float32 or t.numel() != self.B * self.T or not t.is_contiguous():
+                raise RuntimeError(f"expected contiguous float32 HOST blocks of {self.B} x {self.T} samples")
+        rc = self._fn(self._rt, ctypes.c_void_p(xt.data_ptr()), ctypes.c_void_p(dt.data_ptr()), self._yp, self._pp)
+        if rc:
+            _lib.check(rc)
+        return self._y.reshape(xt.shape), self._pre.reshape(xt.shape)
+
+    def close(self):
+        """Stop the resident kernel and hand the carried state and delay history back to the model (`model.hidden`,
+        `model.diffdel.buffer`)."""
+        if self._rt is None:
+            return self.model.hidden, self.model.diffdel.buffer
+        h = torch.empty((self.B, ENGINE_H), dtype=torch.float32)
+        hist = torch.empty((self.B, self.D), dtype=torch.float32)
+        rt, self._rt = self._rt, None
+        _lib.check(_lib.load().ntm_rt_diffdel_close(rt, _ptr(h), _ptr(hist)))
+        self.model.hidden = self.model._from_engine(h.reshape(1, self.B, ENGINE_H)).to(self.device)
+        self.model.diffdel.buffer = hist.reshape(self.B, 1, self.D).to(self.device)
+        return self.model.hidden, self.model.diffdel.buffer
+
+    def __del__(self):
+        try:
+            if getattr(self, "_rt", None) is not None:
+                _lib.load().ntm_rt_diffdel_close(self._rt, None, None)
+                self._rt = None
+        except Exception:
+            pass
