@@ -579,20 +579,21 @@ struct RtStream {
     unsigned magic;
     Handle* hd;
     int B, T;
-    ntm::RtMailbox* mb;       // page-locked, mapped (RNN stream)
-    ntm::RtDelayMailbox* mbd; // page-locked, mapped (DiffDelRNN stream)
+    bool delay;               // DiffDelRNN stream (ntm_rt_diffdel_*)
+    bool check;               // DiffDelRNN: refuse blocks with d > D or NaN (NTM_EDELAY)
+    int64_t D;
+    ntm::RtMailbox* mb;       // page-locked, mapped
     float* h_dev;             // B x 64 state, read at open, written when the server leaves
     float* hist_dev;          // DiffDelRNN: B x D delay history, read at open, written when the server leaves
-    int64_t D;
-    bool check;               // DiffDelRNN: refuse blocks with d > D or NaN (NTM_EDELAY)
     cudaStream_t st;
     unsigned seq;
     bool dead;                // the server left (stop, idle timeout or error)
 };
-RtStream* as_rt(void* p)
+// The stream behind p if it is one of the given kind (an RNN stream for ntm_rt_*, a DiffDelRNN stream for ntm_rt_diffdel_*).
+RtStream* as_rt(void* p, bool delay)
 {
     RtStream* r = static_cast<RtStream*>(p);
-    return (r && r->magic == RT_MAGIC) ? r : nullptr;
+    return (r && r->magic == RT_MAGIC && r->delay == delay) ? r : nullptr;
 }
 double now_s()
 {
@@ -606,7 +607,6 @@ void rt_free(RtStream* r)
     if (r->h_dev) cudaFree(r->h_dev);
     if (r->hist_dev) cudaFree(r->hist_dev);
     if (r->mb) cudaFreeHost(r->mb);
-    if (r->mbd) cudaFreeHost(r->mbd);
     Handle* hd = r->hd;
     r->magic = 0;
     delete r;
@@ -614,14 +614,15 @@ void rt_free(RtStream* r)
 }
 
 // Publish block `++r->seq` (its data is already in the mailbox) and wait until the server has answered it.
-int rt_handshake(RtStream* r, volatile unsigned* seq_in, volatile unsigned* seq_out)
+int rt_handshake(RtStream* r)
 {
     __atomic_thread_fence(__ATOMIC_SEQ_CST);            // the block is in memory before its sequence number
+    ntm::RtMailbox* mb = r->mb;
     const unsigned seq = ++r->seq;
-    *seq_in = seq;
+    mb->seq_in = seq;
     const double t0 = now_s();
     unsigned spins = 0;
-    while (*seq_out != seq) {
+    while (mb->seq_out != seq) {
         if ((++spins & 0xfff) == 0 && now_s() - t0 > 0.05) {
             // slow path: has the server left (idle timeout, error)?
             const cudaError_t q = cudaStreamQuery(r->st);
@@ -636,77 +637,9 @@ int rt_handshake(RtStream* r, volatile unsigned* seq_in, volatile unsigned* seq_
     return NTM_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-int ntm_rt_open(void* handle, int mode, const float* h_host, int64_t B, int64_t block_len, int skip, int idle_timeout_ms,
-                void** rt)
-{
-    if (!rt) return NTM_EINVAL;
-    *rt = nullptr;
-    Handle* hd = as_handle(handle);
-    if (!hd || B < 1 || B > ntm::RT_MAXSTREAMS || block_len < 1 || block_len > ntm::RT_MAXBLK || idle_timeout_ms < 1)
-        return NTM_EINVAL;
-    if (!mode_supported(mode) || mode == NTM_MODE_FP32) return NTM_EUNSUPPORTED;     // the server is the mma.sync kernel
-    DeviceGuard g(hd->device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice);
-    RtStream* r = new (std::nothrow) RtStream();
-    if (!r) return NTM_ENOMEM;
-    hd->refs.fetch_add(1, std::memory_order_relaxed);        // the resident kernel reads the handle's blob until close
-    r->magic = RT_MAGIC; r->hd = hd; r->B = (int)B; r->T = (int)block_len; r->mb = nullptr; r->mbd = nullptr;
-    r->h_dev = nullptr; r->hist_dev = nullptr; r->D = 0; r->check = false; r->st = nullptr; r->seq = 0; r->dead = false;
-    cudaError_t e = cudaHostAlloc(reinterpret_cast<void**>(&r->mb), sizeof(ntm::RtMailbox), cudaHostAllocMapped);
-    if (e == cudaSuccess) {
-        memset(r->mb, 0, sizeof(ntm::RtMailbox));
-        e = cudaMalloc(&r->h_dev, sizeof(float) * 64 * (size_t)B);
-    }
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&r->st, cudaStreamNonBlocking);
-    if (e == cudaSuccess)
-        e = h_host ? cudaMemcpyAsync(r->h_dev, h_host, sizeof(float) * 64 * (size_t)B, cudaMemcpyHostToDevice, r->st)
-                   : cudaMemsetAsync(r->h_dev, 0, sizeof(float) * 64 * (size_t)B, r->st);
-    ntm::RtMailbox* mb_dev = nullptr;
-    if (e == cudaSuccess) e = cudaHostGetDevicePointer(reinterpret_cast<void**>(&mb_dev), r->mb, 0);
-    if (e == cudaSuccess) {
-        ntm::GruArgs a{};
-        a.blob = hd->blob; a.sm_count = hd->sm_count; a.x = &mb_dev->x[0][0]; a.y = &mb_dev->y[0][0]; a.h_in = r->h_dev; a.h_out = r->h_dev;
-        a.B = B; a.T = block_len; a.ldx = ntm::RT_MAXBLK; a.ldy = ntm::RT_MAXBLK; a.skip = skip;
-        a.rt = mb_dev; a.rt_idle_ns = (unsigned long long)idle_timeout_ms * 1000000ull;
-        e = ntm::launch_gru_mma_rt(a, mode_fmt(mode), r->st);
-    }
-    if (e != cudaSuccess) { rt_free(r); return cuda_fail(e); }
-    *rt = r;
-    return NTM_OK;
-}
-
-int ntm_rt_process(void* rt, const float* x_host, float* y_host)
-{
-    RtStream* r = as_rt(rt);
-    if (!r || !r->mb || !x_host || !y_host) return NTM_EINVAL;
-    if (r->dead) return NTM_ECLOSED;
-    ntm::RtMailbox* mb = r->mb;
-    for (int s = 0; s < r->B; ++s) memcpy(&mb->x[s][0], x_host + (size_t)s * r->T, sizeof(float) * (size_t)r->T);
-    const int rc = rt_handshake(r, &mb->seq_in, &mb->seq_out);
-    if (rc != NTM_OK) return rc;
-    for (int s = 0; s < r->B; ++s) memcpy(y_host + (size_t)s * r->T, &mb->y[s][0], sizeof(float) * (size_t)r->T);
-    return NTM_OK;
-}
-
-int ntm_rt_close(void* rt, float* h_host_out)
-{
-    RtStream* r = as_rt(rt);
-    if (!r || !r->mb) return NTM_EINVAL;
-    DeviceGuard g(r->hd->device);
-    r->mb->seq_in = ntm::RT_STOP;
-    cudaError_t e = cudaStreamSynchronize(r->st);        // the server writes the final state on its way out
-    if (e == cudaSuccess && h_host_out)
-        e = cudaMemcpy(h_host_out, r->h_dev, sizeof(float) * 64 * (size_t)r->B, cudaMemcpyDeviceToHost);
-    rt_free(r);
-    return e == cudaSuccess ? NTM_OK : cuda_fail(e);
-}
-
-int ntm_rt_diffdel_open(void* handle, int mode, const float* h_host, const float* hist_host, int64_t B, int64_t block_len,
-                        int64_t D, int skip, int check_delay, int idle_timeout_ms, void** rt)
+// Both kinds of stream: validation, allocation, state and history upload, launch.  An RNN stream has delay == false, D == 0.
+int rt_open(void* handle, int mode, const float* h_host, const float* hist_host, int64_t B, int64_t block_len, int64_t D,
+            int skip, bool delay, bool check, int idle_timeout_ms, void** rt)
 {
     if (!rt) return NTM_EINVAL;
     *rt = nullptr;
@@ -715,19 +648,17 @@ int ntm_rt_diffdel_open(void* handle, int mode, const float* h_host, const float
         idle_timeout_ms < 1)
         return NTM_EINVAL;
     if (!mode_supported(mode) || mode == NTM_MODE_FP32) return NTM_EUNSUPPORTED;     // the server is the mma.sync kernel
-    if (D > 0x7fffffff || ntm::rt_delay_ring_len(B, D) == 0) return NTM_EUNSUPPORTED;   // the pre_d ring must fit on chip
+    if (delay && (D > 0x7fffffff || ntm::rt_delay_ring_len(B, D) == 0)) return NTM_EUNSUPPORTED;   // the ring must fit on chip
     DeviceGuard g(hd->device);
     if (!g.ok) return cuda_fail(cudaErrorInvalidDevice);
-    RtStream* r = new (std::nothrow) RtStream();
+    RtStream* r = new (std::nothrow) RtStream();       // value-initialised: null pointers, seq 0, not dead
     if (!r) return NTM_ENOMEM;
     hd->refs.fetch_add(1, std::memory_order_relaxed);        // the resident kernel reads the handle's blob until close
-    r->magic = RT_MAGIC; r->hd = hd; r->B = (int)B; r->T = (int)block_len; r->mb = nullptr; r->mbd = nullptr;
-    r->h_dev = nullptr; r->hist_dev = nullptr; r->D = D; r->check = check_delay != 0; r->st = nullptr; r->seq = 0;
-    r->dead = false;
+    r->magic = RT_MAGIC; r->hd = hd; r->B = (int)B; r->T = (int)block_len; r->delay = delay; r->check = check; r->D = D;
     const size_t hbytes = sizeof(float) * 64 * (size_t)B, histbytes = sizeof(float) * (size_t)B * (size_t)D;
-    cudaError_t e = cudaHostAlloc(reinterpret_cast<void**>(&r->mbd), sizeof(ntm::RtDelayMailbox), cudaHostAllocMapped);
+    cudaError_t e = cudaHostAlloc(reinterpret_cast<void**>(&r->mb), sizeof(ntm::RtMailbox), cudaHostAllocMapped);
     if (e == cudaSuccess) {
-        memset(r->mbd, 0, sizeof(ntm::RtDelayMailbox));
+        memset(r->mb, 0, sizeof(ntm::RtMailbox));
         e = cudaMalloc(&r->h_dev, hbytes);
     }
     if (e == cudaSuccess && D > 0) e = cudaMalloc(&r->hist_dev, histbytes);
@@ -738,62 +669,105 @@ int ntm_rt_diffdel_open(void* handle, int mode, const float* h_host, const float
     if (e == cudaSuccess && D > 0)
         e = hist_host ? cudaMemcpyAsync(r->hist_dev, hist_host, histbytes, cudaMemcpyHostToDevice, r->st)
                       : cudaMemsetAsync(r->hist_dev, 0, histbytes, r->st);
-    ntm::RtDelayMailbox* mb_dev = nullptr;
-    if (e == cudaSuccess) e = cudaHostGetDevicePointer(reinterpret_cast<void**>(&mb_dev), r->mbd, 0);
+    ntm::RtMailbox* mb_dev = nullptr;
+    if (e == cudaSuccess) e = cudaHostGetDevicePointer(reinterpret_cast<void**>(&mb_dev), r->mb, 0);
     if (e == cudaSuccess) {
-        // the server rolls the history in place: it reads hist_in into its ring at start and writes hist_out when it leaves
         ntm::GruArgs a{};
-        a.B = B; a.T = block_len; a.D = (int)D;
         a.blob = hd->blob; a.sm_count = hd->sm_count; a.h_in = r->h_dev; a.h_out = r->h_dev;
-        a.x = &mb_dev->x[0][0]; a.d = &mb_dev->d[0][0]; a.y = &mb_dev->y[0][0]; a.pre = &mb_dev->pre[0][0];
+        a.B = B; a.T = block_len; a.skip = skip;
+        a.x = &mb_dev->x[0][0]; a.y = &mb_dev->y[0][0];
         a.ldx = a.ldd = a.ldy = a.ldp = ntm::RT_MAXBLK;
-        a.hist_in = r->hist_dev; a.hist_out = r->hist_dev; a.skip = skip;
-        a.rtd = mb_dev; a.rt_idle_ns = (unsigned long long)idle_timeout_ms * 1000000ull;
-        e = ntm::launch_gru_mma_rt_delay(a, mode_fmt(mode), r->st);
+        if (delay) {
+            // the server rolls the history in place: it reads hist_in into its ring at start and writes hist_out when it leaves
+            a.d = &mb_dev->d[0][0]; a.pre = &mb_dev->pre[0][0]; a.D = (int)D;
+            a.hist_in = r->hist_dev; a.hist_out = r->hist_dev;
+        }
+        a.rt = mb_dev; a.rt_idle_ns = (unsigned long long)idle_timeout_ms * 1000000ull;
+        e = ntm::launch_gru_mma_rt(a, mode_fmt(mode), r->st);
     }
     if (e != cudaSuccess) { rt_free(r); return cuda_fail(e); }
     *rt = r;
     return NTM_OK;
 }
 
-int ntm_rt_diffdel_process(void* rt, const float* x_host, const float* d_host, float* y_host, float* pre_d_host)
+// One block: rows into the mailbox, handshake, rows out.  d_host: DiffDelRNN only; pre_d_host: nullptr = not returned.
+int rt_process(RtStream* r, const float* x_host, const float* d_host, float* y_host, float* pre_d_host)
 {
-    RtStream* r = as_rt(rt);
-    if (!r || !r->mbd || !x_host || !d_host || !y_host) return NTM_EINVAL;
     if (r->dead) return NTM_ECLOSED;
-    const size_t n = (size_t)r->B * (size_t)r->T;
+    const size_t T = (size_t)r->T;
     if (r->check) {                 // before the block is handed over: a refused block changes neither state nor history
         const float lim = (float)r->D;
-        for (size_t i = 0; i < n; ++i)
+        for (size_t i = 0; i < (size_t)r->B * T; ++i)
             if (!(d_host[i] <= lim)) return NTM_EDELAY;
     }
-    ntm::RtDelayMailbox* mb = r->mbd;
+    ntm::RtMailbox* mb = r->mb;
     for (int s = 0; s < r->B; ++s) {
-        memcpy(&mb->x[s][0], x_host + (size_t)s * r->T, sizeof(float) * (size_t)r->T);
-        memcpy(&mb->d[s][0], d_host + (size_t)s * r->T, sizeof(float) * (size_t)r->T);
+        memcpy(&mb->x[s][0], x_host + s * T, sizeof(float) * T);
+        if (d_host) memcpy(&mb->d[s][0], d_host + s * T, sizeof(float) * T);
     }
-    const int rc = rt_handshake(r, &mb->seq_in, &mb->seq_out);
+    const int rc = rt_handshake(r);
     if (rc != NTM_OK) return rc;
     for (int s = 0; s < r->B; ++s) {
-        memcpy(y_host + (size_t)s * r->T, &mb->y[s][0], sizeof(float) * (size_t)r->T);
-        if (pre_d_host) memcpy(pre_d_host + (size_t)s * r->T, &mb->pre[s][0], sizeof(float) * (size_t)r->T);
+        memcpy(y_host + s * T, &mb->y[s][0], sizeof(float) * T);
+        if (pre_d_host) memcpy(pre_d_host + s * T, &mb->pre[s][0], sizeof(float) * T);
     }
     return NTM_OK;
 }
 
-int ntm_rt_diffdel_close(void* rt, float* h_host_out, float* hist_host_out)
+// Stop the server, read back the final state and history it writes on its way out (nullptr: skip), free the stream.
+int rt_close(RtStream* r, float* h_host_out, float* hist_host_out)
 {
-    RtStream* r = as_rt(rt);
-    if (!r || !r->mbd) return NTM_EINVAL;
     DeviceGuard g(r->hd->device);
-    r->mbd->seq_in = ntm::RT_STOP;
-    cudaError_t e = cudaStreamSynchronize(r->st);        // the server writes the final state and history on its way out
+    r->mb->seq_in = ntm::RT_STOP;
+    cudaError_t e = cudaStreamSynchronize(r->st);
     if (e == cudaSuccess && h_host_out)
         e = cudaMemcpy(h_host_out, r->h_dev, sizeof(float) * 64 * (size_t)r->B, cudaMemcpyDeviceToHost);
     if (e == cudaSuccess && hist_host_out && r->D > 0)
         e = cudaMemcpy(hist_host_out, r->hist_dev, sizeof(float) * (size_t)r->B * (size_t)r->D, cudaMemcpyDeviceToHost);
     rt_free(r);
     return e == cudaSuccess ? NTM_OK : cuda_fail(e);
+}
+
+}  // namespace
+
+extern "C" {
+
+int ntm_rt_open(void* handle, int mode, const float* h_host, int64_t B, int64_t block_len, int skip, int idle_timeout_ms,
+                void** rt)
+{
+    return rt_open(handle, mode, h_host, nullptr, B, block_len, 0, skip, false, false, idle_timeout_ms, rt);
+}
+
+int ntm_rt_process(void* rt, const float* x_host, float* y_host)
+{
+    RtStream* r = as_rt(rt, false);
+    if (!r || !x_host || !y_host) return NTM_EINVAL;
+    return rt_process(r, x_host, nullptr, y_host, nullptr);
+}
+
+int ntm_rt_close(void* rt, float* h_host_out)
+{
+    RtStream* r = as_rt(rt, false);
+    return r ? rt_close(r, h_host_out, nullptr) : NTM_EINVAL;
+}
+
+int ntm_rt_diffdel_open(void* handle, int mode, const float* h_host, const float* hist_host, int64_t B, int64_t block_len,
+                        int64_t D, int skip, int check_delay, int idle_timeout_ms, void** rt)
+{
+    return rt_open(handle, mode, h_host, hist_host, B, block_len, D, skip, true, check_delay != 0, idle_timeout_ms, rt);
+}
+
+int ntm_rt_diffdel_process(void* rt, const float* x_host, const float* d_host, float* y_host, float* pre_d_host)
+{
+    RtStream* r = as_rt(rt, true);
+    if (!r || !x_host || !d_host || !y_host) return NTM_EINVAL;
+    return rt_process(r, x_host, d_host, y_host, pre_d_host);
+}
+
+int ntm_rt_diffdel_close(void* rt, float* h_host_out, float* hist_host_out)
+{
+    RtStream* r = as_rt(rt, true);
+    return r ? rt_close(r, h_host_out, hist_host_out) : NTM_EINVAL;
 }
 
 int ntm_esr_sums(const float* out, int64_t ldo, const float* target, int64_t ldt, int64_t B, int64_t T, int dc_pre,

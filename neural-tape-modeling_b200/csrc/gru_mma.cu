@@ -54,8 +54,8 @@ struct MmaCfg {
 // costs two PCIe round trips instead of a kernel launch, a prologue and a stream synchronisation.
 // DEFER (HALF only): the output head's accumulators are consumed one iteration later (see the head block); wins when a
 // warp has its SM sub-partition to itself (one CTA per SM: cfg 3, cfg 5, the real-time server), loses otherwise.
-// RTD (RT only): the DiffDelRNN server (a.rtd, RtDelayMailbox) -- each block also brings its delay trajectory and returns
-// pre_d next to y.  The pre_d ring persists across blocks on the time axis of a 64-bit sample counter since open (the
+// RTD (RT only): the DiffDelRNN server -- each block also brings its delay trajectory (a.d) and returns pre_d (a.pre) next
+// to y, through the same mailbox.  The pre_d ring persists across blocks on the time axis of a 64-bit sample counter since open (the
 // carried history at -D .. -1), so every block's y is the one long fused call's, bit for bit; the rolled history is read
 // back from the ring when the server leaves.
 template <int FMT, bool HALF, bool RT = false, bool DEFER = RT, bool SPLIT = false, bool RTD = false>
@@ -309,7 +309,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
             unsigned long long t_wait;
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_wait));
             unsigned sq;
-            while ((sq = RTD ? a.rtd->seq_in : a.rt->seq_in) == rt_seen) {
+            while ((sq = a.rt->seq_in) == rt_seen) {
                 unsigned long long now;
                 asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
                 if (now - t_wait > a.rt_idle_ns) { sq = RT_STOP; break; }
@@ -319,36 +319,22 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         __syncthreads();
         if (rt_flag == RT_STOP) break;
         rt_seen = rt_flag;
-        // fetch the block: every thread keeps up to 8 uncached loads of mapped host memory in flight (one round trip)
-        if (RTD) {                             // (x and d: 16 loads in the same round trip)
-            const int total = ns * (int)a.T;
-            float v[8], w[8];
+        // fetch the block: every thread keeps up to 8 uncached loads of mapped host memory in flight (one round trip;
+        // DiffDelRNN: x and d, 16 loads in the same round trip)
+        const int total = ns * (int)a.T;
+        float v[8], w[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int idx = tid + 128 * i;
-                v[i] = idx < total ? __ldcv(a.x + (idx / (int)a.T) * a.ldx + idx % (int)a.T) : 0.0f;
-                w[i] = idx < total ? __ldcv(a.d + (idx / (int)a.T) * a.ldd + idx % (int)a.T) : 0.0f;
-            }
+        for (int i = 0; i < 8; ++i) {
+            const int idx = tid + 128 * i;
+            v[i] = idx < total ? __ldcv(a.x + (idx / (int)a.T) * a.ldx + idx % (int)a.T) : 0.0f;
+            if (RTD) w[i] = idx < total ? __ldcv(a.d + (idx / (int)a.T) * a.ldd + idx % (int)a.T) : 0.0f;
+        }
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int idx = tid + 128 * i;
-                if (idx < total) {
-                    rt_xblk[(idx / (int)a.T) * RT_MAXBLK + idx % (int)a.T] = v[i];
-                    rt_dblk[(idx / (int)a.T) * RT_MAXBLK + idx % (int)a.T] = w[i];
-                }
-            }
-        } else {
-            const int total = ns * (int)a.T;
-            float v[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int idx = tid + 128 * i;
-                v[i] = idx < total ? __ldcv(a.x + (idx / (int)a.T) * a.ldx + idx % (int)a.T) : 0.0f;
-            }
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int idx = tid + 128 * i;
-                if (idx < total) rt_xblk[(idx / (int)a.T) * RT_MAXBLK + idx % (int)a.T] = v[i];
+        for (int i = 0; i < 8; ++i) {
+            const int idx = tid + 128 * i;
+            if (idx < total) {
+                rt_xblk[(idx / (int)a.T) * RT_MAXBLK + idx % (int)a.T] = v[i];
+                if (RTD) rt_dblk[(idx / (int)a.T) * RT_MAXBLK + idx % (int)a.T] = w[i];
             }
         }
         __syncthreads();
@@ -576,12 +562,8 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         }
         __threadfence_system();                // this block's y (and pre_d) is visible to the host ...
         __syncthreads();
-        if (RTD) {                             // ... before its sequence number is
-            if (tid == 0) a.rtd->seq_out = rt_seen;
-            rt_pos += a.T;
-        } else {
-            if (tid == 0) a.rt->seq_out = rt_seen;
-        }
+        if (tid == 0) a.rt->seq_out = rt_seen; // ... before its sequence number is
+        if (RTD) rt_pos += a.T;
     }
     } while (RT);
 
@@ -624,7 +606,7 @@ cudaError_t launch_mma_one(const GruArgs& a, cudaStream_t st)
     return cudaGetLastError();
 }
 
-template <int FMT, bool SPLIT = false, bool RTD = false>
+template <int FMT, bool SPLIT, bool RTD>
 cudaError_t launch_mma_rt_fmt(const GruArgs& a, cudaStream_t st)
 {
     using C = MmaCfg<FMT, SPLIT>;
@@ -639,6 +621,17 @@ cudaError_t launch_mma_rt_fmt(const GruArgs& a, cudaStream_t st)
     gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT, RTD><<<1, 128, C::SMEM_BYTES + ring_bytes, st>>>(b);
     ++g_launches;
     return cudaGetLastError();
+}
+
+template <bool RTD>
+cudaError_t launch_mma_rt(const GruArgs& a, int fmt, cudaStream_t st)
+{
+    switch (fmt) {
+        case FMT_F16X3: return launch_mma_rt_fmt<FMT_F16, true, RTD>(a, st);
+        case FMT_TF32: return launch_mma_rt_fmt<FMT_TF32, false, RTD>(a, st);
+        case FMT_BF16: return launch_mma_rt_fmt<FMT_BF16, false, RTD>(a, st);
+        default: return launch_mma_rt_fmt<FMT_F16, false, RTD>(a, st);
+    }
 }
 
 template <int FMT>
@@ -666,36 +659,21 @@ cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_he
     }
 }
 
-// The resident real-time server (one CTA, <= 4 streams, blocks of a.T <= RT_MAXBLK samples; see RtMailbox).
+// The resident real-time server (one CTA, <= 4 streams, blocks of a.T <= RT_MAXBLK samples; see RtMailbox).  a.x and a.y
+// point into a.rt; a.d != nullptr selects the DiffDelRNN server, whose a.d and a.pre point into a.rt too (hist_in /
+// hist_out: B x D, may alias).
 cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st)
 {
-    if (a.B <= 0 || a.B > RT_MAXSTREAMS || a.T <= 0 || a.T > RT_MAXBLK || !a.rt || a.d) return cudaErrorInvalidValue;
-    switch (fmt) {
-        case FMT_F16X3: return launch_mma_rt_fmt<FMT_F16, true>(a, st);
-        case FMT_TF32: return launch_mma_rt_fmt<FMT_TF32>(a, st);
-        case FMT_BF16: return launch_mma_rt_fmt<FMT_BF16>(a, st);
-        default: return launch_mma_rt_fmt<FMT_F16>(a, st);
-    }
+    if (a.B <= 0 || a.B > RT_MAXSTREAMS || a.T <= 0 || a.T > RT_MAXBLK || !a.rt) return cudaErrorInvalidValue;
+    if (!a.d) return launch_mma_rt<false>(a, fmt, st);
+    if (!a.pre || a.warmup || a.D < 0 || (a.D > 0 && (!a.hist_in || !a.hist_out))) return cudaErrorInvalidValue;
+    return launch_mma_rt<true>(a, fmt, st);
 }
 
 int rt_delay_ring_len(long long B, long long D)
 {
     const long long rl = delay_ring_len(D, MmaCfg<FMT_F16>::CH);
     return B * rl * 4 <= RT_RING_BUDGET ? (int)rl : 0;
-}
-
-// The DiffDelRNN server (a.rtd; a.x, a.d, a.y, a.pre point into it; hist_in / hist_out: B x D, may alias).
-cudaError_t launch_gru_mma_rt_delay(const GruArgs& a, int fmt, cudaStream_t st)
-{
-    if (a.B <= 0 || a.B > RT_MAXSTREAMS || a.T <= 0 || a.T > RT_MAXBLK || !a.rtd || !a.d || !a.pre || a.warmup || a.D < 0 ||
-        (a.D > 0 && (!a.hist_in || !a.hist_out)))
-        return cudaErrorInvalidValue;
-    switch (fmt) {
-        case FMT_F16X3: return launch_mma_rt_fmt<FMT_F16, true, true>(a, st);
-        case FMT_TF32: return launch_mma_rt_fmt<FMT_TF32, false, true>(a, st);
-        case FMT_BF16: return launch_mma_rt_fmt<FMT_BF16, false, true>(a, st);
-        default: return launch_mma_rt_fmt<FMT_F16, false, true>(a, st);
-    }
 }
 
 }  // namespace ntm

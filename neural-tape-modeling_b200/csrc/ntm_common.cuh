@@ -36,24 +36,14 @@ struct BlobLayout {
 };
 static_assert(BlobLayout::FP32_END % 4 == 0, "tensor-core images must stay 16-byte aligned");
 
-// Mailbox of a real-time stream (ntm_rt_*): page-locked, mapped host memory shared by the host thread and the resident
-// server kernel (gru_mma.cu, RT form).  The host writes a block into x, then bumps seq_in; the kernel writes y, then sets
-// seq_out = seq_in.  seq_in == RT_STOP ends the kernel.
+// Mailbox of a real-time stream (ntm_rt_*, ntm_rt_diffdel_*): page-locked, mapped host memory shared by the host thread and
+// the resident server kernel (gru_mma.cu, RT form).  The host writes a block into x (DiffDelRNN: and its delay trajectory
+// into d), then bumps seq_in; the kernel writes y (DiffDelRNN: and the head output before the delay into pre), then sets
+// seq_out = seq_in.  seq_in == RT_STOP ends the kernel.  An RNN stream leaves d and pre unused.
 constexpr int RT_MAXBLK = 256;          // samples per block, at most
 constexpr int RT_MAXSTREAMS = 4;
 constexpr unsigned RT_STOP = 0xffffffffu;
 struct RtMailbox {
-    volatile unsigned seq_in;
-    unsigned pad0[31];
-    float x[RT_MAXSTREAMS][RT_MAXBLK];
-    volatile unsigned seq_out;
-    unsigned pad1[31];
-    float y[RT_MAXSTREAMS][RT_MAXBLK];
-};
-
-// Mailbox of a real-time DiffDelRNN stream (ntm_rt_diffdel_*; gru_mma.cu, RT + delay form): the same handshake, with the
-// block's delay trajectory d next to x and the head output before the delay (pre) next to y.
-struct RtDelayMailbox {
     volatile unsigned seq_in;
     unsigned pad0[31];
     float x[RT_MAXSTREAMS][RT_MAXBLK];
@@ -82,10 +72,7 @@ struct GruArgs {
     int ring_len;                   // DiffDelRNN, mma.sync kernels: samples of pre_d kept per stream in shared memory (power
                                     // of two >= D + chunk + 1, size_delay_ring; 0: read the delay taps back through L2)
     int sm_count;                   // SMs of the handle's device (host-side dispatch only)
-    union {                         // real-time server forms only:
-        RtMailbox* rt;              //   RNN (x, y point into it)
-        RtDelayMailbox* rtd;        //   DiffDelRNN (x, d, y, pre point into it)
-    };
+    RtMailbox* rt;                  // real-time server forms only (x, y and, DiffDelRNN, d, pre point into it)
     unsigned long long rt_idle_ns;  // the server leaves after this long without a block
 };
 
@@ -112,10 +99,10 @@ void fill_tcs_consts(const float* blob_host, TcsConsts* kc);
 cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_head, cudaStream_t st);
 cudaError_t launch_gru_mma4(const GruArgs& a, int fmt, cudaStream_t st);   // GRU and DiffDelGRU, f16 / bf16 / strict f16x3, four
                                                                              // streams per CTA, 4x unrolled
-cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st);    // resident real-time server, <= 4 streams
-// The same server for DiffDelRNN (a.rtd).  rt_delay_ring_len: its pre_d ring per stream for B streams and history length D, or
-// 0 if the ring does not fit RT_RING_BUDGET (the launcher then refuses the launch).
-cudaError_t launch_gru_mma_rt_delay(const GruArgs& a, int fmt, cudaStream_t st);
+// Resident real-time server, <= 4 streams; a.d != nullptr selects its DiffDelRNN form.  rt_delay_ring_len: the DiffDelRNN
+// server's pre_d ring per stream for B streams and history length D, or 0 if the ring does not fit RT_RING_BUDGET (the
+// launcher then refuses the launch).
+cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st);
 int rt_delay_ring_len(long long B, long long D);
 void pack_tc_images(float* blob_host);   // host: fills BlobLayout::IMG_* from the fp32 part of the blob
 cudaError_t launch_delay(const float* x, long long ldx, const float* d, long long ldd, float* y, long long ldy,

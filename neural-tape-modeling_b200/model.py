@@ -294,31 +294,48 @@ class BlockStream:
         if dev.type != "cuda":
             raise RuntimeError("ntm_b200 has no CPU path; move the model to a CUDA device")
         self.model, self.B, self.T, self.device = model, int(n_streams), int(block_len), dev
-        self._handle = ctypes.c_void_p(model._handle(dev))
-        self._generation = model._engine.generation
+        self._dev = dev.index
+        self._resolve_handle()
         self._mode = _lib.MODES[model.mode]
         self._skip = int(bool(model.skip))
         h = model._hidden_in(self.B, dev)
         self.h = torch.zeros((1, self.B, ENGINE_H), dtype=torch.float32, device=dev) if h is None else h.clone()
         self.y = torch.empty((self.B, 1, self.T), dtype=torch.float32, device=dev)
+        self._ld_out = max(self.T, 1)                       # row stride of the internal output buffers
         self._fn = _lib.load().ntm_gru_forward
         self._hp = ctypes.c_void_p(self.h.data_ptr())
         self._yp = ctypes.c_void_p(self.y.data_ptr())
         self._st = _stream(dev)
 
+    def _resolve_handle(self):
+        """The model's packed-parameter handle; called again once the parameters were re-packed (load_state_dict, .to(),
+        ...), which frees the old one."""
+        self._handle = ctypes.c_void_p(self.model._handle(self.device))
+        self._generation = self.model._engine.generation
+
+    def _ld(self, t, name, min_len=0):
+        """Row stride of `t`, a float32 block of shape (n_streams, 1, min_len .. block_len) on the model's device with unit
+        stride in time."""
+        if t.dtype != torch.float32 or t.get_device() != self._dev or t.dim() != 3 or t.shape[0] != self.B \
+                or t.shape[1] != 1 or not min_len <= t.shape[2] <= self.T or t.stride(2) != 1:
+            raise RuntimeError(f"{name}: expected a float32 CUDA block of shape ({self.B}, 1, {min_len} .. {self.T}) on "
+                               f"{self.device}")
+        return t.stride(0) if self.B > 1 else max(t.shape[2], 1)
+
     def process(self, x, out=None):
         """x (n_streams, 1, block_len) float32 on the model's device -> y (the internal buffer, overwritten by the
-        next call, or `out`).  Asynchronous on the stream that was current when the BlockStream was created."""
-        if x.dtype != torch.float32 or not x.is_cuda or x.dim() != 3 or x.shape[0] != self.B or x.shape[2] > self.T \
-                or x.stride(2) != 1:
-            raise RuntimeError(f"expected a float32 CUDA block of shape ({self.B}, 1, <= {self.T})")
+        next call, or `out`, at least as long as x).  Asynchronous on the stream that was current when the BlockStream
+        was created."""
+        ldx = self._ld(x, "x")
         T = x.shape[2]
-        if self._generation != self.model._engine.generation:     # parameters were re-packed (load_state_dict, .to(), ...):
-            self._handle = ctypes.c_void_p(self.model._handle(self.device))      # the old handle is gone
-            self._generation = self.model._engine.generation
-        y, yp = (self.y, self._yp) if out is None else (out, ctypes.c_void_p(out.data_ptr()))
-        rc = self._fn(self._handle, self._mode, ctypes.c_void_p(x.data_ptr()), x.stride(0) if self.B > 1 else max(T, 1),
-                      yp, y.stride(0) if self.B > 1 else max(T, 1), self._hp, self._hp, self.B, T, self._skip, self._st)
+        if out is None:
+            y, yp, ldy = self.y, self._yp, self._ld_out
+        else:
+            y, yp, ldy = out, ctypes.c_void_p(out.data_ptr()), self._ld(out, "out", T)
+        if self._generation != self.model._engine.generation:
+            self._resolve_handle()
+        rc = self._fn(self._handle, self._mode, ctypes.c_void_p(x.data_ptr()), ldx, yp, ldy, self._hp, self._hp, self.B, T,
+                      self._skip, self._st)
         if rc:
             _lib.check(rc)
         return y if T == y.shape[2] else y[:, :, :T]
@@ -349,49 +366,63 @@ class RealtimeStream:
         h_host = None if h is None else h.reshape(self.B, ENGINE_H).to("cpu", torch.float32).contiguous()
         torch.cuda.current_stream(dev).synchronize()         # the state above is final before the server reads its copy
         self._rt = ctypes.c_void_p()
-        rc = _lib.load().ntm_rt_open(model._handle(dev), _lib.MODES[model.mode], _ptr(h_host), self.B, self.T,
-                                     int(bool(model.skip)), int(idle_timeout_ms), ctypes.byref(self._rt))
-        _lib.check(rc)
+        _lib.check(self._open(h_host, int(idle_timeout_ms)))
         self._y = torch.empty((self.B, self.T), dtype=torch.float32)
         self._fn = _lib.load().ntm_rt_process
         self._yp = ctypes.c_void_p(self._y.data_ptr())
         self.x_in = torch.zeros((self.B, self.T), dtype=torch.float32)       # optional fixed input block for step()
         self._xp = ctypes.c_void_p(self.x_in.data_ptr())
 
+    def _open(self, h_host, idle_timeout_ms):
+        m = self.model
+        return _lib.load().ntm_rt_open(m._handle(self.device), _lib.MODES[m.mode], _ptr(h_host), self.B, self.T,
+                                       int(bool(m.skip)), idle_timeout_ms, ctypes.byref(self._rt))
+
+    def _live(self):
+        """The open server's stream pointer."""
+        if self._rt is None:
+            raise RuntimeError("ntm_b200: real-time stream is closed")
+        return self._rt
+
+    def _host_block(self, b, name):
+        t = torch.as_tensor(b)
+        if t.is_cuda or t.dtype != torch.float32 or t.numel() != self.B * self.T or not t.is_contiguous():
+            raise RuntimeError(f"{name}: expected contiguous float32 HOST blocks of {self.B} x {self.T} samples")
+        return t
+
     def step(self):
         """Lowest-overhead form: process the block the caller wrote into `self.x_in`; returns the internal output
         block (overwritten by the next call)."""
-        rc = self._fn(self._rt, self._xp, self._yp)
+        rc = self._fn(self._live(), self._xp, self._yp)
         if rc:
             _lib.check(rc)
         return self._y
 
     def process(self, x):
-        if self._rt is None:
-            raise RuntimeError("ntm_b200: real-time stream is closed")
-        xt = torch.as_tensor(x)
-        if xt.is_cuda or xt.dtype != torch.float32 or xt.numel() != self.B * self.T or not xt.is_contiguous():
-            raise RuntimeError(f"expected a contiguous float32 HOST block of {self.B} x {self.T} samples")
-        rc = self._fn(self._rt, ctypes.c_void_p(xt.data_ptr()), self._yp)
+        rt = self._live()
+        xt = self._host_block(x, "x")
+        rc = self._fn(rt, ctypes.c_void_p(xt.data_ptr()), self._yp)
         if rc:
             _lib.check(rc)
         return self._y.reshape(xt.shape)
 
-    def close(self):
-        """Stop the resident kernel and hand the carried state back to the model (`model.hidden`)."""
-        if self._rt is None:
-            return self.model.hidden
-        h = torch.empty((self.B, ENGINE_H), dtype=torch.float32)
+    def _stop(self, h=None):
+        """Stop the resident kernel; the final state goes into the host tensor `h` (None: dropped)."""
         rt, self._rt = self._rt, None
         _lib.check(_lib.load().ntm_rt_close(rt, _ptr(h)))
-        self.model.hidden = self.model._from_engine(h.reshape(1, self.B, ENGINE_H)).to(self.device)
+
+    def close(self):
+        """Stop the resident kernel and hand the carried state back to the model (`model.hidden`)."""
+        if self._rt is not None:
+            h = torch.empty((self.B, ENGINE_H), dtype=torch.float32)
+            self._stop(h)
+            self.model.hidden = self.model._from_engine(h.reshape(1, self.B, ENGINE_H)).to(self.device)
         return self.model.hidden
 
     def __del__(self):
         try:
             if getattr(self, "_rt", None) is not None:
-                _lib.load().ntm_rt_close(self._rt, None)
-                self._rt = None
+                self._stop()
         except Exception:
             pass
 
@@ -540,7 +571,7 @@ class DiffDelRNN(RNN):
         return RealtimeDelayStream(self, n_streams, block_len, idle_timeout_ms)
 
 
-class DelayBlockStream:
+class DelayBlockStream(BlockStream):
     """Block-by-block DiffDelRNN processing of `n_streams` streams with the state and the delay history carried on the
     device.
 
@@ -553,55 +584,43 @@ class DelayBlockStream:
     synchronises the stream once per block; a refused block raises AssertionError and changes nothing."""
 
     def __init__(self, model, n_streams, block_len):
-        dev = model._device()
-        if dev.type != "cuda":
-            raise RuntimeError("ntm_b200 has no CPU path; move the model to a CUDA device")
-        self.model, self.B, self.T, self.device = model, int(n_streams), int(block_len), dev
-        self._handle = ctypes.c_void_p(model._handle(dev))
-        self._generation = model._engine.generation
-        self._mode = _lib.MODES[model.mode]
-        self._skip = int(bool(model.skip))
+        super().__init__(model, n_streams, block_len)
         self.D = int(model.diffdel.max_delay)
-        h = model._hidden_in(self.B, dev)
-        self.h = torch.zeros((1, self.B, ENGINE_H), dtype=torch.float32, device=dev) if h is None else h.clone()
-        hist = model.diffdel._history(self.B, dev)
+        hist = model.diffdel._history(self.B, self.device)
         self.hist = (hist.clone(), torch.empty_like(hist))
         self._cur = 0                                       # self.hist[_cur] holds the carried history
-        self.y = torch.empty((self.B, 1, self.T), dtype=torch.float32, device=dev)
-        self.pre_d = torch.empty((self.B, 1, self.T), dtype=torch.float32, device=dev)
+        self.pre_d = torch.empty_like(self.y)
         L = _lib.load()
         self._fn, self._check = L.ntm_diffdel_forward, L.ntm_delay_check
-        self._hp = ctypes.c_void_p(self.h.data_ptr())
+        self._pp = ctypes.c_void_p(self.pre_d.data_ptr())
         self._histp = tuple(ctypes.c_void_p(t.data_ptr()) for t in self.hist)
-        self._st = _stream(dev)
 
     def process(self, x, d, out=None, out_pre_d=None):
         """x, d (n_streams, 1, block_len) float32 on the model's device -> (y, pre_d): the internal buffers, overwritten
-        by the next call, or `out` / `out_pre_d`.  Asynchronous on the stream that was current when the stream was
-        created, except for the delay check."""
-        for t, name in ((x, "x"), (d, "d")):
-            if t.dtype != torch.float32 or not t.is_cuda or t.dim() != 3 or t.shape[0] != self.B or t.shape[1] != 1 \
-                    or t.shape[2] > self.T or t.stride(2) != 1:
-                raise RuntimeError(f"{name}: expected a float32 CUDA block of shape ({self.B}, 1, <= {self.T})")
+        by the next call, or `out` / `out_pre_d`, at least as long as x.  Asynchronous on the stream that was current when
+        the stream was created, except for the delay check."""
+        ldx, ldd = self._ld(x, "x"), self._ld(d, "d")
         if d.shape != x.shape:
             raise RuntimeError(f"x {tuple(x.shape)} and d {tuple(d.shape)} must have the same shape")
         T = x.shape[2]
-
-        def ld(t):
-            return t.stride(0) if self.B > 1 else max(T, 1)
-        if self._generation != self.model._engine.generation:     # parameters were re-packed: the old handle is gone
-            self._handle = ctypes.c_void_p(self.model._handle(self.device))
-            self._generation = self.model._engine.generation
+        if out is None:
+            y, yp, ldy = self.y, self._yp, self._ld_out
+        else:
+            y, yp, ldy = out, ctypes.c_void_p(out.data_ptr()), self._ld(out, "out", T)
+        if out_pre_d is None:
+            pre, pp, ldp = self.pre_d, self._pp, self._ld_out
+        else:
+            pre, pp, ldp = out_pre_d, ctypes.c_void_p(out_pre_d.data_ptr()), self._ld(out_pre_d, "out_pre_d", T)
+        if self._generation != self.model._engine.generation:
+            self._resolve_handle()
         dp = ctypes.c_void_p(d.data_ptr())
         if self.model.diffdel.check_delay and T > 0:
-            rc = self._check(dp, ld(d), self.B, T, self.D, self.device.index, self._st)
+            rc = self._check(dp, ldd, self.B, T, self.D, self._dev, self._st)
             if rc:
                 _lib.check(rc)
-        y = self.y if out is None else out
-        pre = self.pre_d if out_pre_d is None else out_pre_d
-        rc = self._fn(self._handle, self._mode, ctypes.c_void_p(x.data_ptr()), ld(x), dp, ld(d),
-                      ctypes.c_void_p(y.data_ptr()), ld(y), ctypes.c_void_p(pre.data_ptr()), ld(pre), self._hp, self._hp,
-                      self._histp[self._cur], self._histp[self._cur ^ 1], self.B, T, self.D, 0, self._skip, self._st)
+        rc = self._fn(self._handle, self._mode, ctypes.c_void_p(x.data_ptr()), ldx, dp, ldd, yp, ldy, pp, ldp, self._hp,
+                      self._hp, self._histp[self._cur], self._histp[self._cur ^ 1], self.B, T, self.D, 0, self._skip,
+                      self._st)
         if rc:
             _lib.check(rc)
         self._cur ^= 1
@@ -611,12 +630,11 @@ class DelayBlockStream:
 
     def close(self):
         """Hand the carried state and delay history back to the model (`model.hidden`, `model.diffdel.buffer`)."""
-        self.model.hidden = self.model._from_engine(self.h)
         self.model.diffdel.buffer = self.hist[self._cur]
-        return self.model.hidden, self.model.diffdel.buffer
+        return super().close(), self.model.diffdel.buffer
 
 
-class RealtimeDelayStream:
+class RealtimeDelayStream(RealtimeStream):
     """Block-by-block DiffDelRNN processing of up to 4 streams through a RESIDENT server kernel (ntm_rt_diffdel_*,
     csrc/gru_mma.cu RT + delay form).
 
@@ -632,68 +650,47 @@ class RealtimeDelayStream:
     at `close()` or after `idle_timeout_ms` without a block."""
 
     def __init__(self, model, n_streams=1, block_len=64, idle_timeout_ms=5000):
-        dev = model._device()
-        if dev.type != "cuda":
-            raise RuntimeError("ntm_b200 has no CPU path; move the model to a CUDA device")
-        self.model, self.B, self.T, self.device = model, int(n_streams), int(block_len), dev
-        self.D = int(model.diffdel.max_delay)
-        h = model._hidden_in(self.B, dev)
-        h_host = None if h is None else h.reshape(self.B, ENGINE_H).to("cpu", torch.float32).contiguous()
-        hist_host = model.diffdel._history(self.B, dev).reshape(self.B, self.D).to("cpu").contiguous()
-        torch.cuda.current_stream(dev).synchronize()         # state and history are final before the server reads them
-        self._rt = ctypes.c_void_p()
-        rc = _lib.load().ntm_rt_diffdel_open(model._handle(dev), _lib.MODES[model.mode], _ptr(h_host), _ptr(hist_host),
-                                             self.B, self.T, self.D, int(bool(model.skip)),
-                                             int(bool(model.diffdel.check_delay)), int(idle_timeout_ms),
-                                             ctypes.byref(self._rt))
-        _lib.check(rc)
-        self._y = torch.empty((self.B, self.T), dtype=torch.float32)
+        super().__init__(model, n_streams, block_len, idle_timeout_ms)
         self._pre = torch.empty((self.B, self.T), dtype=torch.float32)
         self._fn = _lib.load().ntm_rt_diffdel_process
-        self._yp = ctypes.c_void_p(self._y.data_ptr())
         self._pp = ctypes.c_void_p(self._pre.data_ptr())
-        self.x_in = torch.zeros((self.B, self.T), dtype=torch.float32)       # optional fixed input blocks for step()
-        self.d_in = torch.zeros((self.B, self.T), dtype=torch.float32)
-        self._xp = ctypes.c_void_p(self.x_in.data_ptr())
+        self.d_in = torch.zeros((self.B, self.T), dtype=torch.float32)       # optional fixed delay block for step()
         self._dp = ctypes.c_void_p(self.d_in.data_ptr())
+
+    def _open(self, h_host, idle_timeout_ms):
+        m = self.model
+        self.D = int(m.diffdel.max_delay)
+        hist_host = m.diffdel._history(self.B, self.device).reshape(self.B, self.D).to("cpu").contiguous()
+        return _lib.load().ntm_rt_diffdel_open(m._handle(self.device), _lib.MODES[m.mode], _ptr(h_host), _ptr(hist_host),
+                                               self.B, self.T, self.D, int(bool(m.skip)), int(bool(m.diffdel.check_delay)),
+                                               idle_timeout_ms, ctypes.byref(self._rt))
 
     def step(self):
         """Lowest-overhead form: process the blocks the caller wrote into `self.x_in` / `self.d_in`; returns the internal
         (y, pre_d) blocks (overwritten by the next call)."""
-        rc = self._fn(self._rt, self._xp, self._dp, self._yp, self._pp)
+        rc = self._fn(self._live(), self._xp, self._dp, self._yp, self._pp)
         if rc:
             _lib.check(rc)
         return self._y, self._pre
 
     def process(self, x, d):
-        if self._rt is None:
-            raise RuntimeError("ntm_b200: real-time stream is closed")
-        xt, dt = torch.as_tensor(x), torch.as_tensor(d)
-        for t in (xt, dt):
-            if t.is_cuda or t.dtype != torch.float32 or t.numel() != self.B * self.T or not t.is_contiguous():
-                raise RuntimeError(f"expected contiguous float32 HOST blocks of {self.B} x {self.T} samples")
-        rc = self._fn(self._rt, ctypes.c_void_p(xt.data_ptr()), ctypes.c_void_p(dt.data_ptr()), self._yp, self._pp)
+        rt = self._live()
+        xt, dt = self._host_block(x, "x"), self._host_block(d, "d")
+        rc = self._fn(rt, ctypes.c_void_p(xt.data_ptr()), ctypes.c_void_p(dt.data_ptr()), self._yp, self._pp)
         if rc:
             _lib.check(rc)
         return self._y.reshape(xt.shape), self._pre.reshape(xt.shape)
 
+    def _stop(self, h=None):
+        """Stop the resident kernel; with `h` given, the final state goes into it and the rolled history back to the
+        model (`model.diffdel.buffer`)."""
+        hist = None if h is None else torch.empty((self.B, self.D), dtype=torch.float32)
+        rt, self._rt = self._rt, None
+        _lib.check(_lib.load().ntm_rt_diffdel_close(rt, _ptr(h), _ptr(hist)))
+        if hist is not None:
+            self.model.diffdel.buffer = hist.reshape(self.B, 1, self.D).to(self.device)
+
     def close(self):
         """Stop the resident kernel and hand the carried state and delay history back to the model (`model.hidden`,
         `model.diffdel.buffer`)."""
-        if self._rt is None:
-            return self.model.hidden, self.model.diffdel.buffer
-        h = torch.empty((self.B, ENGINE_H), dtype=torch.float32)
-        hist = torch.empty((self.B, self.D), dtype=torch.float32)
-        rt, self._rt = self._rt, None
-        _lib.check(_lib.load().ntm_rt_diffdel_close(rt, _ptr(h), _ptr(hist)))
-        self.model.hidden = self.model._from_engine(h.reshape(1, self.B, ENGINE_H)).to(self.device)
-        self.model.diffdel.buffer = hist.reshape(self.B, 1, self.D).to(self.device)
-        return self.model.hidden, self.model.diffdel.buffer
-
-    def __del__(self):
-        try:
-            if getattr(self, "_rt", None) is not None:
-                _lib.load().ntm_rt_diffdel_close(self._rt, None, None)
-                self._rt = None
-        except Exception:
-            pass
+        return super().close(), self.model.diffdel.buffer

@@ -2,7 +2,9 @@
 (ntm_rt_diffdel_*, RealtimeDelayStream) and the device-side DelayBlockStream.  Bar: bit-identical to one long
 DiffDelRNN.forward over the concatenated signal from the same state and delay history -- y, pre_d, the final state and
 the rolled history -- plus the delay assert, argument limits and the idle timeout.  Every stream is closed in a
-`finally`, so no resident kernel outlives its test."""
+`finally`, so no resident kernel outlives its test.  The last two tests cover both kinds of stream: the RNN's and the
+DiffDelRNN's share their C-side core and their Python classes."""
+import ctypes
 import time
 
 import numpy as np
@@ -10,7 +12,7 @@ import pytest
 import torch
 
 from conftest import load_ckpt
-from ntm_b200 import DiffDelRNN, lib, signals
+from ntm_b200 import RNN, DiffDelRNN, lib, signals
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -204,6 +206,8 @@ def test_realtime_delay_stream_limits_and_idle_timeout():
             st.close()
         with pytest.raises(RuntimeError, match="closed"):
             st.process(torch.zeros(1, 64), torch.zeros(1, 64))
+        with pytest.raises(RuntimeError, match="closed"):
+            st.step()
         st = m.realtime_stream(1, 64, idle_timeout_ms=200)
         try:
             st.process(torch.zeros(1, 64), torch.zeros(1, 64))
@@ -213,3 +217,89 @@ def test_realtime_delay_stream_limits_and_idle_timeout():
         finally:
             st.close()
         torch.cuda.synchronize()
+
+
+def test_cross_kind_calls_are_refused():
+    """ntm_rt_process / ntm_rt_close on a DiffDelRNN stream and ntm_rt_diffdel_process / _close on an RNN stream return
+    NTM_EINVAL and leave both streams open: they then process and close exactly as if the calls had not been made."""
+    B, T, nblk = 2, 64, 4
+    L = lib.load()
+
+    def ptr(t):
+        return ctypes.c_void_p(t.data_ptr())
+    with torch.inference_mode():
+        m, h, hist = warmed(B, signals.DELAY_MAX)
+        x, d = signals_for(B, T * nblk, signals.DELAY_MAX + 1)
+        ref = one_call(m, h, hist, x, d)
+        g = RNN(input_size=1, hidden_size=64, output_size=1).to(DEV)
+        g.load_state_dict(load_ckpt("cfg1"))
+        g.mode = "f16"
+        g.hidden = h.clone()
+        gref = (g(x.to(DEV).reshape(B, 1, -1)).cpu().reshape(B, -1), g.hidden.cpu())
+        g.hidden, m.hidden, m.diffdel.buffer = h.clone(), h.clone(), hist.clone()
+        torch.cuda.synchronize()
+        rt, rtd = g.realtime_stream(B, T), m.realtime_stream(B, T)
+        try:
+            blk, out = torch.zeros(B, T), torch.empty(B, T)
+            assert L.ntm_rt_process(rtd._rt, ptr(blk), ptr(out)) == -1
+            assert L.ntm_rt_close(rtd._rt, None) == -1
+            assert L.ntm_rt_diffdel_process(rt._rt, ptr(blk), ptr(blk), ptr(out), None) == -1
+            assert L.ntm_rt_diffdel_close(rt._rt, None, None) == -1
+            ys, yds, pds = [], [], []
+            for k in range(nblk):
+                xb, db = x[:, k * T:(k + 1) * T].contiguous(), d[:, k * T:(k + 1) * T].contiguous()
+                ys.append(rt.process(xb).clone())
+                y, p = rtd.process(xb, db)
+                yds.append(y.clone())
+                pds.append(p.clone())
+        finally:
+            h_g = rt.close().cpu()
+            h_m, hist_m = rtd.close()
+    assert torch.equal(torch.cat(ys, 1), gref[0]) and torch.equal(h_g, gref[1])
+    assert_same((torch.cat(yds, 1), torch.cat(pds, 1), h_m.cpu(), hist_m.cpu()), ref)
+
+
+@pytest.mark.parametrize("kind", ["rnn", "diffdel"])
+def test_block_stream_refuses_bad_blocks_and_outputs(kind):
+    """A caller's output that is too short, has the wrong shape, lives on the host or has another dtype, and an input
+    block with two channels, raise before anything is written: the outputs keep their contents, and the stream continues
+    exactly like one that never saw the bad calls."""
+    B, T = 2, 64
+    with torch.inference_mode():
+        if kind == "rnn":
+            m = RNN(input_size=1, hidden_size=64, output_size=1).to(DEV)
+            m.load_state_dict(load_ckpt("cfg1"))
+            m.mode = "f16"
+            m.initialize_hidden()
+        else:
+            m, _, _ = warmed(B, signals.DELAY_MAX)
+            m.initialize_hidden(B, signals.DELAY_MAX)
+        x = torch.from_numpy(signals.stream_batch(B, 2 * T)).to(DEV).reshape(B, 1, -1)
+        d = torch.full_like(x, 3.5)
+
+        def blocks(k):
+            sl = slice(k * T, (k + 1) * T)
+            return (x[:, :, sl],) if kind == "rnn" else (x[:, :, sl], d[:, :, sl])
+        good, bad = m.block_stream(B, T), m.block_stream(B, T)
+        outs = [torch.full((B, 1, T // 2), 7.0, device=DEV),                  # shorter than the block
+                torch.full((B, 2, T), 7.0, device=DEV),                       # two channels
+                torch.full((B + 1, 1, T), 7.0, device=DEV),                   # one stream too many
+                torch.full((B, 1, T), 7.0),                                   # host
+                torch.full((B, 1, T), 7.0, device=DEV, dtype=torch.float64)]
+        for o in outs:
+            before = o.clone()
+            with pytest.raises(RuntimeError, match="^out: "):
+                bad.process(*blocks(0), o)
+            if kind == "diffdel":
+                with pytest.raises(RuntimeError, match="^out_pre_d: "):
+                    bad.process(*blocks(0), None, o)
+            torch.cuda.synchronize()
+            assert torch.equal(o, before)
+        with pytest.raises(RuntimeError, match="^x: "):
+            bad.process(torch.zeros((B, 2, T), device=DEV), *blocks(0)[1:])
+        for k in range(2):
+            want, got = good.process(*blocks(k)), bad.process(*blocks(k))
+            if kind == "rnn":
+                want, got = (want,), (got,)
+            for w, g in zip(want, got):
+                assert torch.equal(w, g)

@@ -59,6 +59,8 @@ def test_realtime_stream_numpy_blocks_and_shapes():
         rt.close()
         with pytest.raises(RuntimeError, match="closed"):
             rt.process(np.zeros((2, 16), np.float32))
+        with pytest.raises(RuntimeError, match="closed"):
+            rt.step()
 
 
 def test_realtime_stream_limits_and_idle_timeout():
