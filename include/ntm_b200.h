@@ -96,7 +96,10 @@ int ntm_gru_forward(void* handle, int mode, const float* x, int64_t ldx, float* 
                     const float* h_in, float* h_out, int64_t B, int64_t T, int skip, void* stream);
 
 /*
- * pre_d = head(GRU(x, h));  y = delay(pre_d, d)  in ONE kernel (delay read fused after the GRU output).
+ * pre_d = head(GRU(x, h));  y = delay(pre_d, d).  Where the last D + 129 samples of pre_d per stream fit on chip
+ * (tensor-core modes at a few streams per SM, not in warm-up) the delay read is fused into the recurrent kernel: one
+ * launch.  Otherwise the GRU writes pre_d and the stand-alone delay line (ntm_delay_forward's kernels) follows on the
+ * same stream: three launches.
  * Replaces: DiffDelRNN.forward, code/model.py:393-424 (GRU + Linear(bias=False) + self.diffdel).
  *   d: delay in samples per output sample.  hist_in / hist_out: (B x D) carried delay history
  *   (TimeVaryingDelayLine.buffer, code/model.py:267,314-315); hist_out must not alias hist_in.

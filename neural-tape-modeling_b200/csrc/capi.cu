@@ -104,13 +104,16 @@ struct LaunchCfg {
     bool defer_head = false;                 // K_MMA, 4 streams per CTA: the deferred-head form
     int tcs_tiles = 0;                       // K_TCS: 128-stream tiles per CTA (1, 2)
     bool static_schedule = false;            // K_TCS: one CTA per tile group, no job queue
+    int ring_len = 0;                        // DiffDelRNN, K_MMA / K_MMA4: the fused form's pre_d ring (GruArgs::ring_len);
+                                             // 0: the GRU into pre_d, then the stand-alone delay line
 };
 
 constexpr long long TCS_MIN_STREAMS_PER_SM = 110;     // crossover mma.sync -> stream-major tcgen05 kernel (DESIGN.md 3.3)
 
-// Every kernel-selection rule of the engine: (mode, batch, SMs, tuning pair) -> configuration, or NTM_EINVAL for a tuning
-// pair that has no meaning in this mode (the table in include/ntm_b200.h).
-int resolve_launch(int mode, long long B, int sm_count, Tuning tune, LaunchCfg* out)
+// Every kernel-selection rule of the engine: (mode, batch, SMs, DiffDelRNN launch with history length D and warm-up flag,
+// tuning pair) -> configuration, or NTM_EINVAL for a tuning pair that has no meaning in this mode (the table in
+// include/ntm_b200.h).
+int resolve_launch(int mode, long long B, int sm_count, bool delay, long long D, int warmup, Tuning tune, LaunchCfg* out)
 {
     LaunchCfg c;
     const int s = tune.s, ks = tune.ks;
@@ -142,7 +145,7 @@ int resolve_launch(int mode, long long B, int sm_count, Tuning tune, LaunchCfg* 
     const bool lean_auto = strict ? B <= 4ll * sm_count : B <= 12ll * sm_count;
     if (automatic) {
         // latency regime (few streams per SM): warp-level mma.sync kernels; throughput regime (>= one 128-stream tile per
-        // SM): stream-major tcgen05 kernel (every operand format; DiffDelRNN batches run the delay read as a second pass)
+        // SM): stream-major tcgen05 kernel (every operand format)
         if (B >= (long long)sm_count * TCS_MIN_STREAMS_PER_SM) {
             c.kernel = K_TCS;
             // one tile per SM (time-multiplexed by the job queue) beats two resident tiles until ~190 streams per SM (measured)
@@ -171,19 +174,36 @@ int resolve_launch(int mode, long long B, int sm_count, Tuning tune, LaunchCfg* 
         // the deferred head wins while every 4-stream CTA has an SM of its own (B <= 4 streams per SM; rounded modes)
         c.defer_head = c.mma_streams == 4 && !strict && (B + 3) / 4 <= sm_count;
     }
+    // DiffDelRNN: the mma.sync kernels read the delay taps from an on-chip ring of pre_d at the chunk flush where the ring
+    // fits (ntm_common.cuh delay_ring_len).  Every other launch -- a longer history, a warm-up call, the fp32 and tcgen05
+    // kernels -- runs the delay line as a second, HBM-bound pass over pre_d (delay.cu: 12 bytes per sample, near the copy
+    // peak).  Reading the taps back through L2 inside the recurrent kernel instead stalls the whole persistent CTA at every
+    // chunk flush (256 x 30 s at D = 10001, f16: 239 vs 283 ms), and the tcgen05 kernel's job queue may still be producing,
+    // on another SM, the samples a tap reaches back to.
+    if (delay && !warmup && (c.kernel == K_MMA || c.kernel == K_MMA4))
+        c.ring_len = ntm::delay_ring_len(D, c.kernel == K_MMA ? c.mma_streams : 4, ntm::DELAY_RING_BUDGET);
     *out = c;
     return NTM_OK;
 }
 
-int run_gru(Handle* hd, int mode, const ntm::GruArgs& a, cudaStream_t st)
+// One recurrent launch (a.d != nullptr: DiffDelRNN).  A DiffDelRNN configuration without a ring runs in two passes on `st`:
+// the recurrent kernel as a plain GRU with its head output into pre_d, then the delay line and the history roll over it.
+int run_gru(Handle* hd, int mode, const ntm::GruArgs& a0, cudaStream_t st)
 {
     if (!mode_supported(mode)) return NTM_EUNSUPPORTED;
     unsigned long long tv = hd->tuning.load(std::memory_order_relaxed);
     if (tv == ~0ull) tv = g_tuning.load(std::memory_order_relaxed);
     LaunchCfg c;
-    const int rc = resolve_launch(mode, a.B, hd->sm_count, unpack_tuning(tv), &c);
+    const int rc = resolve_launch(mode, a0.B, hd->sm_count, a0.d != nullptr, a0.D, a0.warmup, unpack_tuning(tv), &c);
     if (rc != NTM_OK) return rc;
     const int fmt = mode_fmt(mode);
+    const bool two_pass = a0.d != nullptr && c.ring_len == 0;
+    ntm::GruArgs a = a0;
+    a.ring_len = c.ring_len;
+    if (two_pass) {
+        a.y = a0.pre; a.ldy = a0.ldp;
+        a.d = nullptr; a.pre = nullptr;
+    }
     switch (c.kernel) {
         case K_FP32: CU(ntm::launch_gru_fp32(a, c.fp32_streams, c.fp32_ksplit, st)); break;
         case K_MMA: CU(ntm::launch_gru_mma(a, fmt, c.mma_streams, c.defer_head, st)); break;
@@ -192,6 +212,9 @@ int run_gru(Handle* hd, int mode, const ntm::GruArgs& a, cudaStream_t st)
     }
     hd->last_kernel.store(c.kernel, std::memory_order_relaxed);
     g_last_kernel.store(c.kernel, std::memory_order_relaxed);
+    if (two_pass)         // warm-up: y = pre_d, history still rolled
+        CU(ntm::launch_delay(a0.pre, a0.ldp, a0.d, a0.ldd, a0.y, a0.ldy, a0.hist_in, a0.hist_out, a0.B, a0.T, a0.D,
+                             a0.warmup, st));
     return NTM_OK;
 }
 
@@ -648,7 +671,8 @@ int rt_open(void* handle, int mode, const float* h_host, const float* hist_host,
         idle_timeout_ms < 1)
         return NTM_EINVAL;
     if (!mode_supported(mode) || mode == NTM_MODE_FP32) return NTM_EUNSUPPORTED;     // the server is the mma.sync kernel
-    if (delay && (D > 0x7fffffff || ntm::rt_delay_ring_len(B, D) == 0)) return NTM_EUNSUPPORTED;   // the ring must fit on chip
+    const int ring_len = delay && D <= 0x7fffffff ? ntm::delay_ring_len(D, B, ntm::RT_RING_BUDGET) : 0;
+    if (delay && ring_len == 0) return NTM_EUNSUPPORTED;              // the ring must fit on chip
     DeviceGuard g(hd->device);
     if (!g.ok) return cuda_fail(cudaErrorInvalidDevice);
     RtStream* r = new (std::nothrow) RtStream();       // value-initialised: null pointers, seq 0, not dead
@@ -679,7 +703,7 @@ int rt_open(void* handle, int mode, const float* h_host, const float* hist_host,
         a.ldx = a.ldd = a.ldy = a.ldp = ntm::RT_MAXBLK;
         if (delay) {
             // the server rolls the history in place: it reads hist_in into its ring at start and writes hist_out when it leaves
-            a.d = &mb_dev->d[0][0]; a.pre = &mb_dev->pre[0][0]; a.D = (int)D;
+            a.d = &mb_dev->d[0][0]; a.pre = &mb_dev->pre[0][0]; a.D = (int)D; a.ring_len = ring_len;
             a.hist_in = r->hist_dev; a.hist_out = r->hist_dev;
         }
         a.rt = mb_dev; a.rt_idle_ns = (unsigned long long)idle_timeout_ms * 1000000ull;

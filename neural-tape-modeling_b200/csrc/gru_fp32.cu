@@ -1,8 +1,8 @@
 // Exact-fp32 persistent GRU kernel (CUDA cores) -- the parity anchor and the batch-1 real-time path.
 //
 // Replaces the per-timestep loop behind `self.GRU(x, self.hidden)` + `self.output(x)` of
-// RNN.forward / DiffDelRNN.forward (code/model.py:81-82, :412-413; gate equations torch rnn.py:1221-1224)
-// and, for DiffDelRNN, the delay read of code/model.py:422 fused at every chunk flush.
+// RNN.forward / DiffDelRNN.forward (code/model.py:81-82, :412-413; gate equations torch rnn.py:1221-1224).
+// For DiffDelRNN it writes pre_d and the stand-alone delay line (delay.cu) runs behind it (capi.cu run_gru).
 //
 // Layout: one CTA owns S streams for ALL T timesteps (no per-step launch, no HBM round trip of the state).
 //   - W_hh (192x64) lives in REGISTERS: thread (j, q) of 64*KS threads holds the three gate rows of hidden
@@ -13,8 +13,8 @@
 //     hidden unit end up owning different streams and no activation is computed twice.  The only things on
 //     the recurrence's critical path are: LDS -> FMA chain -> shuffles -> gates -> STS -> one barrier.
 //   - the 64-wide output head is NOT in the step loop: at the end of a chunk it is evaluated for all CH steps
-//     at once from the state ring (a [CH*S x 64] . [64] product), then flushed with coalesced stores; the
-//     fused delay read follows the flush.  x is staged per chunk with cp.async (double-buffered).
+//     at once from the state ring (a [CH*S x 64] . [64] product), then flushed with coalesced stores.  x is staged
+//     per chunk with cp.async (double-buffered).
 #include "ntm_common.cuh"
 
 namespace ntm {
@@ -117,10 +117,6 @@ __global__ void __launch_bounds__(64 * KS, 2) gru_fp32_kernel(const GruArgs a)
     const float bin = blob[BlobLayout::B_IH + 128 + j], bhn = blob[BlobLayout::B_HH + 128 + j];
     const float bo = blob[BlobLayout::B_OUT];
     if (tid < 64) wos[tid] = blob[BlobLayout::W_OUT + tid];
-
-    const bool delay = a.d != nullptr;
-    float* __restrict__ head_out = delay ? a.pre : a.y;
-    const long long ldo = delay ? a.ldp : a.ldy;
 
     // ---- initial state -> ring slot 0 ------------------------------------------------------------
     for (int idx = tid; idx < S * 64; idx += NT) {
@@ -226,39 +222,15 @@ __global__ void __launch_bounds__(64 * KS, 2) gru_fp32_kernel(const GruArgs a)
         }
         for (int idx = tid; idx < S * CH; idx += NT) {
             const int s = idx / CH, tt = idx % CH;
-            if (s < ns && tt < n) head_out[(b0 + s) * ldo + t0 + tt] = ys[s * CH + tt];
-        }
-        if (delay) {
-            __syncthreads();                   // this chunk's pre_d is visible CTA-wide (L2 reads below)
-            for (int idx = tid; idx < S * CH; idx += NT) {
-                const int s = idx / CH, tt = idx % CH;
-                if (s < ns && tt < n) {
-                    const long long t = t0 + tt;
-                    float v;
-                    if (a.warmup) {
-                        v = ys[s * CH + tt];
-                    } else {
-                        const float* prow = a.pre + (b0 + s) * a.ldp;
-                        const float* hrow = a.hist_in + (b0 + s) * (long long)a.D;
-                        v = delay_read(a.d[(b0 + s) * a.ldd + t], t, a.D, [&](long long i) {
-                            return i >= 0 ? __ldcg(prow + i) : hrow[a.D + i];
-                        });
-                    }
-                    a.y[(b0 + s) * a.ldy + t] = v;
-                }
-            }
+            if (s < ns && tt < n) a.y[(b0 + s) * a.ldy + t0 + tt] = ys[s * CH + tt];
         }
     }
 
-    // ---- final state; rolled delay history ------------------------------------------------------
+    // ---- final state ------------------------------------------------------------------------------
 #pragma unroll
     for (int i = 0; i < SO; ++i) {
         const int s = i * KS + q;
         if (s < ns) a.h_out[(b0 + s) * 64 + j] = hown[i];
-    }
-    if (delay) {
-        __syncthreads();
-        delay_roll_history<NT>(a, b0, ns, tid);
     }
 }
 
@@ -283,6 +255,7 @@ cudaError_t launch_one(const GruArgs& a, cudaStream_t st)
 cudaError_t launch_gru_fp32(const GruArgs& a, int streams, int ksplit, cudaStream_t st)
 {
     if (a.B <= 0 || a.T <= 0) return cudaSuccess;
+    if (a.d) return cudaErrorInvalidValue;          // plain GRU only
     if (ksplit == 2) {
         switch (streams) {
             case 1: return launch_one<2, 1>(a, st);

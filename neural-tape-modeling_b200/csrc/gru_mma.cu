@@ -36,7 +36,7 @@ constexpr float LOG2E_F = 1.4426950408889634f;
 template <int FMT, bool SPLIT = false>
 struct MmaCfg {
     static constexpr int S = 8;                      // columns of the state tile (streams per CTA of the 8-stream form)
-    static constexpr int CH = 128;                   // steps per staged chunk (measured at 1024 streams: 32 -> 232.7 ns/step, 64 -> 238, 128 -> 221.7, 256 -> 220.1)
+    static constexpr int CH = MMA_CH;                // steps per staged chunk (measured at 1024 streams: 32 -> 232.7 ns/step, 64 -> 238, 128 -> 221.7, 256 -> 220.1)
     static constexpr int YP_LD = S + 2;              // even: float2 stores of the head partials
     static constexpr int HB_BYTES = S * Frag<FMT, SPLIT>::ROW_BYTES;
     static constexpr int OFF_HB = 0;                               // [2][S][ROW_BYTES]
@@ -251,6 +251,9 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
     static_assert(2 * RT_MAXSTREAMS * RT_MAXBLK <= 2 * CH * S, "the server's d and pre_d blocks fit in ds");
     float* const rt_dblk = ds;
     float* const rt_pblk = ds + RT_MAXSTREAMS * RT_MAXBLK;
+    // DiffDelRNN (code/model.py:393-424): the head output is pre_d, y is the fractional-delay read of it (delay_read), fused
+    // at the chunk flush with its taps from the on-chip pre_d ring (ntm_common.cuh; capi.cu runs this form only where the
+    // ring fits); the delay trajectory is staged like x
     const bool delay = RTD || a.d != nullptr;
     float* __restrict__ head_out = delay ? a.pre : a.y;
     const long long ldo = delay ? a.ldp : a.ldy;
@@ -272,7 +275,6 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
     };
 
     const int rmask = a.ring_len - 1;
-    const bool use_ring = RTD || (delay && !a.warmup && a.ring_len > 0);
     auto load_d = [&](int buf, long long t0) {               // the chunk's delay trajectory, staged like x
         const int n = (int)((a.T - t0) < (long long)CH ? (a.T - t0) : (long long)CH);
         float* dstb = ds + buf * CH * S;
@@ -282,7 +284,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         }
         cp_async_commit();
     };
-    if (use_ring) delay_ring_prefill<128>(a, b0, ns, tid, ring);
+    if (delay) delay_ring_prefill<128>(a, b0, ns, tid, ring);
 
     // ---- initial state: fp32 in registers (hst[unit][stream]), rounded copy into state tile 0 ---------------------
     float hst[2][2];
@@ -340,7 +342,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         __syncthreads();
     }
     load_x(0, 0);
-    if (use_ring && !RTD) load_d(0, 0);
+    if (delay && !RTD) load_d(0, 0);
     for (long long c = 0; c < nchunks; ++c) {
         const long long t0 = c * CH;
         const int n = (int)((a.T - t0) < (long long)CH ? (a.T - t0) : (long long)CH);
@@ -350,7 +352,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
         __syncthreads();                       // xs[xb] landed; state tile `cur` complete; previous flush done
         if (c + 1 < nchunks) {
             load_x(xb ^ 1, t0 + CH);
-            if (use_ring && !RTD) load_d(xb ^ 1, t0 + CH);
+            if (delay && !RTD) load_d(xb ^ 1, t0 + CH);
         }
 
         float hpend[4];
@@ -515,8 +517,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
                 }
                 if (RT) rt_yblk[s * RT_MAXBLK + t0 + tt] = v;
                 else head_out[(b0 + s) * ldo + t0 + tt] = v;
-                if (delay && a.warmup) a.y[(b0 + s) * a.ldy + t0 + tt] = v;
-                if (use_ring) ring[s * a.ring_len + ((int)(t0 + tt) & rmask)] = v;
+                if (delay) ring[s * a.ring_len + ((int)(t0 + tt) & rmask)] = v;
             }
         }
         if (RTD) {
@@ -530,7 +531,7 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
                                                                   [&](long long i) { return rrow[(int)i & rmask]; });
                 }
             }
-        } else if (use_ring) {
+        } else if (delay) {
             // delay taps from the on-chip ring (the last ring_len >= D + CH samples of pre_d, history included) and the
             // staged trajectory: no L2 round trip of the samples this CTA has just produced
             __syncthreads();
@@ -544,9 +545,6 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
                         delay_read(dcur[tt * S + s], tg, a.D, [&](long long i) { return rrow[(int)i & rmask]; });
                 }
             }
-        } else if (delay && !a.warmup) {
-            __syncthreads();                   // this chunk's pre_d is visible CTA-wide (L2 reads below)
-            delay_chunk_l2<128, SC, CH>(a, b0, ns, tid, t0, n);
         }
     }
 
@@ -575,15 +573,9 @@ __global__ void __launch_bounds__(128, (FMT == FMT_TF32 || HALF || SPLIT) ? 2 : 
             const int s = (2 * tig + e) / CS;
             if (s < ns) a.h_out[(b0 + s) * 64 + u0 + u] = hst[u][e];
         }
-    if (RTD) {                                 // rolled history: ring positions rt_pos - D .. rt_pos - 1
+    if (delay) {                               // rolled history from the ring (the server's time axis: samples since open)
         __syncthreads();
-        for (long long idx = tid; idx < (long long)ns * a.D; idx += 128) {
-            const int s = (int)(idx / a.D), i = (int)(idx % a.D);
-            a.hist_out[(b0 + s) * (long long)a.D + i] = ring[s * a.ring_len + ((int)(rt_pos - a.D + i) & rmask)];
-        }
-    } else if (delay) {
-        __syncthreads();
-        delay_roll_history<128>(a, b0, ns, tid);
+        delay_ring_roll<128>(a, b0, ns, tid, ring, RTD ? rt_pos : a.T);
     }
 }
 
@@ -599,9 +591,8 @@ cudaError_t launch_mma_one(const GruArgs& a, cudaStream_t st)
     if (e != cudaSuccess) return e;
     constexpr int SC = HALF ? 4 : C::S;
     const long long grid = (a.B + SC - 1) / SC;
-    GruArgs b = a;
-    const int smem_bytes = C::SMEM_BYTES + size_delay_ring(b, SC, C::CH);
-    gru_mma_kernel<FMT, HALF, false, DEFER, SPLIT><<<(unsigned)grid, 128, smem_bytes, st>>>(b);
+    const int smem_bytes = C::SMEM_BYTES + (a.d ? a.ring_len * SC * 4 : 0);
+    gru_mma_kernel<FMT, HALF, false, DEFER, SPLIT><<<(unsigned)grid, 128, smem_bytes, st>>>(a);
     ++g_launches;
     return cudaGetLastError();
 }
@@ -610,15 +601,12 @@ template <int FMT, bool SPLIT, bool RTD>
 cudaError_t launch_mma_rt_fmt(const GruArgs& a, cudaStream_t st)
 {
     using C = MmaCfg<FMT, SPLIT>;
-    GruArgs b = a;
-    b.ring_len = RTD ? rt_delay_ring_len(a.B, a.D) : 0;
-    if (RTD && b.ring_len == 0) return cudaErrorInvalidValue;
-    const int ring_bytes = (int)(b.B * b.ring_len * 4);
+    const int ring_bytes = RTD ? (int)(a.B * a.ring_len * 4) : 0;
     cudaError_t e = cudaFuncSetAttribute(gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT, RTD>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          C::SMEM_BYTES + (RTD ? RT_RING_BUDGET : 0));
     if (e != cudaSuccess) return e;
-    gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT, RTD><<<1, 128, C::SMEM_BYTES + ring_bytes, st>>>(b);
+    gru_mma_kernel<FMT, true, true, !SPLIT, SPLIT, RTD><<<1, 128, C::SMEM_BYTES + ring_bytes, st>>>(a);
     ++g_launches;
     return cudaGetLastError();
 }
@@ -644,11 +632,13 @@ cudaError_t launch_mma_fmt(const GruArgs& a, int streams, bool defer_head, cudaS
 }  // namespace
 
 // fmt: FMT_F16 / FMT_BF16 / FMT_TF32 / FMT_F16X3 (strict: f16 hi/lo pairs, three MMAs per product).  streams: streams per CTA,
-// 4 (HALF) or 8.  defer_head: the deferred-head form of the 4-stream kernel (rounded modes only; see DEFER).
+// 4 (HALF) or 8.  defer_head: the deferred-head form of the 4-stream kernel (rounded modes only; see DEFER).  DiffDelRNN
+// (a.d != nullptr): a.ring_len from delay_ring_len at `streams` streams per CTA and DELAY_RING_BUDGET.
 cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_head, cudaStream_t st)
 {
     if (a.B <= 0 || a.T <= 0) return cudaSuccess;
     if (streams != 4 && streams != 8) return cudaErrorInvalidValue;
+    if (a.d && a.ring_len <= a.D + MMA_CH) return cudaErrorInvalidValue;
     switch (fmt) {
         case FMT_F16X3:
             return streams == 4 ? launch_mma_one<FMT_F16, true, false, true>(a, st)
@@ -661,19 +651,14 @@ cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_he
 
 // The resident real-time server (one CTA, <= 4 streams, blocks of a.T <= RT_MAXBLK samples; see RtMailbox).  a.x and a.y
 // point into a.rt; a.d != nullptr selects the DiffDelRNN server, whose a.d and a.pre point into a.rt too (hist_in /
-// hist_out: B x D, may alias).
+// hist_out: B x D, may alias; a.ring_len from delay_ring_len at B streams and RT_RING_BUDGET).
 cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st)
 {
     if (a.B <= 0 || a.B > RT_MAXSTREAMS || a.T <= 0 || a.T > RT_MAXBLK || !a.rt) return cudaErrorInvalidValue;
     if (!a.d) return launch_mma_rt<false>(a, fmt, st);
-    if (!a.pre || a.warmup || a.D < 0 || (a.D > 0 && (!a.hist_in || !a.hist_out))) return cudaErrorInvalidValue;
+    if (!a.pre || a.D < 0 || (a.D > 0 && (!a.hist_in || !a.hist_out)) || a.ring_len <= a.D + MMA_CH)
+        return cudaErrorInvalidValue;
     return launch_mma_rt<true>(a, fmt, st);
-}
-
-int rt_delay_ring_len(long long B, long long D)
-{
-    const long long rl = delay_ring_len(D, MmaCfg<FMT_F16>::CH);
-    return B * rl * 4 <= RT_RING_BUDGET ? (int)rl : 0;
 }
 
 }  // namespace ntm

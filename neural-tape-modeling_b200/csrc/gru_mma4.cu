@@ -35,7 +35,6 @@ using namespace mmaf;
 namespace {
 
 constexpr float LOG2E_F4 = 1.4426950408889634f;
-constexpr int MMA4_CH = 128;         // steps per staged chunk
 constexpr int MMA4_XPAD = 8;         // padding of a staged x row in floats
 constexpr int MMA4_YPAD = 4;         // padding of a head-partial row in floats, >= 4
 
@@ -43,7 +42,7 @@ template <int FMT>
 struct Mma4Cfg {
     using F = Frag<FMT, false>;
     static constexpr int SC = 4;                     // streams per CTA (columns 0, 2, 4, 6 of the n8 tile)
-    static constexpr int CH = MMA4_CH;               // steps per staged chunk
+    static constexpr int CH = MMA_CH;                // steps per staged chunk
     static constexpr int XLD = CH + MMA4_XPAD;       // staged x row of one stream
     static constexpr int YLD = CH + MMA4_YPAD;       // head partials of one (warp, stream): position p holds sample p - 1
     static constexpr int TILE_BYTES = 8 * F::ROW_BYTES;
@@ -149,13 +148,12 @@ __global__ void __launch_bounds__(128, 2) gru_mma4_kernel(const GruArgs a)
 
     // DiffDelRNN (code/model.py:393-424): the head output is pre_d, y is the fractional-delay read of it (delay_read,
     // ntm_common.cuh: bit-exact against the reference given the same pre_d), fused at the chunk flush.  The taps come from an
-    // on-chip ring of the last ring_len >= D + CH samples of pre_d per stream (carried history included) when it fits, from the
-    // chunk just written through L2 otherwise; the delay trajectory is staged like x.
+    // on-chip ring of the last ring_len >= D + CH samples of pre_d per stream (carried history included; capi.cu runs this
+    // form only where the ring fits); the delay trajectory is staged like x.
     const bool delay = a.d != nullptr;
     float* __restrict__ head_out = delay ? a.pre : a.y;
     const long long ldo = delay ? a.ldp : a.ldy;
     const int rmask = a.ring_len - 1;
-    const bool use_ring = delay && !a.warmup && a.ring_len > 0;
     auto load_d = [&](int buf, long long t0) {
         const int n = (int)((a.T - t0) < (long long)CH ? (a.T - t0) : (long long)CH);
         float* dstb = ds + buf * SC * CH;
@@ -165,7 +163,7 @@ __global__ void __launch_bounds__(128, 2) gru_mma4_kernel(const GruArgs a)
         }
         cp_async_commit();
     };
-    if (use_ring) delay_ring_prefill<128>(a, b0, ns, tid, ring);
+    if (delay) delay_ring_prefill<128>(a, b0, ns, tid, ring);
 
     // ---- initial state: fp32 in registers, rounded copy into state tile 0; the odd (dead) columns of both tiles stay zero ----
     float hst[2] = {0.0f, 0.0f};
@@ -260,7 +258,7 @@ __global__ void __launch_bounds__(128, 2) gru_mma4_kernel(const GruArgs a)
     const long long nchunks = (a.T + CH - 1) / CH;
     int cur = 0;                               // tile holding the current state at a chunk boundary (0 unless a chunk was odd)
     load_x(0, 0);
-    if (use_ring) load_d(0, 0);
+    if (delay) load_d(0, 0);
     for (long long c = 0; c < nchunks; ++c) {
         const long long t0 = c * CH;
         const int n = (int)((a.T - t0) < (long long)CH ? (a.T - t0) : (long long)CH);
@@ -270,7 +268,7 @@ __global__ void __launch_bounds__(128, 2) gru_mma4_kernel(const GruArgs a)
         __syncthreads();                       // xs[xb] landed; state tile `cur` complete; previous flush done
         if (c + 1 < nchunks) {
             load_x(xb ^ 1, t0 + CH);
-            if (use_ring) load_d(xb ^ 1, t0 + CH);
+            if (delay) load_d(xb ^ 1, t0 + CH);
         }
 
         const float* xrow = xcur + tig * XLD;
@@ -307,11 +305,10 @@ __global__ void __launch_bounds__(128, 2) gru_mma4_kernel(const GruArgs a)
                           yp[(3 * SC + s) * YLD + t + 1] + bo;
                 if (a.skip) v += xcur[s * XLD + t];
                 head_out[(b0 + s) * ldo + t0 + t] = v;
-                if (delay && a.warmup) a.y[(b0 + s) * a.ldy + t0 + t] = v;
-                if (use_ring) ring[s * a.ring_len + ((int)(t0 + t) & rmask)] = v;
+                if (delay) ring[s * a.ring_len + ((int)(t0 + t) & rmask)] = v;
             }
         }
-        if (use_ring) {
+        if (delay) {
             __syncthreads();
             const float* dcur = ds + xb * SC * CH;
             for (int idx = tid; idx < SC * CH; idx += 128) {
@@ -322,15 +319,12 @@ __global__ void __launch_bounds__(128, 2) gru_mma4_kernel(const GruArgs a)
                     a.y[(b0 + s) * a.ldy + tg] = delay_read(dcur[idx], tg, a.D, [&](long long i) { return rrow[(int)i & rmask]; });
                 }
             }
-        } else if (delay && !a.warmup) {
-            __syncthreads();                   // this chunk's pre_d is visible CTA-wide (L2 reads below)
-            delay_chunk_l2<128, SC, CH>(a, b0, ns, tid, t0, n);
         }
     }
     if (tig < ns) { a.h_out[(b0 + tig) * 64 + u0] = hst[0]; a.h_out[(b0 + tig) * 64 + u1] = hst[1]; }
-    if (delay) {
+    if (delay) {                               // rolled history from the ring
         __syncthreads();
-        delay_roll_history<128>(a, b0, ns, tid);
+        delay_ring_roll<128>(a, b0, ns, tid, ring, a.T);
     }
 }
 
@@ -344,20 +338,21 @@ cudaError_t launch_mma4_one(const GruArgs& a, cudaStream_t st)
                                     C::SMEM_BYTES + DELAY_RING_BUDGET);
     });
     if (e != cudaSuccess) return e;
-    GruArgs b = a;
-    const int smem_bytes = C::SMEM_BYTES + size_delay_ring(b, C::SC, C::CH);
-    gru_mma4_kernel<FMT, STRICT><<<(unsigned)((a.B + C::SC - 1) / C::SC), 128, smem_bytes, st>>>(b);
+    const int smem_bytes = C::SMEM_BYTES + (a.d ? a.ring_len * C::SC * 4 : 0);
+    gru_mma4_kernel<FMT, STRICT><<<(unsigned)((a.B + C::SC - 1) / C::SC), 128, smem_bytes, st>>>(a);
     ++g_launches;
     return cudaGetLastError();
 }
 
 }  // namespace
 
-// GRU and DiffDelGRU batches, f16 / bf16 operands or the strict f16x3 mode, four streams per CTA.
+// GRU and DiffDelGRU batches, f16 / bf16 operands or the strict f16x3 mode, four streams per CTA.  DiffDelRNN (a.d !=
+// nullptr): a.ring_len from delay_ring_len at four streams per CTA and DELAY_RING_BUDGET.
 cudaError_t launch_gru_mma4(const GruArgs& a, int fmt, cudaStream_t st)
 {
     if (a.B <= 0 || a.T <= 0) return cudaSuccess;
     if (fmt != FMT_F16 && fmt != FMT_BF16 && fmt != FMT_F16X3) return cudaErrorInvalidValue;
+    if (a.d && a.ring_len <= a.D + MMA_CH) return cudaErrorInvalidValue;
     if (fmt == FMT_F16X3) return launch_mma4_one<FMT_F16, true>(a, st);
     return fmt == FMT_BF16 ? launch_mma4_one<FMT_BF16>(a, st) : launch_mma4_one<FMT_F16>(a, st);
 }

@@ -647,32 +647,21 @@ void pack_tc_images(float* blob_host)
 }
 
 // fmt: FMT_F16 / FMT_BF16 / FMT_TF32 / FMT_F16X3.  tiles: 128-stream tiles per CTA (1 or 2).  static_schedule: one CTA per
-// tile group for all T steps even where the job queue would run.  DiffDelRNN batches (a.d != nullptr): the GRU + head pass
-// writes pre_d, the delay read runs as a second, HBM-bound pass over it (csrc/delay.cu: 12 bytes per sample at ~4.7 TB/s
-// against ~75 ps per sample of recurrent work: +3 %) -- the taps reach up to D samples back into other time chunks' output,
-// which the job-queue schedule of this kernel may still be producing on another SM.
-cudaError_t launch_gru_tcs(const GruArgs& a0, const TcsConsts& kc, int fmt, int sm_count, int tiles, bool static_schedule,
+// tile group for all T steps even where the job queue would run.  Plain GRU only: a DiffDelRNN batch runs this kernel into
+// pre_d and the stand-alone delay line behind it (capi.cu run_gru).
+cudaError_t launch_gru_tcs(const GruArgs& a, const TcsConsts& kc, int fmt, int sm_count, int tiles, bool static_schedule,
                            cudaStream_t st)
 {
-    if (a0.B <= 0 || a0.T <= 0) return cudaSuccess;
-    GruArgs a = a0;
-    const bool delay = a0.d != nullptr;
-    if (delay) {                               // pass 1: plain GRU + head into pre_d
-        a.y = a0.pre; a.ldy = a0.ldp;
-        a.d = nullptr; a.pre = nullptr;
-    }
+    if (a.B <= 0 || a.T <= 0) return cudaSuccess;
+    if (a.d) return cudaErrorInvalidValue;
     const bool two = tiles == 2;
     const bool ss = static_schedule;
-    cudaError_t e;
     switch (fmt) {
-        case FMT_BF16: e = two ? launch_tcs_one<FMT_BF16, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_BF16, 1>(a, kc, sm_count, ss, st); break;
-        case FMT_TF32: e = two ? launch_tcs_one<FMT_TF32, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_TF32, 1>(a, kc, sm_count, ss, st); break;
-        case FMT_F16X3: e = two ? launch_tcs_one<FMT_F16X3, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_F16X3, 1>(a, kc, sm_count, ss, st); break;
-        default: e = two ? launch_tcs_one<FMT_F16, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_F16, 1>(a, kc, sm_count, ss, st); break;
+        case FMT_BF16: return two ? launch_tcs_one<FMT_BF16, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_BF16, 1>(a, kc, sm_count, ss, st);
+        case FMT_TF32: return two ? launch_tcs_one<FMT_TF32, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_TF32, 1>(a, kc, sm_count, ss, st);
+        case FMT_F16X3: return two ? launch_tcs_one<FMT_F16X3, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_F16X3, 1>(a, kc, sm_count, ss, st);
+        default: return two ? launch_tcs_one<FMT_F16, 2>(a, kc, sm_count, ss, st) : launch_tcs_one<FMT_F16, 1>(a, kc, sm_count, ss, st);
     }
-    if (e != cudaSuccess || !delay) return e;
-    // pass 2: y = delay(pre_d, d) with the carried history (warm-up: y = pre_d, history still rolled)
-    return launch_delay(a0.pre, a0.ldp, a0.d, a0.ldd, a0.y, a0.ldy, a0.hist_in, a0.hist_out, a0.B, a0.T, a0.D, a0.warmup, st);
 }
 
 }  // namespace ntm

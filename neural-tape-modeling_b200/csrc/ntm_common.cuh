@@ -69,8 +69,8 @@ struct GruArgs {
     int D;
     int warmup;
     int skip;
-    int ring_len;                   // DiffDelRNN, mma.sync kernels: samples of pre_d kept per stream in shared memory (power
-                                    // of two >= D + chunk + 1, size_delay_ring; 0: read the delay taps back through L2)
+    int ring_len;                   // DiffDelRNN, mma.sync kernels: samples of pre_d kept per stream in shared memory
+                                    // (delay_ring_len; capi.cu chooses it)
     int sm_count;                   // SMs of the handle's device (host-side dispatch only)
     RtMailbox* rt;                  // real-time server forms only (x, y and, DiffDelRNN, d, pre point into it)
     unsigned long long rt_idle_ns;  // the server leaves after this long without a block
@@ -91,7 +91,8 @@ struct TcsConsts {
 };
 
 // per-TU launchers -------------------------------------------------------------------------------
-// The launchers run exactly the configuration they are given (capi.cu resolve_launch chooses it).
+// The launchers run exactly the configuration they are given (capi.cu resolve_launch chooses it).  Only the mma.sync
+// launchers have a DiffDelRNN form (a.d != nullptr, with a.ring_len set); the others run the plain GRU.
 cudaError_t launch_gru_fp32(const GruArgs& a, int streams, int ksplit, cudaStream_t st);
 cudaError_t launch_gru_tcs(const GruArgs& a, const TcsConsts& kc, int fmt, int sm_count, int tiles, bool static_schedule,
                            cudaStream_t st);
@@ -99,11 +100,8 @@ void fill_tcs_consts(const float* blob_host, TcsConsts* kc);
 cudaError_t launch_gru_mma(const GruArgs& a, int fmt, int streams, bool defer_head, cudaStream_t st);
 cudaError_t launch_gru_mma4(const GruArgs& a, int fmt, cudaStream_t st);   // GRU and DiffDelGRU, f16 / bf16 / strict f16x3, four
                                                                              // streams per CTA, 4x unrolled
-// Resident real-time server, <= 4 streams; a.d != nullptr selects its DiffDelRNN form.  rt_delay_ring_len: the DiffDelRNN
-// server's pre_d ring per stream for B streams and history length D, or 0 if the ring does not fit RT_RING_BUDGET (the
-// launcher then refuses the launch).
+// Resident real-time server, <= 4 streams; a.d != nullptr selects its DiffDelRNN form.
 cudaError_t launch_gru_mma_rt(const GruArgs& a, int fmt, cudaStream_t st);
-int rt_delay_ring_len(long long B, long long D);
 void pack_tc_images(float* blob_host);   // host: fills BlobLayout::IMG_* from the fp32 part of the blob
 cudaError_t launch_delay(const float* x, long long ldx, const float* d, long long ldd, float* y, long long ldy,
                          const float* hist_in, float* hist_out, long long B, long long T, long long D, int warmup,
@@ -168,38 +166,31 @@ __device__ __forceinline__ float delay_read(float dt, long long t, int D, LoadPa
     return acc;
 }
 
-// On-chip pre_d ring of a DiffDelRNN launch of the mma.sync kernels (gru_mma.cu, gru_mma4.cu) with `streams` streams per CTA
-// and chunks of `chunk` steps: the last ring_len samples of pre_d per stream, ring_len the smallest power of two (>= 64)
-// that is >= D + chunk + 1, stay in shared memory if they fit in DELAY_RING_BUDGET bytes per CTA (so that four CTAs still
-// share an SM); longer histories read their taps back through L2.  Sets b.ring_len (0: no ring) and returns the ring's bytes.
-// The real-time DiffDelRNN server is one CTA on an SM of its own and keeps its ring across blocks in up to RT_RING_BUDGET
-// bytes: with its 128-step chunks, ring_len 32768 (D <= 32639) for one stream, 16384 (D <= 16255) for two, 8192 (D <= 8063)
-// for three or four.  Its total shared memory stays under the 227 KB a CTA may opt into.
+// On-chip pre_d ring of the fused DiffDelRNN form of the mma.sync kernels (gru_mma.cu, gru_mma4.cu): the last ring_len samples
+// of pre_d per stream stay in shared memory, the carried history at positions -D .. -1, so that the delay taps of a chunk
+// never leave the chip.  ring_len is the smallest power of two (>= 64) that is >= D + MMA_CH + 1.  A batched launch gets
+// DELAY_RING_BUDGET bytes per CTA, so that four CTAs still share an SM: D <= 1919 at four streams per CTA, D <= 895 at eight.
+// Every other DiffDelRNN launch runs the plain GRU into pre_d and the stand-alone delay line (delay.cu) behind it (capi.cu
+// run_gru).  The real-time DiffDelRNN server is one CTA on an SM of its own and keeps its ring across blocks in up to
+// RT_RING_BUDGET bytes: ring_len 32768 (D <= 32639) for one stream, 16384 (D <= 16255) for two, 8192 (D <= 8063) for three
+// or four.  Its total shared memory stays under the 227 KB a CTA may opt into.
+constexpr int MMA_CH = 128;   // steps per staged chunk of the mma.sync kernels
 constexpr int DELAY_RING_BUDGET = 48 * 1024;
 constexpr int RT_RING_BUDGET = 128 * 1024;
-inline long long delay_ring_len(long long D, int chunk)
+// ring_len for history length D and `streams` streams per CTA, or 0 if the ring does not fit `budget` bytes
+inline int delay_ring_len(long long D, long long streams, long long budget)
 {
     long long rl = 64;
-    while (rl < D + chunk + 1) rl *= 2;
-    return rl;
-}
-inline int size_delay_ring(GruArgs& b, int streams, int chunk)
-{
-    b.ring_len = 0;
-    if (b.d == nullptr || b.warmup) return 0;
-    const long long rl = delay_ring_len(b.D, chunk);
-    if (rl * streams * 4 > DELAY_RING_BUDGET) return 0;
-    b.ring_len = (int)rl;
-    return (int)(rl * streams * 4);
+    while (rl < D + MMA_CH + 1) rl *= 2;
+    return rl * streams * 4 <= budget ? (int)rl : 0;
 }
 
-// DiffDelRNN delay tail of the fused recurrent kernels (gru_fp32.cu, gru_mma.cu, gru_mma4.cu), for a CTA of NT threads that owns
-// the ns streams from b0 on.  hist_in and hist_out hold each stream's last D samples of pre_d, oldest first.  ptxas
-// reschedules the kernels' step loops when the shape of this code changes, so compare their SASS after editing it.  The ring
-// delay pass of the mma.sync kernels and gru_fp32.cu's delay pass (warm-up store inside) stay in their kernels: every shared
-// form of them tried did that.
+// DiffDelRNN ring helpers of the mma.sync kernels, for a CTA of NT threads that owns the ns streams from b0 on.  hist_in and
+// hist_out hold each stream's last D samples of pre_d, oldest first.  ptxas reschedules the kernels' step loops when the
+// shape of this code changes, so compare their SASS after editing it.  The ring delay read stays in each kernel: every
+// shared form of it tried did that.
 
-// Carried history -> positions -D .. -1 of the pre_d ring (mma.sync kernels, a.ring_len > 0).
+// Carried history -> positions -D .. -1 of the pre_d ring.
 template <int NT>
 __device__ __forceinline__ void delay_ring_prefill(const GruArgs& a, long long b0, int ns, int tid, float* ring)
 {
@@ -211,35 +202,17 @@ __device__ __forceinline__ void delay_ring_prefill(const GruArgs& a, long long b
     }
 }
 
-// y of samples [t0, t0 + n) of the chunk (CH steps, SC streams per CTA), the taps read back through L2: from the pre_d this
-// CTA has just written (__ldcg) and from hist_in.
-template <int NT, int SC, int CH>
-__device__ __forceinline__ void delay_chunk_l2(const GruArgs& a, long long b0, int ns, int tid, long long t0, int n)
-{
-    for (int idx = tid; idx < SC * CH; idx += NT) {
-        const int s = idx / CH, tt = idx % CH;
-        if (s < ns && tt < n) {
-            const long long tg = t0 + tt;
-            const float* prow = a.pre + (b0 + s) * a.ldp;
-            const float* hrow = a.hist_in + (b0 + s) * (long long)a.D;
-            a.y[(b0 + s) * a.ldy + tg] =
-                delay_read(a.d[(b0 + s) * a.ldd + tg], tg, a.D,
-                           [&](long long i) { return i >= 0 ? __ldcg(prow + i) : hrow[a.D + i]; });
-        }
-    }
-}
-
-// Rolled delay history (code/model.py:314-315): hist_out = the last D samples of (hist_in || pre_d), once the CTA has
-// written all of pre_d.
+// Rolled delay history (code/model.py:314-315): hist_out = ring positions end - D .. end - 1, once the CTA has written
+// pre_d up to position end - 1 (end: a.T for a batched launch, the samples since open for the server).  They are still in
+// the ring because ring_len >= D + MMA_CH + 1.
 template <int NT>
-__device__ __forceinline__ void delay_roll_history(const GruArgs& a, long long b0, int ns, int tid)
+__device__ __forceinline__ void delay_ring_roll(const GruArgs& a, long long b0, int ns, int tid, const float* ring,
+                                                long long end)
 {
+    const int rmask = a.ring_len - 1;
     for (long long idx = tid; idx < (long long)ns * a.D; idx += NT) {
-        const int s = (int)(idx / a.D);
-        const long long i = idx % a.D;
-        const long long src = a.T - a.D + i;
-        a.hist_out[(b0 + s) * (long long)a.D + i] =
-            src >= 0 ? __ldcg(a.pre + (b0 + s) * a.ldp + src) : a.hist_in[(b0 + s) * (long long)a.D + a.D + src];
+        const int s = (int)(idx / a.D), i = (int)(idx % a.D);
+        a.hist_out[(b0 + s) * (long long)a.D + i] = ring[s * a.ring_len + ((int)(end - a.D + i) & rmask)];
     }
 }
 

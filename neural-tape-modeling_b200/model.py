@@ -578,8 +578,9 @@ class DelayBlockStream(BlockStream):
     Semantically identical to calling `model(x_block, d_block)` repeatedly (code/model.py:393-424 with `self.hidden` and
     `self.diffdel.buffer` carried): both start from the model (`initialize_hidden(B, max_D)`, `warm_start()` and a
     broadcast to B streams first give `predict()` semantics) and are written back by `close()`.  Buffers, raw pointers, the
-    handle and the CUDA stream are resolved once, so a block costs one ctypes call + one kernel launch; the history
-    alternates between two device buffers because the kernel's hist_out must not alias its hist_in.  When
+    handle and the CUDA stream are resolved once, so a block costs one ctypes call and one engine launch while the last
+    D + 129 samples of pre_d fit on chip (DESIGN.md 3.6; three launches otherwise: GRU, delay read, history roll); the history
+    alternates between two device buffers because hist_out must not alias hist_in.  When
     `model.diffdel.check_delay` is set (the default), every block first runs the reference's delay assert, which
     synchronises the stream once per block; a refused block raises AssertionError and changes nothing."""
 

@@ -318,11 +318,13 @@ def test_full_size_cfg2_properties():
 @pytest.mark.parametrize("mode,tuning,kernel", [("f16", (0, 0), 4), ("f16x3", (0, 0), 4), ("f16", (4, 3), 1),
                                                 ("f16", (8, 3), 1), ("tf32", (0, 0), 1), ("fp32", (0, 0), 0)])
 def test_tc_diffdel_delay_read_paths_bit_exact(mode, tuning, kernel, max_delay):
-    """The fused delay read of the mma.sync kernels keeps the last D + 129 samples of pre_d per stream (D = max_delay + 1)
-    in shared memory when they fit (D <= 1919 at four streams per CTA, D <= 895 at eight: max_delay = 1000 takes the ring
-    in one and L2 in the other) and reads its taps back through L2 otherwise, as the fp32 kernel always does.  Every
-    kernel and path must reproduce the oracle's delay line bit for bit on the engine's own pre_d and warm history, across
-    segment boundaries; a warm-up segment returns pre_d itself and still rolls the history."""
+    """The mma.sync kernels fuse the delay read where the last D + 129 samples of pre_d per stream (D = max_delay + 1) fit
+    in shared memory (D <= 1919 at four streams per CTA, D <= 895 at eight: max_delay = 1000 takes the ring in one and not
+    in the other), outside a warm-up call: one engine launch.  Every other DiffDelRNN launch -- a longer history, a
+    warm-up segment, the fp32 kernel -- runs the GRU into pre_d and then the stand-alone delay line: three launches
+    (GRU, delay read, history roll).  Every kernel and path must reproduce the oracle's delay line bit for bit on the
+    engine's own pre_d and warm history, across segment boundaries; a warm-up segment returns pre_d itself and still rolls
+    the history."""
     lib.load().ntm_set_tuning(*tuning)
     m = DiffDelRNN(input_size=1, hidden_size=64, output_size=1, skip=False, max_delay=max_delay).to(DEV)
     m.load_state_dict(load_ckpt("cfg3"))
@@ -342,9 +344,14 @@ def test_tc_diffdel_delay_read_paths_bit_exact(mode, tuning, kernel, max_delay):
         m.diffdel.buffer = m.diffdel.buffer.expand(B, 1, -1).contiguous()
         ys, ps, s = [], [], 0
         warm = slice(4032, 4532)                            # the warm-up segment
+        ring_fits = kernel != 0 and max_delay + 1 <= (895 if tuning == (8, 3) else 1919)
         for n in (31, 4000, 1, 500, 4468):
+            launches = lib.query(lib.Q_KERNEL_LAUNCHES)
             yy, pp = m(x[:, :, s:s + n], d[:, :, s:s + n], warmup=s == warm.start)
             assert lib.query(lib.Q_LAST_KERNEL) == kernel
+            # (less the one launch of the delay check forward runs while check_delay is on)
+            fused = ring_fits and s != warm.start
+            assert lib.query(lib.Q_KERNEL_LAUNCHES) - launches - 1 == (1 if fused else 3), (s, n)
             ys.append(yy)
             ps.append(pp)
             s += n
